@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the spline-coupling hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload two_moons_conditional|bounded16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload two_moons_conditional|bounded16] [--dump-outputs DIR]
   python bench.py --impl reference ...        # the reference's CPU implementation of the path
 
 One step = one ``Flow.__call__`` (log-prob) pass over one batch of synthetic events.  At N=1
@@ -18,6 +18,9 @@ metric through the public API from pinned HOST buffers (H2D of x and c, D2H of l
 the timed region); roofline for the dominant kernel; cpu_baseline = the numpy oracle ("port",
 NOT the reference: JAX is not installable in this image) on a bounded sample of the same
 workload.  ``--impl reference`` times that CPU port with all host cores.
+
+``--dump-outputs DIR`` writes what the timed path returned in its last step (log_prob, float32) as DIR/log_prob.npy.
+Inputs and parameters are seeded, so the same arguments give the same inputs and two builds can be compared.
 """
 from __future__ import annotations
 
@@ -48,7 +51,7 @@ def peaks():
         d = json.load(open(p))
         return dict(hbm=d["hbm_gbs"], bf16=d["bf16_tflops"], bf16_sustained=d.get("bf16_tflops_sustained"),
                     source="measured (MEASURED_PEAKS.json)")
-    return dict(hbm=6650.0, bf16=1590.0, bf16_sustained=1400.0, source="fallback (B200_PROFILING.md)")
+    return dict(hbm=6650.0, bf16=1590.0, bf16_sustained=1400.0, source="fallback (no MEASURED_PEAKS.json beside bench.py)")
 
 
 def chain_flops_per_event(w):
@@ -258,6 +261,24 @@ def ncu_traffic(workload, M):
     return json.load(open(p)).get(f"{workload}:{M}")
 
 
+DUMP_MAX_ROWS = 1 << 22   # 16 MiB of float32 per dumped 1-D array
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32.  An array of more than DUMP_MAX_ROWS rows is replaced by a
+    fixed sample of them: the rows np.sort(np.random.default_rng(0).choice(rows, DUMP_MAX_ROWS, replace=False)), so
+    runs with the same arguments write the same rows and two builds can be compared output for output."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        n = a.shape[0]
+        if n > DUMP_MAX_ROWS:
+            idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ROWS, replace=False))
+            a = a[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+
+
 def loop_events_per_s(fn, n_events, min_seconds=0.5, warm=3):
     """Device-timed events/s of fn(i) repeated until at least `min_seconds` have been timed (extras)."""
     import torch
@@ -384,7 +405,7 @@ def run_gpu(args):
         t0 = time.perf_counter()
         for i in range(K):
             ev[i][0].record()
-            step(W + i)
+            out = step(W + i)
             if drain is not None and i == K - 1:
                 drain()
             ev[i][1].record()
@@ -397,15 +418,18 @@ def run_gpu(args):
             t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             total_ms = float(t.item())
-        return total_ms, per, launches, (t0, t1)
+        return total_ms, per, launches, (t0, t1), out
 
     K, W = args.steps, max(args.warmup, 3)
     sampler = ClockSampler(local) if rank == 0 else None
-    total_ms, per, launches, (t0, t1) = timed(step_device, K, W)
+    total_ms, per, launches, (t0, t1), lp_last = timed(step_device, K, W)
     clocks = sampler.stop(t0, t1) if sampler else None
     value = world * M * K / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"log_prob": lp_last})   # what Flow.__call__ returned in the last timed step
+    del lp_last
 
-    e2e_ms, _, _, _ = timed(step_e2e, K, W, drain=drain_e2e)
+    e2e_ms, _, _, _, _ = timed(step_e2e, K, W, drain=drain_e2e)
     e2e_value = world * M * K / (e2e_ms * 1e-3)
     # the host buffer of the last timed step must hold that step's result (bit-exact against a device-resident rerun)
     last = W + K - 1
@@ -767,7 +791,14 @@ def main():
     ap.add_argument("--train-micro-batch", type=int, default=0, help="override TrainEngine's micro-batch (0: default)")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra legs (other eval config, deep_set)")
     ap.add_argument("--deep-set", type=int, default=1, help="run the deep_set (configs[2]) train-step leg at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the log_prob of the last timed step (rank 0) to DIR/log_prob.npy, float32; beyond "
+                         f"{DUMP_MAX_ROWS} events a fixed sample of them")
     args = ap.parse_args()
+    if args.impl == "native" and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the native path computed; the reference arm has no such output")
     if args.impl == "reference":
         run_reference(args)
     else:
