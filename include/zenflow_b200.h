@@ -149,8 +149,9 @@ int zf_rqs_inverse_normalized(void* stream, const float* y, const float* dx, con
                               int64_t M, int32_t d, int32_t K, float* x, int32_t* idx);
 
 /* Developer switch (parity tests): force a chain kernel ("simt", "umma", "umma8"; NULL / "" = automatic) and a train
- * GEMM ("simt"; NULL = tcgen05).  The ZF_CHAIN_IMPL / ZF_GEMM_IMPL environment variables give the initial values
- * and are read once per process. */
+ * GEMM ("simt" = the fp32 FFMA GEMM; "legacy" = the tcgen05 GEMM with register-path loaders for every shape; NULL / "" =
+ * tcgen05, fed by the copy engine where the operands allow tensor maps).  The ZF_CHAIN_IMPL / ZF_GEMM_IMPL environment
+ * variables give the initial values and are read once per process. */
 int zf_debug_set_impl(const char* chain_impl, const char* gemm_impl);
 
 /* Exhaustive device self-test of the exact-arithmetic fast paths the bin search relies on
@@ -172,9 +173,11 @@ int zf_selftest_umma_f16(void* stream, const float* A, const float* B, int32_t N
  * csrc/zf_img_gemm.cu); flags bit 0 / 1: A / B stored MN-major, bit 2: descriptor-field probe (developer) */
 int zf_selftest_umma_bf16(void* stream, const float* A, const float* B, int32_t N, int32_t K, float* out, int32_t flags);
 
-/* Self-test of the tcgen05 GEMM family used by the train step (zf_umma_gemm.cu), fp32 in/out:
+/* Self-test of the train step's GEMM family through the train step's own dispatcher (activation swish), fp32 in/out;
+ * the GEMM switch of zf_debug_set_impl selects which of the three GEMMs runs:
  * mode 0: C[I][J] = opA(A[I][R]) B[R][J] + bias; mode 1: C[I][J] = (A[I][R] B[J][R]^T) * swish'(Z[I][J]);
- * mode 2: C[I][J] += opA(A[R][I])^T B[R][J], colsum[J] += column sums of B (r_slab rows per CTA). */
+ * mode 2: C[I][J] += opA(A[R][I])^T B[R][J], colsum[J] += column sums of B (r_slab rows per CTA of the FFMA GEMM;
+ * the tcgen05 GEMM sizes its own slabs). */
 int zf_selftest_umma_gemm(void* stream, int32_t mode, const float* A, int64_t lda, const float* B, int64_t ldb,
                           float* C, int64_t ldc, const float* bias, float* colsum, const float* Z, int64_t ldz,
                           int32_t a_swish, int64_t I, int64_t J, int64_t R, int64_t r_slab);

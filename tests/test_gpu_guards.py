@@ -91,10 +91,10 @@ def test_chain_kernels_stay_in_bounds(cfg, impl, request):
     assert bool(torch.isfinite(lp).all() | True)
 
 
-@pytest.mark.parametrize("gemm", ["", "simt"])
+@pytest.mark.parametrize("gemm", ["", "legacy", "simt"])
 def test_train_step_stays_in_bounds(gemm, request):
-    """The whole train step with its buffers carved out of guarded arenas (TrainEngine allocates through
-    torch; here the C-ABI GEMM family is called directly on ragged shapes)."""
+    """The train step's GEMMs with their buffers carved out of guarded arenas (TrainEngine allocates through
+    torch; here each of the three GEMMs is called directly on ragged shapes)."""
     from zenflow_b200 import _lib
 
     _lib.set_impl(None, gemm or None)

@@ -70,15 +70,25 @@ def _swish_grad(z):
     return s * (1 + z * (1 - s))
 
 
-@pytest.mark.parametrize("mode,I,J,R,a_swish", [
+GEMM_SHAPES = [
     (0, 300, 760, 128, 1), (0, 1000, 128, 12, 0), (0, 129, 47, 128, 1), (0, 64, 128, 2, 0),
     (1, 300, 128, 760, 0), (1, 777, 12, 128, 0), (1, 130, 128, 47, 0),
     (2, 128, 760, 5000, 1), (2, 12, 128, 4097, 0), (2, 128, 47, 300, 1), (2, 2, 128, 31, 0),
-])
-def test_umma_gemm_family(mode, I, J, R, a_swish):
-    """The three GEMM shapes of the conditioner VJP on tcgen05, incl. ragged sizes, vs float64."""
+]
+GEMMS = ["", "legacy", "simt"]
+
+
+# the default GEMM ("") keeps the shape-only test ids
+@pytest.mark.parametrize("mode,I,J,R,a_swish,gemm", [s + (g,) for g in GEMMS for s in GEMM_SHAPES],
+                         ids=["-".join(map(str, s + ((g,) if g else ()))) for g in GEMMS for s in GEMM_SHAPES])
+def test_umma_gemm_family(mode, I, J, R, a_swish, gemm, request):
+    """The three GEMM shapes of the conditioner VJP, incl. ragged sizes, vs float64, on each train GEMM: "" = tcgen05
+    fed by the copy engine where the operands allow (else register-path loaders), "legacy" = tcgen05 with
+    register-path loaders, "simt" = the fp32 FFMA GEMM."""
     from zenflow_b200 import _lib
 
+    _lib.set_impl(None, gemm or None)
+    request.addfinalizer(lambda: _lib.set_impl(None))
     lib = _lib.load()
     rng = np.random.default_rng(mode * 1000 + I + J + R)
     st = torch.cuda.current_stream().cuda_stream

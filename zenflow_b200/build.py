@@ -26,7 +26,6 @@ NVCC_FLAGS = [
 ]
 
 
-# developer builds: ZF_NVCC_EXTRA="-DZF_EXPERIMENTAL" compiles the measured-slower kernel variants back in
 EXTRA_FLAGS = [f for f in os.environ.get("ZF_NVCC_EXTRA", "").split() if f]
 
 

@@ -1,6 +1,7 @@
-// C-ABI plumbing: thread-local error message, launch counter, per-device attribute cache.
+// C-ABI plumbing: thread-local error message, launch counter, per-device attribute cache, shared-memory opt-in.
 #include "zf_common.cuh"
 
+#include <map>
 #include <mutex>
 #include <string.h>
 
@@ -48,6 +49,20 @@ int get_device_info(DeviceInfo* out) {
         have[dev] = true;
     }
     *out = cache[dev];
+    return ZF_OK;
+}
+
+int smem_optin(const void* fn, size_t bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<const void*, int>, size_t> done;
+    int dev = 0;
+    ZF_CUDA_CHECK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(mu);
+    size_t& have = done[{fn, dev}];
+    if (have < bytes) {
+        ZF_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        have = bytes;
+    }
     return ZF_OK;
 }
 

@@ -25,13 +25,9 @@
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
-#include <map>
-#include <mutex>
 #include <vector>
 
 namespace zf {
-
-void count_launch();
 
 constexpr int TM = 64;        // samples per tile
 constexpr int KC = 16;        // k rows per staged weight chunk
@@ -612,9 +608,9 @@ __host__ __device__ inline UCst ucst_layout(int Fmax, int Hmax, int BLmax, bool 
 }
 constexpr int USTEPS = 40;   // step descriptors kept in shared memory (longer programs read them from global)
 constexpr int VJP_ROW = 97;   // floats per theta row of the VJP kernel (odd: one thread per row without bank conflicts)
-__host__ __device__ inline size_t umma_hs_floats(int Fmax, bool) { return (size_t)Fmax * UM; }   // x - mean, [Fmax][UM]
+__host__ __device__ inline size_t umma_hs_floats(int Fmax) { return (size_t)Fmax * UM; }   // x - mean, [Fmax][UM]
 __host__ __device__ inline size_t umma_smem_floats(int D, int C, int Fmax, int Hmax, int BLmax, bool vjp = false, bool img = false) {
-    return 2 * (size_t)UM * (D + C) + umma_hs_floats(Fmax, img) + (vjp ? 1 : 2) * (size_t)ucst_layout(Fmax, Hmax, BLmax, img).total + 11 * UM +
+    return 2 * (size_t)UM * (D + C) + umma_hs_floats(Fmax) + (vjp ? 1 : 2) * (size_t)ucst_layout(Fmax, Hmax, BLmax, img).total + 11 * UM +
            (vjp ? 2 * UM * VJP_ROW : 2 * 8 * UM * 4) +
            (size_t)URING * URING_FLOATS + 2 * B_COUNT + 32 + USTEPS * sizeof(StepDesc) / sizeof(float);
 }
@@ -660,41 +656,13 @@ __device__ __forceinline__ float theta_block_finish(int col, const float* __rest
 }
 
 
-// Locate the bin from tensor memory.  The three raw blocks are loaded in a software pipeline (the next
-// block's TMEM load is in flight while the current one is processed) and the D buffer is handed back to
-// the MMA warp (release()) right after the last load, before the second pass and the spline evaluation.
-template <int KT, bool INVERSE, class Release>
-__device__ __forceinline__ void spline_row_tmem(uint32_t dbase, uint32_t cross_off, const float* __restrict__ bias, float v,
-                                                RqsBin& b, Release release) {
-    constexpr int cs_ = INVERSE ? KT : 0, co_ = INVERSE ? 0 : KT;
-    const KnotNorm kn = make_knot_norm(KT);
-    float pa[KT], pb[KT], wa[KT], wb[KT];
-    RqsCheck chk;
-    theta_block_issue<KT>(dbase, cross_off, cs_, pa, wa);
-    umma::wait_ld();
-    const float amax_s = theta_block_finish<KT>(cs_, bias, pa, wa);   // (wa is dead before pb / wb come alive)
-    theta_block_issue<KT>(dbase, cross_off, co_, pb, wb);          // in flight during the search pass
-    if (__any_sync(0xffffffffu, !(amax_s < kThetaFastBound)))
-        rqs_block_search<KT, true>(pa, v, kn, b.idx, b.ks, b.bs, chk);
-    else
-        rqs_block_search<KT, false>(pa, v, kn, b.idx, b.ks, b.bs, chk);
-    umma::wait_ld();
-    const float amax_o = theta_block_finish<KT>(co_, bias, pb, wb);
-    theta_block_issue<KT>(dbase, cross_off, 2 * KT, pa, wa);       // slopes reuse the searched block's registers
-    umma::wait_ld();
-    release();                                          // every TMEM read of this row is done
-    if (__any_sync(0xffffffffu, !(amax_o < kThetaFastBound)))
-        rqs_block_other<KT, true>(pb, b.idx, kn, b.ko, b.bo, chk);
-    else
-        rqs_block_other<KT, false>(pb, b.idx, kn, b.ko, b.bo, chk);
-    (void)theta_block_finish<KT>(2 * KT, bias, pa, wa);
-    rqs_block_slopes<KT>(pa, b.idx, b.dk, b.dkp1);
-}
-
-// The same row with the lean block forms of zf_math.cuh (rows are issue-bound: ~1.3k instead of ~1.9k instructions
-// for K = 32).  Bins are bit-identical to spline_row_tmem; the other-axis knot, the bin height / width and the
-// knot derivatives are fp32-tolerance quantities either way.  scr: this thread's scratch column (float4, stride
-// apart, KT / 4 entries).  Rows with |theta| >= kThetaFastBound (or inf) take spline_row_tmem's IEEE path.
+// One spline row of this thread's event from a D buffer in tensor memory, with the lean block forms of zf_math.cuh
+// (rows are issue-bound: ~1.3k instead of ~1.9k instructions for K = 32).  The three raw blocks are loaded in a software
+// pipeline (the next block's TMEM load is in flight while the current one is processed) and the D buffer is handed
+// back to the MMA warp (release()) right after the last load.  Bins are bit-identical to the IEEE path
+// (rqs_block_search<KT, true>); the other-axis knot, the bin height / width and the knot derivatives are
+// fp32-tolerance quantities either way.  scr: this thread's scratch column (float4, stride apart, KT / 4 entries).
+// Rows with |theta| >= kThetaFastBound (or inf) take the IEEE path (rqs_block_search / rqs_block_other<KT, true>).
 template <int KT>
 __device__ __forceinline__ float theta_block_finish_lean(int col, const float* __restrict__ bias, float (&p)[KT],
                                                          const float (&w)[KT]) {
@@ -725,7 +693,7 @@ __device__ __forceinline__ void spline_row_tmem_lean(uint32_t dbase, uint32_t cr
     theta_block_issue<KT>(dbase, cross_off, 2 * KT, pa, wa);       // raw slopes reuse the searched block's registers
     umma::wait_ld();
     release();                                          // every TMEM read of this row is done
-    if (__any_sync(0xffffffffu, !(amax_o < kThetaFastBound))) rqs_block_other<KT, true>(pb, b.idx, kn, b.ko, b.bo, chk);
+    if (__any_sync(0xffffffffu, !(amax_o < kThetaFastBound))) rqs_block_other<KT>(pb, b.idx, kn, b.ko, b.bo, chk);
     else rqs_block_other_lean<KT>(pb, b.idx, kn, scr, stride, b.ko, b.bo);
     rqs_block_slopes_lean<KT>(pa, wa, umma::kF16LoUnscale, bias + 2 * KT, b.idx, scr, stride, b.dk, b.dkp1);
 }
@@ -734,7 +702,8 @@ __device__ __forceinline__ void spline_row_tmem_lean(uint32_t dbase, uint32_t cr
 // single dim and would otherwise leave group 1 idle: group 0 normalises the searched axis and finds the bin while
 // group 1 normalises the other axis; the bin goes over through shared memory, group 1 selects the other-axis knot
 // and the slopes and hands them back; then group 0 evaluates y (or x) while group 1 evaluates log|dy/dx|.
-// Operation for operation the same arithmetic as spline_row_tmem + rqs_eval_*.
+// Operation for operation the same arithmetic as the IEEE and exact-fast block forms (rqs_block_search<KT, SAFE> +
+// rqs_block_other_pre / _post<KT, SAFE>) + rqs_eval_*.
 __device__ __forceinline__ void pair_barrier(int id) { asm volatile("bar.sync %0, 256;" ::"r"(id) : "memory"); }
 
 template <int KT, bool INVERSE>
@@ -855,8 +824,7 @@ __device__ __forceinline__ float vjp_row_tmem(uint32_t dbase, const float* __res
 // ---- the epilogue / SIMT role of the tensor-core chain kernel ------------------------------------------------
 // NG column groups of 4 warps each (group g = warp / 4 owns CW = 32 / NG columns of every 32-column K-chunk and
 // every NG-th feature / bounded column); TMEM lane quarter = warp % 4 (hardware rule).  Spline rows are run by
-// groups 0 and 1 (one transformed dim each, alternating accumulator buffers).  HELPER = groups 2.. of the
-// 4-group kernel, compiled without the spline code so that they fit a small register allocation.
+// groups 0 and 1 (one transformed dim each, alternating accumulator buffers).
 struct UCtx {
     const ChainArgs& a;
     float *xs, *cs, *xraw, *hs, *cst, *ldx, *pairx;
@@ -895,7 +863,6 @@ template <bool INVERSE, bool VJP = false>
 __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
     static_assert(!(INVERSE && VJP), "the VJP kernel recomputes the forward conditioner");
     constexpr int NG = 2;
-    constexpr bool HELPER = false;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int q = warp & 3, half = warp >> 2, m = q * 32 + lane;   // half = column group g in [0, NG)
     constexpr int ET = NG * 128, CW = 32 / NG;                    // epilogue threads; columns per thread and K-chunk
@@ -1247,7 +1214,7 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                         }
                     }
                 }
-            } else if (!HELPER && d == 1 && half < 2) {
+            } else if (d == 1 && half < 2) {
                 // one transformed dim: the two spline groups share its row (see spline_row_search_half)
                 mbar_wait(&bars[B_DFULL_D + 0], p_fd);
                 p_fd ^= 1u;
@@ -1278,32 +1245,33 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                     pair_barrier(4);
                     if (!INVERSE) ldc += rqs_eval_forward_ld(v, bin);
                 }
-            } else if (!HELPER)
-            for (int jj = half; jj < d && half < 2; jj += 2) {
-                mbar_wait(&bars[B_DFULL_D + half], p_fd);
-                p_fd ^= 1u;
-                umma::fence_after_sync();
-                ZF_TR(trs);   // theta ready
-                const uint32_t dbase = umma::taddr(tb, lane_base, tc_dmain(half));
-                float* px = xs + pmod(jj - rot, D) * UM + m;
-                const float v = *px;
-                RqsBin bin;
-                auto release = [&]() {
-                    umma::fence_before_sync();
-                    umma::mbar_arrive(&bars[B_DEMPTY_D + half]);
-                    ZF_TR(trs);   // released
-                };
-                float4* scr = cx.scratch + (size_t)half * 8 * UM + m;   // [half][K / 4][UM] float4
-                if (K == 16) spline_row_tmem_lean<16, INVERSE>(dbase, TC_XOFF, bls + jj * NL, v, bin, scr, UM, release);
-                else spline_row_tmem_lean<32, INVERSE>(dbase, TC_XOFF, bls + jj * NL, v, bin, scr, UM, release);
-                if (m < nm) put_idx(a, s, m0 + m, jj, bin.idx);
-                if (!INVERSE) {
-                    float y, ld;
-                    rqs_eval_forward(v, bin, y, ld);
-                    *px = y;
-                    ldc += ld;
-                } else {
-                    *px = rqs_eval_inverse(v, bin);
+            } else {
+                for (int jj = half; jj < d && half < 2; jj += 2) {
+                    mbar_wait(&bars[B_DFULL_D + half], p_fd);
+                    p_fd ^= 1u;
+                    umma::fence_after_sync();
+                    ZF_TR(trs);   // theta ready
+                    const uint32_t dbase = umma::taddr(tb, lane_base, tc_dmain(half));
+                    float* px = xs + pmod(jj - rot, D) * UM + m;
+                    const float v = *px;
+                    RqsBin bin;
+                    auto release = [&]() {
+                        umma::fence_before_sync();
+                        umma::mbar_arrive(&bars[B_DEMPTY_D + half]);
+                        ZF_TR(trs);   // released
+                    };
+                    float4* scr = cx.scratch + (size_t)half * 8 * UM + m;   // [half][K / 4][UM] float4
+                    if (K == 16) spline_row_tmem_lean<16, INVERSE>(dbase, TC_XOFF, bls + jj * NL, v, bin, scr, UM, release);
+                    else spline_row_tmem_lean<32, INVERSE>(dbase, TC_XOFF, bls + jj * NL, v, bin, scr, UM, release);
+                    if (m < nm) put_idx(a, s, m0 + m, jj, bin.idx);
+                    if (!INVERSE) {
+                        float y, ld;
+                        rqs_eval_forward(v, bin, y, ld);
+                        *px = y;
+                        ldc += ld;
+                    } else {
+                        *px = rqs_eval_inverse(v, bin);
+                    }
                 }
             }
             ZF_TR(trs);   // spline rows done
@@ -1374,7 +1342,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
     float* cs = xs + D * UM;                  // [C][UM]
     float* xraw = cs + C * UM;                // [UM][D] | [UM][C]  next tile as it lies in global memory (cp.async)
     float* hs = xraw + UM * (D + C);          // [Fmax][UM]  x - mean (couplings whose first Dense reads it from shared memory)
-    float* cst = hs + umma_hs_floats(a.u_fmax, a.u_w0img != 0);   // [2][cl.total] per-coupling constants
+    float* cst = hs + umma_hs_floats(a.u_fmax);   // [2][cl.total] per-coupling constants
     // the VJP kernel runs ONE coupling: its constants are fetched once and both buffer indices name the same block
     const int cst_stride = VJP ? 0 : cl.total;
     float* ldx = cst + (VJP ? 1 : 2) * cl.total;
@@ -2160,6 +2128,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
 // ---- host side ------------------------------------------------------------------------
 
 struct Plan {
+    int D = 0, C = 0;                     // chain dim and conditioning dim
     std::vector<PackJob> jobs;
     int rot_total = 0;
     int act_rows = KC;
@@ -2168,7 +2137,7 @@ struct Plan {
     int n_couplings = 0;
     int Fmax = 1, Hmax = 1, BLmax = 32;   // shared-memory sizing of the two-pipeline kernel
     bool all_d1 = true;                   // every coupling transforms a single dim
-    bool w0img = false;                   // constant blocks carry the first Dense's operand image (tensor-core first Dense)
+    bool w0img = false;                   // constant blocks carry the first Dense's operand image (choose_chain_kernel)
 };
 
 // for_vjp: the plan of the fused VJP kernel (a chain of one coupling, multi-dim or not)
@@ -2178,6 +2147,8 @@ static int build_plan(const zf_chain* chain, Plan& plan, bool for_vjp = false) {
     ZF_REQUIRE(D >= 1 && D <= ZF_MAX_DIM, "dim must be in [1, %d] (got %d)", ZF_MAX_DIM, D);
     ZF_REQUIRE(C >= 0 && C <= 1024, "cdim must be in [0, 1024] (got %d)", C);
     ZF_REQUIRE(chain->n_ops >= 0 && (chain->n_ops == 0 || chain->ops), "ops is NULL");
+    plan.D = D;
+    plan.C = C;
     int rot = 0;
     for (int i = 0; i < chain->n_ops; ++i) {
         const zf_op& op = chain->ops[i];
@@ -2259,7 +2230,7 @@ static int build_plan(const zf_chain* chain, Plan& plan, bool for_vjp = false) {
         plan.jobs.push_back(job);
     }
     plan.rot_total = rot;
-    // multi-dim couplings with at most 16 conditioner inputs: first Dense on the tensor cores (single-tile kernel)
+    // constant-block layout: see choose_chain_kernel
     plan.w0img = plan.umma_ok && plan.n_couplings > 0 && (for_vjp || !plan.all_d1) && plan.Fmax <= 16;
 
     // workspace layout: StepDesc array, then per-step blocks (all multiples of 4 floats)
@@ -2310,13 +2281,6 @@ static LatentConst make_latent(int kind, float peakness) {
 
 enum PackMode : int { kPackAndRun = 0, kPackOnly = 1, kRunPacked = 2 };
 
-// Developer switches: which chain kernel (simt | umma | umma8) and which
-// train GEMM (simt | umma) run.  The environment (ZF_CHAIN_IMPL, ZF_GEMM_IMPL) is read ONCE per process;
-// zf_debug_set_impl overrides it afterwards (the parity tests compare the implementations inside one process).
-struct ImplSwitch {
-    char chain[16];
-    char gemm[16];
-};
 ImplSwitch& impl_switch() {
     static ImplSwitch sw = [] {
         ImplSwitch v{};
@@ -2328,9 +2292,52 @@ ImplSwitch& impl_switch() {
     }();
     return sw;
 }
-static const char* chain_impl_env() {
-    const char* v = impl_switch().chain;
-    return v[0] ? v : nullptr;
+enum class ChainKernel { kNone, kFfma, kUmma, kUmmaPP, kUmmaVjp };
+struct ChainLaunch {
+    ChainKernel kernel;
+    size_t smem;   // dynamic shared memory, bytes
+};
+
+// Which kernel runs a planned chain on this device, and the dynamic shared memory it needs.  impl is the chain
+// developer switch (impl_switch().chain).  With
+//   tc       = every coupling fits the tensor-core kernels (Plan::umma_ok), there is at least one, and impl != simt
+//   fits(k)  = k's shared memory is within the device's opt-in limit
+// an eval pass (forward, inverse, log_prob, sample) takes the first row that applies:
+//   tc, fits(single-tile), all_d1, n_steps <= USTEPS, impl != umma8, fits(two-tile)  chain_umma_pp_kernel
+//   tc, fits(single-tile)                                                            chain_umma_kernel
+//   !tc, impl == umma                                                                ZF_ERR_UNSUPPORTED
+//   fits(FFMA tile)        (a tc chain beyond the single-tile kernel's memory too)   chain_kernel
+//   otherwise                                                                        ZF_ERR_UNSUPPORTED
+// and the VJP of one coupling (vjp, the plan of vjp_plan):
+//   tc, fits(single-tile VJP)   chain_umma_kernel<false, true>;   otherwise kNone (zf_coupling_backward's unfused path)
+// The constant blocks are laid out by build_plan, before the device is known: for tc couplings with Fmax <= 16 they carry
+// the first Dense's operand image (Plan::w0img: first Dense on the tensor cores), except in the eval passes of flows
+// whose couplings all transform one dim.  Those take the two-tile kernel, whose first Dense is FFMA, and keep the FFMA
+// first Dense when they fall back to the single-tile kernel (umma8, n_steps > USTEPS, two-tile memory).
+static int choose_chain_kernel(const Plan& plan, const DeviceInfo& di, bool vjp, const char* impl, ChainLaunch* out) {
+    const size_t limit = (size_t)di.max_smem_optin;
+    const bool tc = plan.umma_ok && plan.n_couplings > 0 && impl[0] != 's';
+    const size_t usmem = umma_smem_floats(plan.D, plan.C, plan.Fmax, plan.Hmax, plan.BLmax, vjp, plan.w0img) * sizeof(float);
+    if (vjp) {
+        *out = (tc && usmem <= limit) ? ChainLaunch{ChainKernel::kUmmaVjp, usmem} : ChainLaunch{ChainKernel::kNone, 0};
+        return ZF_OK;
+    }
+    if (!tc && strcmp(impl, "umma") == 0)
+        return fail(ZF_ERR_UNSUPPORTED, "ZF_CHAIN_IMPL=umma but this chain does not fit the tensor-core kernel");
+    if (tc && usmem <= limit) {
+        const size_t psmem = umma_pp_smem_floats(plan.D, plan.C, plan.Fmax, plan.Hmax, plan.BLmax) * sizeof(float);
+        if (plan.all_d1 && (int)plan.jobs.size() <= USTEPS && strcmp(impl, "umma8") != 0 && psmem <= limit)
+            *out = {ChainKernel::kUmmaPP, psmem};
+        else
+            *out = {ChainKernel::kUmma, usmem};
+        return ZF_OK;
+    }
+    const size_t smem = ((size_t)(plan.D + plan.C) * TM + 2 * (size_t)plan.act_rows * TM + 2 * KC * NCOL) * sizeof(float);
+    if (smem > limit)
+        return fail(ZF_ERR_UNSUPPORTED, "chain tile needs %zu bytes of shared memory (limit %d): layers too wide", smem,
+                    di.max_smem_optin);
+    *out = {ChainKernel::kFfma, smem};
+    return ZF_OK;
 }
 
 static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int latent_kind, float peakness,
@@ -2390,84 +2397,37 @@ static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int l
     a.lc = make_latent(latent_kind, peakness);
     a.idx_out = idx_out;
     a.n_couplings = plan.n_couplings;
+    a.u_fmax = plan.Fmax;
+    a.u_hmax = plan.Hmax;
+    a.u_blmax = plan.BLmax;
+    a.u_w0img = plan.w0img ? 1 : 0;
 
-    // once per device and kernel: opt in to the large dynamic shared-memory carve-out
-    auto set_smem = [&](const void* fn, size_t bytes) -> int {
-        static std::mutex mu;
-        static std::map<std::pair<const void*, int>, size_t> done;
-        std::lock_guard<std::mutex> lock(mu);
-        size_t& have = done[{fn, di.device}];
-        if (have < bytes) {
-            ZF_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-            have = bytes;
-        }
+    ChainLaunch k;
+    if (int rc = choose_chain_kernel(plan, di, false, impl_switch().chain, &k)) return rc;
+    auto launch = [&](auto kern, long long blocks, unsigned threads) -> int {
+        if (int rc = smem_optin((const void*)kern, k.smem)) return rc;
+        kern<<<(unsigned)blocks, threads, k.smem, stream>>>(a);
+        count_launch();
+        ZF_CUDA_CHECK(cudaGetLastError());
         return ZF_OK;
     };
-
-    // tensor-core kernel when every coupling fits it (ZF_CHAIN_IMPL=simt forces the FFMA kernel)
-    const char* impl = chain_impl_env();
-    const bool want_umma = plan.umma_ok && plan.n_couplings > 0 && !(impl && impl[0] == 's');
-    if (impl && strcmp(impl, "umma") == 0 && !want_umma)
-        return fail(ZF_ERR_UNSUPPORTED, "ZF_CHAIN_IMPL=umma but this chain does not fit the tensor-core kernel");
-    if (want_umma) {
-        a.u_fmax = plan.Fmax;
-        a.u_hmax = plan.Hmax;
-        a.u_blmax = plan.BLmax;
-        a.u_w0img = plan.w0img ? 1 : 0;
-        const size_t usmem = umma_smem_floats(a.D, a.C, plan.Fmax, plan.Hmax, plan.BLmax, false, plan.w0img) * sizeof(float);
-        if (usmem <= (size_t)di.max_smem_optin) {
-            const long long tiles = (M + UM - 1) / UM;
-            const unsigned ugrid = (unsigned)std::min<long long>(tiles, (long long)di.sm_count);
-            // flows whose couplings transform one dim: two tiles in flight (chain_umma_pp_kernel); ZF_CHAIN_IMPL=umma8
-            // keeps the single-tile kernel for them
-            if (plan.all_d1 && a.n_steps <= USTEPS && !(impl && strcmp(impl, "umma8") == 0)) {
-                const size_t psmem = umma_pp_smem_floats(a.D, a.C, plan.Fmax, plan.Hmax, plan.BLmax) * sizeof(float);
-                if (psmem <= (size_t)di.max_smem_optin) {
-                    const unsigned pgrid = (unsigned)std::min<long long>((tiles + 1) / 2, (long long)di.sm_count);
-                    if (mode == kModeInverse) {
-                        if (int rc = set_smem((const void*)chain_umma_pp_kernel<true>, psmem)) return rc;
-                        chain_umma_pp_kernel<true><<<pgrid, PP_THREADS, psmem, stream>>>(a);
-                    } else {
-                        if (int rc = set_smem((const void*)chain_umma_pp_kernel<false>, psmem)) return rc;
-                        chain_umma_pp_kernel<false><<<pgrid, PP_THREADS, psmem, stream>>>(a);
-                    }
-                    count_launch();
-                    ZF_CUDA_CHECK(cudaGetLastError());
-                    return ZF_OK;
-                }
-            }
-            auto launch = [&](auto kern, unsigned threads) -> int {
-                if (int rc = set_smem((const void*)kern, usmem)) return rc;
-                kern<<<ugrid, threads, usmem, stream>>>(a);
-                return ZF_OK;
-            };
-            int rc;
-            if (mode == kModeInverse) rc = launch(chain_umma_kernel<true>, 320);
-            else rc = launch(chain_umma_kernel<false>, 320);
-            if (rc != ZF_OK) return rc;
-            count_launch();
-            ZF_CUDA_CHECK(cudaGetLastError());
-            return ZF_OK;
+    const bool inv = mode == kModeInverse;
+    const long long utiles = (M + UM - 1) / UM;
+    switch (k.kernel) {
+        case ChainKernel::kUmmaPP: {   // two tiles in flight per CTA
+            const long long blocks = std::min<long long>((utiles + 1) / 2, di.sm_count);
+            return inv ? launch(chain_umma_pp_kernel<true>, blocks, PP_THREADS) : launch(chain_umma_pp_kernel<false>, blocks, PP_THREADS);
+        }
+        case ChainKernel::kUmma: {
+            const long long blocks = std::min<long long>(utiles, di.sm_count);
+            return inv ? launch(chain_umma_kernel<true>, blocks, 320) : launch(chain_umma_kernel<false>, blocks, 320);
+        }
+        default: {   // kFfma (an eval pass is never kNone or kUmmaVjp)
+            const int bps = (2 * (k.smem + 1024) <= (size_t)di.max_smem_optin) ? 2 : 1;
+            const long long blocks = std::min<long long>((M + TM - 1) / TM, (long long)di.sm_count * bps);
+            return inv ? launch(chain_kernel<true>, blocks, kChainThreads) : launch(chain_kernel<false>, blocks, kChainThreads);
         }
     }
-    const size_t smem = ((size_t)(a.D + a.C) * TM + 2 * (size_t)a.act_rows * TM + 2 * KC * NCOL) * sizeof(float);
-    if (smem > (size_t)di.max_smem_optin)
-        return fail(ZF_ERR_UNSUPPORTED, "chain tile needs %zu bytes of shared memory (limit %d): layers too wide", smem,
-                    di.max_smem_optin);
-    const int bps = (2 * (smem + 1024) <= (size_t)di.max_smem_optin) ? 2 : 1;
-    const long long n_tiles = (M + TM - 1) / TM;
-    const unsigned grid = (unsigned)std::min<long long>(n_tiles, (long long)di.sm_count * bps);
-
-    if (mode == kModeInverse) {
-        if (int rc = set_smem((const void*)chain_kernel<true>, smem)) return rc;
-        chain_kernel<true><<<grid, kChainThreads, smem, stream>>>(a);
-    } else {
-        if (int rc = set_smem((const void*)chain_kernel<false>, smem)) return rc;
-        chain_kernel<false><<<grid, kChainThreads, smem, stream>>>(a);
-    }
-    count_launch();
-    ZF_CUDA_CHECK(cudaGetLastError());
-    return ZF_OK;
 }
 
 // ---- fused conditioner recompute + spline VJP of ONE coupling (tensor-core path of zf_coupling_backward) ---------
@@ -2480,17 +2440,15 @@ static int vjp_plan(const zf_coupling* cp, int D, int C, Plan& plan, zf_op& op, 
     return build_plan(&chain, plan, true);
 }
 
-// floats of packed parameters the fused VJP kernel needs, 0 when this coupling / device does not fit it
 size_t coupling_vjp_ws_floats(const zf_coupling* cp, int D, int C) {
     Plan plan;
     zf_op op;
     zf_chain chain;
-    const char* impl = chain_impl_env();
-    if (impl && impl[0] == 's') return 0;
-    if (vjp_plan(cp, D, C, plan, op, chain) != ZF_OK || !plan.umma_ok || plan.n_couplings != 1) return 0;
     DeviceInfo di;
-    if (get_device_info(&di) != ZF_OK) return 0;
-    if (umma_smem_floats(D, C, plan.Fmax, plan.Hmax, plan.BLmax, true, plan.w0img) * sizeof(float) > (size_t)di.max_smem_optin) return 0;
+    ChainLaunch k;
+    if (vjp_plan(cp, D, C, plan, op, chain) != ZF_OK || get_device_info(&di) != ZF_OK ||
+        choose_chain_kernel(plan, di, true, impl_switch().chain, &k) != ZF_OK || k.kernel != ChainKernel::kUmmaVjp)
+        return 0;
     return plan.ws_floats;
 }
 
@@ -2537,20 +2495,13 @@ int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, c
         ZF_REQUIRE(((reinterpret_cast<uintptr_t>(img_act[l]) | reinterpret_cast<uintptr_t>(act_g[l])) & 15) == 0,
                    "coupling_vjp: images must be 16-byte aligned");
     }
-    const size_t smem = umma_smem_floats(D, C, plan.Fmax, plan.Hmax, plan.BLmax, true, plan.w0img) * sizeof(float);
-    static std::mutex mu;
-    static std::map<int, size_t> done;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        size_t& have = done[di.device];
-        if (have < smem) {
-            ZF_CUDA_CHECK(cudaFuncSetAttribute((const void*)chain_umma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            have = smem;
-        }
-    }
+    ChainLaunch k;
+    if (int rc = choose_chain_kernel(plan, di, true, impl_switch().chain, &k)) return rc;
+    ZF_REQUIRE(k.kernel == ChainKernel::kUmmaVjp, "coupling_vjp: the coupling does not take the fused kernel (coupling_vjp_ws_floats is 0)");
+    if (int rc = smem_optin((const void*)chain_umma_kernel<false, true>, k.smem)) return rc;
     const long long tiles = (M + UM - 1) / UM;
     if (tiles == 0) return ZF_OK;
-    chain_umma_kernel<false, true><<<(unsigned)std::min<long long>(tiles, (long long)di.sm_count), 320, smem, stream>>>(a);
+    chain_umma_kernel<false, true><<<(unsigned)std::min<long long>(tiles, (long long)di.sm_count), 320, k.smem, stream>>>(a);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;

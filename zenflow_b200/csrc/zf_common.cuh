@@ -36,6 +36,39 @@ struct DeviceInfo {
 // Cached per device (once-per-device init is the only global mutable state).
 int get_device_info(DeviceInfo* out);
 
+// Opt kernel `fn` in to `bytes` of dynamic shared memory on the current device.  The attribute is per device, so the
+// largest value set is remembered per (function, device) and only a larger request calls the runtime again.
+int smem_optin(const void* fn, size_t bytes);
+
+// Adds one to the launch counter of zf_launch_count.
+void count_launch();
+
+// Developer switches, for tests and measurements that compare implementations (zf_chain.cu):
+//   chain  "" automatic | "simt" FFMA chain_kernel | "umma" tensor-core kernel or an error | "umma8" single-tile
+//          tensor-core kernel for single-dim flows too (choose_chain_kernel)
+//   gemm   "" automatic | "simt" FFMA gemm_kernel | "legacy" tcgen05 GEMM with register-path loaders (launch_gemm)
+// The environment (ZF_CHAIN_IMPL, ZF_GEMM_IMPL) is read once per process; zf_debug_set_impl overrides it afterwards.
+struct ImplSwitch {
+    char chain[16];
+    char gemm[16];
+};
+ImplSwitch& impl_switch();
+
+// ---- entry points shared between translation units -------------------------------------
+
+// tcgen05 GEMM family of the train step (zf_umma_gemm.cu); same argument convention as the FFMA gemm of zf_train.cu.
+int launch_umma_gemm(cudaStream_t st, int mode, const float* A, long long lda, const float* B, long long ldb, float* C,
+                     long long ldc, const float* bias, float* colsum, const float* Z, long long ldz, int a_swish,
+                     long long I, long long J, long long R, long long r_slab);
+
+// Fused conditioner recompute + spline VJP of one coupling (zf_chain.cu).  ws_floats is 0 when the coupling or the
+// device does not take the fused kernel.
+size_t coupling_vjp_ws_floats(const zf_coupling* cp, int D, int C);
+int coupling_vjp_pack(cudaStream_t stream, const zf_coupling* cp, int D, int C, float* ws);
+int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, const float* ws, const float* x_in, const float* c,
+                     const float* gy, int gy_rot, const float* glp, long long M, float* gx, void* img_h0, int wh0, void* const* img_act,
+                     float* const* act_g, void* img_dtheta);
+
 // One weight image of pack_w_images (zf_img_gemm.cu): Wimg(n, k) = W[n * ldw + (k / NL) * P + k % NL] for n < n_valid and
 // k % NL < P, else 0, as the bf16x2 hi | lo operand image of img_nt_kernel.  block0 / blocks are filled by the launcher.
 struct PackWJob {
@@ -44,6 +77,18 @@ struct PackWJob {
     int ldw, n_valid, N, KW, P, NL;
     int block0, blocks;
 };
+
+// Dense VJPs on event-row images (zf_img_gemm.cu).
+size_t img_bytes(long long M, int W);
+size_t w_image_bytes(int N, int KW);
+int pack_w_images(cudaStream_t st, const PackWJob* jobs, int n);
+int launch_img_nt(cudaStream_t st, const void* X, int KW, const void* Wimg, int N, const float* G, int ldg, void* out_img,
+                  float* out_f32, int ldo, int n_valid, long long M);
+int launch_img_tn(cudaStream_t st, const void* A, const void* B, int WB, float* C, long long ldca, long long ldcb, int a_valid,
+                  int b_valid, float* colsum, float* arow_sum, int arow_col, long long M);
+
+// In-place all-reduce over the data-parallel ranks of `comm` (zf_dp.cu); op 0 = sum, 1 = min.  A null comm is a no-op.
+int dp_allreduce(cudaStream_t st, void* comm, void* buf, long long n, int is_f64, int op);
 
 // ---- PTX wrappers ----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

@@ -27,8 +27,6 @@ typedef enum { ncclSum = 0, ncclProd = 1, ncclMax = 2, ncclMin = 3 } ncclRedOp_t
 
 namespace zf {
 
-void count_launch();
-
 struct NcclApi {
     void* handle = nullptr;
     ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;

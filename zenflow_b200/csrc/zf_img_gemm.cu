@@ -16,12 +16,8 @@
 #include "zf_umma.cuh"
 
 #include <algorithm>
-#include <map>
-#include <mutex>
 
 namespace zf {
-
-void count_launch();
 
 constexpr int IG_THREADS = 192;   // warps 0-3: epilogue (one thread per accumulator lane), warp 4: producer, warp 5: MMA issuer
 
@@ -352,20 +348,6 @@ __global__ void __launch_bounds__(256) pack_w_images_kernel(const __grid_constan
     }
 }
 
-static int set_smem_once(const void* fn, size_t bytes) {
-    static std::mutex mu;
-    static std::map<std::pair<const void*, int>, size_t> done;
-    int dev = 0;
-    ZF_CUDA_CHECK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(mu);
-    size_t& have = done[{fn, dev}];
-    if (have < bytes) {
-        ZF_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        have = bytes;
-    }
-    return ZF_OK;
-}
-
 size_t img_bytes(long long M, int W) { return (size_t)((M + 127) / 128) * 2 * W * 256; }
 size_t w_image_bytes(int N, int KW) { return (size_t)2 * N * KW * 2; }
 
@@ -393,7 +375,7 @@ int launch_img_nt(cudaStream_t st, const void* X, int KW, const void* Wimg, int 
     DeviceInfo di;
     if (int rc = get_device_info(&di)) return rc;
     const size_t smem = (size_t)NT_STAGES * NT_STAGE_BYTES + 256;
-    if (int rc = set_smem_once((const void*)img_nt_kernel, smem)) return rc;
+    if (int rc = smem_optin((const void*)img_nt_kernel, smem)) return rc;
     ImgNtArgs a{static_cast<const char*>(X), KW, static_cast<const char*>(Wimg), N, G, ldg, static_cast<char*>(out_img), out_f32, ldo, n_valid, M};
     const long long tiles = (M + 127) / 128;
     if (tiles == 0) return ZF_OK;
@@ -409,7 +391,7 @@ int launch_img_tn(cudaStream_t st, const void* A, const void* B, int WB, float* 
     DeviceInfo di;
     if (int rc = get_device_info(&di)) return rc;
     const size_t smem = (size_t)TN_SLOTS * TN_SLOT_BYTES + 4096 + 256;
-    if (int rc = set_smem_once((const void*)img_tn_kernel, smem)) return rc;
+    if (int rc = smem_optin((const void*)img_tn_kernel, smem)) return rc;
     const long long tiles = (M + 127) / 128;
     if (tiles == 0) return ZF_OK;
     const int NS = std::min(TN_NS, WB);

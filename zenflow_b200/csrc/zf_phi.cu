@@ -19,11 +19,6 @@
 
 namespace zf {
 
-void count_launch();
-int launch_umma_gemm(cudaStream_t st, int mode, const float* A, long long lda, const float* B, long long ldb, float* C,
-                     long long ldc, const float* bias, float* colsum, const float* Z, long long ldz, int a_swish,
-                     long long I, long long J, long long R, long long r_slab);
-
 // sums[f] = sum_n x[n][f], sums[F + f] = sum_n x[n][f]^2 (double)
 __global__ void __launch_bounds__(256) phi_moments_kernel(const float* __restrict__ x, long long N, int F, double* sums) {
     extern __shared__ double sh[];

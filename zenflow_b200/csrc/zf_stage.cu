@@ -13,8 +13,6 @@
 
 namespace zf {
 
-void count_launch();
-
 struct StageArgs {
     const float* theta;
     const float* v;
@@ -198,7 +196,7 @@ static int launch_stage(cudaStream_t stream, const float* theta, const float* v,
     if (grid > a.n_tiles) grid = a.n_tiles;
 
     auto run = [&](auto kernel) -> int {
-        ZF_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (int rc = smem_optin((const void*)kernel, smem)) return rc;
         kernel<<<(unsigned)grid, threads, smem, stream>>>(a);
         count_launch();
         ZF_CUDA_CHECK(cudaGetLastError());

@@ -16,9 +16,6 @@
 
 namespace zf {
 
-void count_launch();
-int dp_allreduce(cudaStream_t st, void* comm, void* buf, long long n, int is_f64, int op);
-
 struct StepGroup {
     int kind;                 // ZF_OP_SHIFT_BOUNDS or ZF_OP_COUPLING
     int op_index;

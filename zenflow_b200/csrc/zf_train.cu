@@ -23,8 +23,6 @@
 
 namespace zf {
 
-void count_launch();
-
 // ---------------------------------------------------------------------------------------------
 // ShiftBounds batch min/max
 // ---------------------------------------------------------------------------------------------
@@ -431,16 +429,10 @@ __global__ void __launch_bounds__(256) gemm_kernel(const __grid_constant__ GemmA
     if (MODE == 2 && g.colsum && blockIdx.x == 0 && tid < GT && j0 + tid < g.J) atomicAdd(&g.colsum[j0 + tid], csum);
 }
 
-struct ImplSwitch { char chain[16]; char gemm[16]; };
-ImplSwitch& impl_switch();
-int launch_umma_gemm(cudaStream_t st, int mode, const float* A, long long lda, const float* B, long long ldb, float* C,
-                     long long ldc, const float* bias, float* colsum, const float* Z, long long ldz, int a_swish,
-                     long long I, long long J, long long R, long long r_slab);
-
 static int launch_gemm(cudaStream_t st, int mode, const GemmArgs& g) {
     // tensor-core (tcgen05, 3xTF32) GEMM by default; ZF_GEMM_IMPL=simt, or an activation other than swish,
     // keeps the fp32 FFMA kernel
-    const char* impl = impl_switch().gemm;   // read once per process (zf_chain.cu)
+    const char* impl = impl_switch().gemm;
     if (impl[0] != 's' && g.act == ZF_ACT_SWISH)
         return launch_umma_gemm(st, mode, g.A, g.lda, g.B, g.ldb, g.C, g.ldc, g.bias, g.colsum, g.Z, g.ldz, g.a_swish,
                                 g.I, g.J, g.R, mode == 2 ? 4096 : 0);
@@ -692,6 +684,15 @@ static void fill_cols(const zf_shift_bounds* sb, int D, SbCols& c) {
 
 using namespace zf;
 
+extern "C" int zf_selftest_umma_gemm(void* stream, int32_t mode, const float* A, int64_t lda, const float* B, int64_t ldb,
+                                     float* C, int64_t ldc, const float* bias, float* colsum, const float* Z, int64_t ldz,
+                                     int32_t a_swish, int64_t I, int64_t J, int64_t R, int64_t r_slab) {
+    ZF_REQUIRE(A && B && C && mode >= 0 && mode <= 2 && I >= 1 && J >= 1 && R >= 1, "selftest_umma_gemm: bad argument");
+    ZF_REQUIRE(mode != 2 || (I <= 128 && r_slab >= 32 && r_slab % 32 == 0), "selftest_umma_gemm: mode 2 needs I <= 128 and r_slab % 32 == 0");
+    const GemmArgs g{A, lda, B, ldb, C, ldc, bias, colsum, Z, ldz, a_swish, ZF_ACT_SWISH, I, J, R, r_slab};
+    return launch_gemm((cudaStream_t)stream, mode, g);
+}
+
 extern "C" int zf_shift_bounds_minmax(void* stream, const zf_shift_bounds* sb, const float* x, int64_t M, int32_t D,
                                       float* minmax, void* scratch) {
     ZF_REQUIRE(sb && x && minmax && scratch, "shift_bounds_minmax: null argument");
@@ -763,23 +764,6 @@ extern "C" int zf_flow_loss_grad(void* stream, int32_t latent_kind, float peakne
                                  double* lp_sum) {
     return zf_flow_loss_grad_ct(stream, latent_kind, peakness, z, log_det, M, D, global_count, nullptr, lp, gz, glp, lp_sum);
 }
-
-// tensor-core path: conditioner recompute + spline VJP in one kernel (zf_chain.cu), Dense VJPs on event-row images
-// (zf_img_gemm.cu)
-namespace zf {
-size_t coupling_vjp_ws_floats(const zf_coupling* cp, int D, int C);
-int coupling_vjp_pack(cudaStream_t stream, const zf_coupling* cp, int D, int C, float* ws);
-int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, const float* ws, const float* x_in, const float* c,
-                     const float* gy, int gy_rot, const float* glp, long long M, float* gx, void* img_h0, int wh0, void* const* img_act,
-                     float* const* act_g, void* img_dtheta);
-size_t img_bytes(long long M, int W);
-size_t w_image_bytes(int N, int KW);
-int pack_w_images(cudaStream_t st, const PackWJob* jobs, int n);
-int launch_img_nt(cudaStream_t st, const void* X, int KW, const void* Wimg, int N, const float* G, int ldg, void* out_img,
-                  float* out_f32, int ldo, int n_valid, long long M);
-int launch_img_tn(cudaStream_t st, const void* A, const void* B, int WB, float* C, long long ldca, long long ldcb, int a_valid,
-                  int b_valid, float* colsum, float* arow_sum, int arow_col, long long M);
-}  // namespace zf
 
 // Workspace of zf_coupling_backward.
 // Fused path (hidden width 128, K in {16, 32}: the tensor-core kernels): the cotangent of theta has each dim's 3K-1
@@ -940,7 +924,7 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
     if (sp_stages < 1) return fail(ZF_ERR_UNSUPPORTED, "coupling_backward: spline tile does not fit shared memory");
     const size_t sp_smem = (size_t)sp_stages * tile_bytes + 64;
     auto sp_kernel = (K == 16) ? spline_bwd_kernel<16> : (K == 32) ? spline_bwd_kernel<32> : spline_bwd_kernel<0>;
-    ZF_CUDA_CHECK(cudaFuncSetAttribute(sp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp_smem));
+    if (int rc = smem_optin((const void*)sp_kernel, sp_smem)) return rc;
 
     float* ws = static_cast<float*>(workspace);
     int widths[ZF_MAX_LAYERS + 2];

@@ -20,8 +20,6 @@
 
 namespace zf {
 
-void count_launch();
-
 struct UGemmArgs {
     const float* A; long long lda;
     const float* B; long long ldb;
@@ -62,9 +60,6 @@ template <bool RCONTIG>
 __device__ __forceinline__ float4 ug_load_unit(const float* __restrict__ X, long long ld, long long row, long long row_max,
                                                long long r, long long r_max, bool vec_ok) {
     float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
-#ifdef ZF_GEMM_EXP_NOLOAD   // timing experiment only
-    return make_float4((float)row, (float)r, 1.f, 2.f);
-#endif
     if (row < row_max) {
         if (RCONTIG && vec_ok && r + 3 < r_max) {
             o = __ldg(reinterpret_cast<const float4*>(X + row * ld + r));
@@ -171,13 +166,8 @@ __global__ void __launch_bounds__(UG_THREADS, (TN == 256) ? 1 : 2) umma_gemm_ker
                 umma::split_tf32(v.x, hi.x, lo.x); umma::split_tf32(v.y, hi.y, lo.y);
                 umma::split_tf32(v.z, hi.z, lo.z); umma::split_tf32(v.w, hi.w, lo.w);
                 const int off = (r4 * 16 + (row >> 3)) * 32 + (row & 7) * 4;
-#ifdef ZF_GEMM_EXP_NOSTORE   // timing experiment only
-                if (hi.x == 1234.5f && lo.y == 0.25f)
-#endif
-                {
                 *reinterpret_cast<float4*>(st + off) = hi;
                 *reinterpret_cast<float4*>(st + A_FLOATS + off) = lo;
-                }
             }
 #pragma unroll
             for (int q = 0; q < UB; ++q) {
@@ -189,13 +179,8 @@ __global__ void __launch_bounds__(UG_THREADS, (TN == 256) ? 1 : 2) umma_gemm_ker
                 umma::split_tf32(v.x, hi.x, lo.x); umma::split_tf32(v.y, hi.y, lo.y);
                 umma::split_tf32(v.z, hi.z, lo.z); umma::split_tf32(v.w, hi.w, lo.w);
                 const int off = (r4 * (TN / 8) + (row >> 3)) * 32 + (row & 7) * 4;
-#ifdef ZF_GEMM_EXP_NOSTORE
-                if (hi.x == 1234.5f && lo.y == 0.25f)
-#endif
-                {
                 *reinterpret_cast<float4*>(st + 2 * A_FLOATS + off) = hi;
                 *reinterpret_cast<float4*>(st + 2 * A_FLOATS + B_FLOATS + off) = lo;
-                }
             }
         };
         float4 ra0[UA], rb0[UB], ra1[UA], rb1[UB];
@@ -238,9 +223,6 @@ __global__ void __launch_bounds__(UG_THREADS, (TN == 256) ? 1 : 2) umma_gemm_ker
             umma::ld16(umma::taddr(tb, q * 32, n0), v);
             umma::ld16(umma::taddr(tb, q * 32, TN + n0), w);
             umma::wait_ld();
-#ifdef ZF_GEMM_EXP_NOEPI
-            if (v[0] == 1234.5f)
-#endif
             if (i < g.I) {
                 float x[16];
 #pragma unroll
@@ -641,12 +623,7 @@ static int launch_tma(cudaStream_t st, const UGemmArgs& g, bool* used) {
     dim3 grid((unsigned)((g.I + 127) / 128), (unsigned)((g.J + TN - 1) / TN), 1);
     if (MODE == 2) grid.z = (unsigned)((g.R + g.r_slab - 1) / g.r_slab);
     if (grid.x == 0 || grid.y == 0 || g.R <= 0) { *used = true; return ZF_OK; }
-    static bool attr_done = false;   // per kernel instantiation; the attribute is idempotent, races are harmless
-    if (!attr_done) {
-        ZF_CUDA_CHECK(cudaFuncSetAttribute(umma_gemm_tma_kernel<MODE, TN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)TgCfg<TN>::SMEM));
-        attr_done = true;
-    }
+    if (int rc = smem_optin((const void*)umma_gemm_tma_kernel<MODE, TN>, TgCfg<TN>::SMEM)) return rc;
     umma_gemm_tma_kernel<MODE, TN><<<grid, TG_THREADS, TgCfg<TN>::SMEM, st>>>(ta);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
@@ -661,15 +638,13 @@ static int launch_one(cudaStream_t st, const UGemmArgs& g) {
     dim3 grid((unsigned)((g.I + 127) / 128), (unsigned)((g.J + TN - 1) / TN), 1);
     if (MODE == 2) grid.z = (unsigned)((g.R + g.r_slab - 1) / g.r_slab);
     if (grid.x == 0 || grid.y == 0 || g.R <= 0) return ZF_OK;
-    ZF_CUDA_CHECK(cudaFuncSetAttribute(umma_gemm_kernel<MODE, TN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = smem_optin((const void*)umma_gemm_kernel<MODE, TN>, smem)) return rc;
     umma_gemm_kernel<MODE, TN><<<grid, UG_THREADS, smem, st>>>(g);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;
 }
 
-struct ImplSwitch { char chain[16]; char gemm[16]; };
-ImplSwitch& impl_switch();
 // developer switch "legacy": the register-path loaders for every shape (zf_debug_set_impl)
 static bool gemm_force_legacy() { return impl_switch().gemm[0] == 'l'; }
 
@@ -702,11 +677,3 @@ int launch_umma_gemm(cudaStream_t st, int mode, const float* A, long long lda, c
 }
 
 }  // namespace zf
-
-extern "C" int zf_selftest_umma_gemm(void* stream, int32_t mode, const float* A, int64_t lda, const float* B, int64_t ldb,
-                                     float* C, int64_t ldc, const float* bias, float* colsum, const float* Z, int64_t ldz,
-                                     int32_t a_swish, int64_t I, int64_t J, int64_t R, int64_t r_slab) {
-    ZF_REQUIRE(A && B && C && mode >= 0 && mode <= 2 && I >= 1 && J >= 1 && R >= 1, "selftest_umma_gemm: bad argument");
-    ZF_REQUIRE(mode != 2 || (I <= 128 && r_slab >= 32 && r_slab % 32 == 0), "selftest_umma_gemm: mode 2 needs I <= 128 and r_slab % 32 == 0");
-    return zf::launch_umma_gemm((cudaStream_t)stream, mode, A, lda, B, ldb, C, ldc, bias, colsum, Z, ldz, a_swish, I, J, R, r_slab);
-}

@@ -3,7 +3,6 @@
 #include "zf_umma.cuh"
 
 namespace zf {
-void count_launch();
 
 __global__ void __launch_bounds__(160) umma_selftest_kernel(const float* __restrict__ A, const float* __restrict__ B,
                                                             int N, int K, float* __restrict__ out, int mask_mode) {
@@ -233,7 +232,7 @@ extern "C" int zf_selftest_umma_bf16(void* stream, const float* A, const float* 
     ZF_REQUIRE(A && B && out, "selftest_umma_bf16: null argument");
     ZF_REQUIRE(N >= 16 && N <= 128 && N % 16 == 0 && K >= 16 && K <= 128 && K % 16 == 0, "selftest_umma_bf16: bad N/K");
     const size_t smem = (size_t)2 * (128 + N) * K * sizeof(uint16_t);
-    ZF_CUDA_CHECK(cudaFuncSetAttribute(zf::umma_selftest_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = zf::smem_optin((const void*)zf::umma_selftest_bf16_kernel, smem)) return rc;
     zf::umma_selftest_bf16_kernel<<<1, 160, smem, (cudaStream_t)stream>>>(A, B, N, K, out, flags);
     zf::count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
@@ -245,7 +244,7 @@ extern "C" int zf_selftest_umma_f16(void* stream, const float* A, const float* B
     ZF_REQUIRE(A && B && out, "selftest_umma_f16: null argument");
     ZF_REQUIRE(N >= 16 && N <= 128 && N % 16 == 0 && K >= 16 && K <= 128 && K % 16 == 0, "selftest_umma_f16: bad N/K");
     const size_t smem = (size_t)2 * N * K * sizeof(__half);
-    ZF_CUDA_CHECK(cudaFuncSetAttribute(zf::umma_selftest_f16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = zf::smem_optin((const void*)zf::umma_selftest_f16_kernel, smem)) return rc;
     zf::umma_selftest_f16_kernel<<<1, 160, smem, (cudaStream_t)stream>>>(A, B, N, K, out, variant);
     zf::count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
@@ -257,7 +256,7 @@ extern "C" int zf_selftest_umma(void* stream, const float* A, const float* B, in
     ZF_REQUIRE(A && B && out, "selftest_umma: null argument");
     ZF_REQUIRE(N >= 16 && N <= 128 && N % 16 == 0 && K >= 8 && K <= 128 && K % 8 == 0, "selftest_umma: bad N/K");
     const size_t smem = (size_t)2 * N * K * sizeof(float);
-    ZF_CUDA_CHECK(cudaFuncSetAttribute(zf::umma_selftest_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = zf::smem_optin((const void*)zf::umma_selftest_kernel, smem)) return rc;
     zf::umma_selftest_kernel<<<1, 160, smem, (cudaStream_t)stream>>>(A, B, N, K, out, mask_mode);
     zf::count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
@@ -342,11 +341,11 @@ __global__ void __launch_bounds__(192) umma_rate_kernel(int N, int reps, int mod
 }  // namespace zf
 
 extern "C" int zf_debug_umma_rate(int32_t N, int32_t reps, int32_t mode, int32_t ctas, long long* host_out) {
+    const size_t smem = (size_t)2 * N * 32 * sizeof(float);
+    if (zf::smem_optin((const void*)zf::umma_rate_kernel, smem)) return 1;
     long long* d = nullptr;
     if (cudaMalloc(&d, 4 * sizeof(long long)) != cudaSuccess) return 1;
     cudaMemset(d, 0, 4 * sizeof(long long));
-    const size_t smem = (size_t)2 * N * 32 * sizeof(float);
-    cudaFuncSetAttribute(zf::umma_rate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     zf::umma_rate_kernel<<<ctas, 192, smem>>>(N, reps, mode, d);
     const int rc = (int)cudaDeviceSynchronize();
     cudaMemcpy(host_out, d, 4 * sizeof(long long), cudaMemcpyDeviceToHost);

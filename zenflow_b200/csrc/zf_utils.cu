@@ -11,8 +11,6 @@
 
 namespace zf {
 
-void count_launch();
-
 __global__ void __launch_bounds__(256) squareplus_kernel(const float* __restrict__ x, long long n, float* __restrict__ y) {
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
         y[i] = squareplus_rn(x[i]);
