@@ -150,7 +150,8 @@ int zf_rqs_inverse_normalized(void* stream, const float* y, const float* dx, con
 
 /* Developer switch (parity tests): force a chain kernel ("simt", "umma", "umma8"; NULL / "" = automatic) and a train
  * GEMM ("simt" = the fp32 FFMA GEMM; "legacy" = the tcgen05 GEMM with register-path loaders for every shape; NULL / "" =
- * tcgen05, fed by the copy engine where the operands allow tensor maps).  The ZF_CHAIN_IMPL / ZF_GEMM_IMPL environment
+ * tcgen05, fed by the copy engine where the operands allow tensor maps).  The GEMM switch applies to every Dense layer
+ * the fused VJP kernel does not take, and to the Deep-Set Phi's.  The ZF_CHAIN_IMPL / ZF_GEMM_IMPL environment
  * variables give the initial values and are read once per process. */
 int zf_debug_set_impl(const char* chain_impl, const char* gemm_impl);
 

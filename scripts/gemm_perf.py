@@ -1,4 +1,6 @@
-"""Developer timing of the train step's tcgen05 GEMMs (zf_selftest_umma_gemm) at the conditioner's shapes."""
+"""Developer timing of the train step's GEMMs (zf_selftest_umma_gemm -> launch_gemm) at the conditioner's shapes.
+   python scripts/gemm_perf.py [legacy|simt]: no argument times the default choice (tcgen05, fed by the copy engine where
+   the operands allow), 'legacy' the tcgen05 GEMM with register-path loaders, 'simt' the fp32 FFMA GEMM."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -8,7 +10,7 @@ if os.environ.get("ZF_LIB"):
 from zenflow_b200 import _lib
 lib = _lib.load()
 if len(sys.argv) > 1:
-    _lib.set_impl(None, sys.argv[1])   # 'legacy': register-path loaders
+    _lib.set_impl(None, sys.argv[1])
 M = 262144
 dev = "cuda"
 def t(fn, n=5):

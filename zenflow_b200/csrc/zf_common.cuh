@@ -46,7 +46,8 @@ void count_launch();
 // Developer switches, for tests and measurements that compare implementations (zf_chain.cu):
 //   chain  "" automatic | "simt" FFMA chain_kernel | "umma" tensor-core kernel or an error | "umma8" single-tile
 //          tensor-core kernel for single-dim flows too (choose_chain_kernel)
-//   gemm   "" automatic | "simt" FFMA gemm_kernel | "legacy" tcgen05 GEMM with register-path loaders (launch_gemm)
+//   gemm   "" automatic | "simt" FFMA gemm_kernel | "legacy" tcgen05 GEMM with register-path loaders, for every train
+//          GEMM: the unfused coupling backward and the Deep-Set Phi (launch_gemm)
 // The environment (ZF_CHAIN_IMPL, ZF_GEMM_IMPL) is read once per process; zf_debug_set_impl overrides it afterwards.
 struct ImplSwitch {
     char chain[16];
@@ -56,10 +57,21 @@ ImplSwitch& impl_switch();
 
 // ---- entry points shared between translation units -------------------------------------
 
-// tcgen05 GEMM family of the train step (zf_umma_gemm.cu); same argument convention as the FFMA gemm of zf_train.cu.
-int launch_umma_gemm(cudaStream_t st, int mode, const float* A, long long lda, const float* B, long long ldb, float* C,
-                     long long ldc, const float* bias, float* colsum, const float* Z, long long ldz, int a_swish,
-                     long long I, long long J, long long R, long long r_slab);
+// One product of the train step's fp32 GEMM family (zf_gemm.cu; the modes are described there).
+struct GemmArgs {
+    const float* A; long long lda;
+    const float* B; long long ldb;
+    float* C; long long ldc;
+    const float* bias;
+    float* colsum;
+    const float* Z; long long ldz;
+    int a_swish;         // apply the activation to A on load
+    int act;             // zf_act_kind (0 = swish) of opA and of the derivative that multiplies mode 1's product
+    long long I, J, R;   // output rows, output cols, reduction length
+    long long r_slab;    // mode 2, FFMA kernel only: reduction rows per CTA; the tcgen05 kernels choose their own slabs
+};
+// Runs one product; the only place that chooses between the three GEMM kernels (the table is at its definition).
+int launch_gemm(cudaStream_t st, int mode, const GemmArgs& g);
 
 // Fused conditioner recompute + spline VJP of one coupling (zf_chain.cu).  ws_floats is 0 when the coupling or the
 // device does not take the fused kernel.

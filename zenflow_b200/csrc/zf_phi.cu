@@ -8,7 +8,7 @@
 //   zf_phi_forward   c (S, out) from x (N, in); train mode uses batch moments, updates the running statistics and
 //                    keeps the layer pre-activations in the workspace for zf_phi_backward
 //   zf_phi_backward  parameter cotangents (+=) from gc (S, out) = d loss / d c (what zf_flow_value_and_grad returns)
-// The Dense layers run on the train step's tcgen05 GEMM family (zf_umma_gemm.cu); BatchNorm, dropout and the pooling
+// The Dense layers run on the train step's GEMM family (launch_gemm, zf_gemm.cu); BatchNorm, dropout and the pooling
 // are small SIMT kernels.  Dropout draws its keep-mask from Philox keyed by (seed, row, column) (jax's threefry
 // stream cannot be reproduced without JAX) or takes an explicit multiplier matrix (parity tests).
 #include "zf_common.cuh"
@@ -200,10 +200,14 @@ extern "C" int zf_phi_forward(void* stream, const zf_phi* phi, const float* x, i
     count_launch();
     for (int l = 0; l <= L; ++l) {   // Z_{l+1} = act(Z_l) W_l + b_l (pre-activations are kept)
         ZF_REQUIRE(phi->kernel[l] && phi->bias[l], "phi_forward: Dense_%d leaf is NULL", l);
-        if (int rc = launch_umma_gemm(st, 0, ws + p.off_act[l], p.widths[l], phi->kernel[l], p.widths[l + 1],
-                                      ws + p.off_act[l + 1], p.widths[l + 1], phi->bias[l], nullptr, nullptr, 0, l > 0, N,
-                                      p.widths[l + 1], p.widths[l], 0))
-            return rc;
+        GemmArgs g{};
+        g.A = ws + p.off_act[l]; g.lda = p.widths[l];
+        g.B = phi->kernel[l]; g.ldb = p.widths[l + 1];
+        g.C = ws + p.off_act[l + 1]; g.ldc = p.widths[l + 1];
+        g.bias = phi->bias[l];
+        g.a_swish = l > 0;
+        g.I = N; g.J = p.widths[l + 1]; g.R = p.widths[l];
+        if (int rc = launch_gemm(st, 0, g)) return rc;
     }
     ZF_CUDA_CHECK(cudaMemsetAsync(c_out, 0, (size_t)S * O * sizeof(float), st));
     if (nnz > 0) {
@@ -241,16 +245,21 @@ extern "C" int zf_phi_backward(void* stream, const zf_phi* phi, const zf_couplin
     }
     for (int l = L; l >= 0; --l) {
         ZF_REQUIRE(grads->kernel[l] && grads->bias[l], "phi_backward: Dense_%d gradient leaf is NULL", l);
-        // dW_l += act(Z_l)^T dZ_{l+1}, db_l += colsum(dZ_{l+1})
-        if (int rc = launch_umma_gemm(st, 2, ws + p.off_act[l], p.widths[l], gcur, p.widths[l + 1], grads->kernel[l],
-                                      p.widths[l + 1], nullptr, grads->bias[l], nullptr, 0, l > 0, p.widths[l], p.widths[l + 1],
-                                      N, 2048))
-            return rc;
-        // dZ_l = (dZ_{l+1} W_l^T) * swish'(Z_l)   (l = 0: d/d(BatchNorm output), no activation)
-        if (int rc = launch_umma_gemm(st, 1, gcur, p.widths[l + 1], phi->kernel[l], p.widths[l + 1], gnext, p.widths[l], nullptr,
-                                      nullptr, l == 0 ? nullptr : ws + p.off_act[l], p.widths[l], 0, N, p.widths[l],
-                                      p.widths[l + 1], 0))
-            return rc;
+        GemmArgs gw{};  // dW_l += act(Z_l)^T dZ_{l+1}, db_l += colsum(dZ_{l+1})
+        gw.A = ws + p.off_act[l]; gw.lda = p.widths[l];
+        gw.B = gcur; gw.ldb = p.widths[l + 1];
+        gw.C = grads->kernel[l]; gw.ldc = p.widths[l + 1];
+        gw.colsum = grads->bias[l];
+        gw.a_swish = l > 0;
+        gw.I = p.widths[l]; gw.J = p.widths[l + 1]; gw.R = N; gw.r_slab = 2048;
+        if (int rc = launch_gemm(st, 2, gw)) return rc;
+        GemmArgs ga{};  // dZ_l = (dZ_{l+1} W_l^T) * swish'(Z_l)   (l = 0: d/d(BatchNorm output), no activation)
+        ga.A = gcur; ga.lda = p.widths[l + 1];
+        ga.B = phi->kernel[l]; ga.ldb = p.widths[l + 1];
+        ga.C = gnext; ga.ldc = p.widths[l];
+        ga.Z = (l == 0) ? nullptr : ws + p.off_act[l]; ga.ldz = p.widths[l];
+        ga.I = N; ga.J = p.widths[l]; ga.R = p.widths[l + 1];
+        if (int rc = launch_gemm(st, 1, ga)) return rc;
         std::swap(gcur, gnext);
     }
     // BatchNorm parameters (train-mode statistics of the matching forward are still in the workspace)

@@ -306,148 +306,6 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
 }
 
 // ---------------------------------------------------------------------------------------------
-// generic fp32 GEMM family for the conditioner recompute / backward (64x64x16 tiles, 4x4 per thread)
-//   mode 0 (NN): C[m][n]  = sum_k opA(A[m][k]) * B[k][n] + bias[n]
-//   mode 1 (NT): C[m][k]  = (sum_n A[m][n] * B[k][n]) * swish'(Z[m][k])          (Z optional)
-//   mode 2 (TN): C[k][n] += sum_m opA(A[m][k]) * B[m][n];  colsum[n] += sum_m B[m][n]
-// opA = the activation `act` (swish by default) when a_swish: stored pre-activations are re-activated on load.
-// ---------------------------------------------------------------------------------------------
-struct GemmArgs {
-    const float* A; long long lda;
-    const float* B; long long ldb;
-    float* C; long long ldc;
-    const float* bias;
-    float* colsum;
-    const float* Z; long long ldz;
-    int a_swish;         // apply the activation to A on load
-    int act;             // zf_act_kind (0 = swish) of opA and of the derivative that multiplies mode 1's product
-    long long I, J, R;   // output rows, output cols, reduction length
-    long long r_slab;    // mode 2: reduction rows per CTA (gridDim.z slabs)
-};
-
-constexpr int GT = 64, GK = 16, GS = 68;
-
-
-// pattern T: S[r][t] = X[(t0+t)*ld + r0+r]   (r contiguous in memory)
-__device__ __forceinline__ void load_T(float (*S)[GS], const float* __restrict__ X, long long ld, long long t0,
-                                       long long tmax, long long r0, long long rmax, int act, int tid) {
-#pragma unroll
-    for (int q = 0; q < (GT * GK) / 256; ++q) {
-        const int e = tid + q * 256;
-        const int r = e % GK, t = e / GK;
-        float v = 0.f;
-        if (t0 + t < tmax && r0 + r < rmax) {
-            v = X[(t0 + t) * ld + r0 + r];
-            if (act >= 0) v = act_apply(act, v);
-        }
-        S[r][t] = v;
-    }
-}
-// pattern D: S[r][t] = X[(r0+r)*ld + t0+t]   (t contiguous in memory)
-__device__ __forceinline__ void load_D(float (*S)[GS], const float* __restrict__ X, long long ld, long long t0,
-                                       long long tmax, long long r0, long long rmax, int act, int tid) {
-#pragma unroll
-    for (int q = 0; q < (GT * GK) / 256; ++q) {
-        const int e = tid + q * 256;
-        const int t = e % GT, r = e / GT;
-        float v = 0.f;
-        if (t0 + t < tmax && r0 + r < rmax) {
-            v = X[(r0 + r) * ld + t0 + t];
-            if (act >= 0) v = act_apply(act, v);
-        }
-        S[r][t] = v;
-    }
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(256) gemm_kernel(const __grid_constant__ GemmArgs g) {
-    __shared__ __align__(16) float As[GK][GS];
-    __shared__ __align__(16) float Bs[GK][GS];
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const long long i0 = (long long)blockIdx.x * GT, j0 = (long long)blockIdx.y * GT;
-    long long rbeg = 0, rend = g.R;
-    if (MODE == 2) {
-        rbeg = (long long)blockIdx.z * g.r_slab;
-        rend = rbeg + g.r_slab < g.R ? rbeg + g.r_slab : g.R;
-    }
-    float acc[4][4];
-#pragma unroll
-    for (int a = 0; a < 4; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
-    float csum = 0.f;
-
-    for (long long r0 = rbeg; r0 < rend; r0 += GK) {
-        if (MODE == 0) {
-            load_T(As, g.A, g.lda, i0, g.I, r0, rend, g.a_swish ? g.act : -1, tid);
-            load_D(Bs, g.B, g.ldb, j0, g.J, r0, rend, -1, tid);
-        } else if (MODE == 1) {
-            load_T(As, g.A, g.lda, i0, g.I, r0, rend, -1, tid);
-            load_T(Bs, g.B, g.ldb, j0, g.J, r0, rend, -1, tid);
-        } else {
-            load_D(As, g.A, g.lda, i0, g.I, r0, rend, g.a_swish ? g.act : -1, tid);
-            load_D(Bs, g.B, g.ldb, j0, g.J, r0, rend, -1, tid);
-        }
-        __syncthreads();
-        if (MODE == 2 && g.colsum && blockIdx.x == 0 && tid < GT) {
-#pragma unroll
-            for (int r = 0; r < GK; ++r) csum += Bs[r][tid];
-        }
-#pragma unroll
-        for (int r = 0; r < GK; ++r) {
-            const float4 a = *reinterpret_cast<const float4*>(&As[r][tx * 4]);
-            const float4 b = *reinterpret_cast<const float4*>(&Bs[r][ty * 4]);
-            const float a_[4] = {a.x, a.y, a.z, a.w}, b_[4] = {b.x, b.y, b.z, b.w};
-#pragma unroll
-            for (int p = 0; p < 4; ++p)
-#pragma unroll
-                for (int q = 0; q < 4; ++q) acc[p][q] = fmaf(a_[p], b_[q], acc[p][q]);
-        }
-        __syncthreads();
-    }
-
-#pragma unroll
-    for (int p = 0; p < 4; ++p) {
-        const long long i = i0 + tx * 4 + p;
-        if (i >= g.I) continue;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const long long j = j0 + ty * 4 + q;
-            if (j >= g.J) continue;
-            float v = acc[p][q];
-            if (MODE == 0) {
-                if (g.bias) v += g.bias[j];
-                g.C[i * g.ldc + j] = v;
-            } else if (MODE == 1) {
-                if (g.Z) v *= act_grad(g.act, g.Z[i * g.ldz + j]);
-                g.C[i * g.ldc + j] = v;
-            } else {
-                atomicAdd(&g.C[i * g.ldc + j], v);
-            }
-        }
-    }
-    if (MODE == 2 && g.colsum && blockIdx.x == 0 && tid < GT && j0 + tid < g.J) atomicAdd(&g.colsum[j0 + tid], csum);
-}
-
-static int launch_gemm(cudaStream_t st, int mode, const GemmArgs& g) {
-    // tensor-core (tcgen05, 3xTF32) GEMM by default; ZF_GEMM_IMPL=simt, or an activation other than swish,
-    // keeps the fp32 FFMA kernel
-    const char* impl = impl_switch().gemm;
-    if (impl[0] != 's' && g.act == ZF_ACT_SWISH)
-        return launch_umma_gemm(st, mode, g.A, g.lda, g.B, g.ldb, g.C, g.ldc, g.bias, g.colsum, g.Z, g.ldz, g.a_swish,
-                                g.I, g.J, g.R, mode == 2 ? 4096 : 0);
-    dim3 grid((unsigned)((g.I + GT - 1) / GT), (unsigned)((g.J + GT - 1) / GT), 1);
-    if (mode == 2) grid.z = (unsigned)((g.R + g.r_slab - 1) / g.r_slab);
-    if (grid.x == 0 || grid.y == 0) return ZF_OK;
-    if (mode == 0) gemm_kernel<0><<<grid, 256, 0, st>>>(g);
-    else if (mode == 1) gemm_kernel<1><<<grid, 256, 0, st>>>(g);
-    else gemm_kernel<2><<<grid, 256, 0, st>>>(g);
-    count_launch();
-    ZF_CUDA_CHECK(cudaGetLastError());
-    return ZF_OK;
-}
-
-// ---------------------------------------------------------------------------------------------
 // spline VJP: theta row -> d(theta) row in place; d/dx of the transformed columns; pass-through
 // of the conditioning columns' cotangent
 // ---------------------------------------------------------------------------------------------
@@ -683,15 +541,6 @@ static void fill_cols(const zf_shift_bounds* sb, int D, SbCols& c) {
 }  // namespace zf
 
 using namespace zf;
-
-extern "C" int zf_selftest_umma_gemm(void* stream, int32_t mode, const float* A, int64_t lda, const float* B, int64_t ldb,
-                                     float* C, int64_t ldc, const float* bias, float* colsum, const float* Z, int64_t ldz,
-                                     int32_t a_swish, int64_t I, int64_t J, int64_t R, int64_t r_slab) {
-    ZF_REQUIRE(A && B && C && mode >= 0 && mode <= 2 && I >= 1 && J >= 1 && R >= 1, "selftest_umma_gemm: bad argument");
-    ZF_REQUIRE(mode != 2 || (I <= 128 && r_slab >= 32 && r_slab % 32 == 0), "selftest_umma_gemm: mode 2 needs I <= 128 and r_slab % 32 == 0");
-    const GemmArgs g{A, lda, B, ldb, C, ldc, bias, colsum, Z, ldz, a_swish, ZF_ACT_SWISH, I, J, R, r_slab};
-    return launch_gemm((cudaStream_t)stream, mode, g);
-}
 
 extern "C" int zf_shift_bounds_minmax(void* stream, const zf_shift_bounds* sb, const float* x, int64_t M, int32_t D,
                                       float* minmax, void* scratch) {
