@@ -139,6 +139,23 @@ ffi::Error BindGradients(ffi::RemainingRets rets, int first_ret, ChainStorage* c
     return ffi::Error::Success();
 }
 
+// The entries accumulate into the gradient buffers: start them from zero.
+void ZeroGradients(const ChainStorage& cs, int D, int C, cudaStream_t stream) {
+    const int F = D - D / 2 + C, d = D / 2;
+    for (size_t k = 0; k < cs.grads.size(); ++k) {
+        const zf_coupling& cp = cs.couplings[k];
+        cudaMemsetAsync(cs.grads[k].bn_scale, 0, sizeof(float) * F, stream);
+        cudaMemsetAsync(cs.grads[k].bn_bias, 0, sizeof(float) * F, stream);
+        int fan_in = F;
+        for (int l = 0; l <= cp.n_hidden; ++l) {
+            const int out = l < cp.n_hidden ? cp.hidden[l] : d * (3 * cp.knots - 1);
+            cudaMemsetAsync(cs.grads[k].kernel[l], 0, sizeof(float) * (size_t)fan_in * out, stream);
+            cudaMemsetAsync(cs.grads[k].bias[l], 0, sizeof(float) * out, stream);
+            fan_in = out;
+        }
+    }
+}
+
 struct Shapes { int64_t M; int D, C; };
 ffi::Error ReadShapes(const F32& x, int32_t cdim, ffi::RemainingArgs leaves, Shapes* s, const float** c) {
     if (x.dimensions().size() != 2) return Invalid("x must be (M, D)");
@@ -230,19 +247,7 @@ ffi::Error TrainImpl(cudaStream_t stream, ffi::ScratchAllocator scratch, F32 x, 
             if (!g.has_value()) return Invalid("result gc missing");
             gc = g.value()->typed_data();
         }
-        for (size_t k = 0; k < cs.grads.size(); ++k) {   // the entry accumulates: start from zero
-            const zf_coupling& cp = cs.couplings[k];
-            const int F = s.D - s.D / 2 + s.C, d = s.D / 2;
-            cudaMemsetAsync(cs.grads[k].bn_scale, 0, sizeof(float) * F, stream);
-            cudaMemsetAsync(cs.grads[k].bn_bias, 0, sizeof(float) * F, stream);
-            int fan_in = F;
-            for (int l = 0; l <= cp.n_hidden; ++l) {
-                const int out = l < cp.n_hidden ? cp.hidden[l] : d * (3 * cp.knots - 1);
-                cudaMemsetAsync(cs.grads[k].kernel[l], 0, sizeof(float) * (size_t)fan_in * out, stream);
-                cudaMemsetAsync(cs.grads[k].bias[l], 0, sizeof(float) * out, stream);
-                fan_in = out;
-            }
-        }
+        ZeroGradients(cs, s.D, s.C, stream);
     }
     cudaMemsetAsync(lp_sum.value()->typed_data(), 0, sizeof(double), stream);
     const size_t bytes = zf_flow_value_and_grad_workspace_bytes(&cs.chain, s.M, micro_batch);
@@ -255,6 +260,40 @@ ffi::Error TrainImpl(cudaStream_t stream, ffi::ScratchAllocator scratch, F32 x, 
                                              x.typed_data(), c, s.M, global_count, ct, lp.value()->typed_data(),
                                              lp_sum.value()->typed_data(), gc, nullptr, nullptr, nullptr, nullptr, *ws, bytes,
                                              micro_batch));
+}
+
+// ---- jax.grad of Flow.__call__(x, c, train=False), flow.py:22-48: the backward rule of flow_log_prob ------------
+// Operands: x [, c], the cotangent of lp (M,), the leaves.  Results: gx (M, D) [, gc (M, C)], then one cotangent per
+// trainable leaf in op order.  The running statistics are read, never written (they get zero cotangents on the
+// Python side).
+ffi::Error LogProbVjpImpl(cudaStream_t stream, ffi::ScratchAllocator scratch, F32 x, ffi::RemainingArgs rest,
+                          ffi::RemainingRets rets, ffi::Span<const int32_t> program, ffi::Span<const double> bounds,
+                          double margin, int32_t cdim, int32_t latent, float peakness, int64_t micro_batch) {
+    Shapes s;
+    const float* c;
+    if (auto e = ReadShapes(x, cdim, rest, &s, &c); e.failure()) return e;
+    int first = cdim > 0 ? 1 : 0;
+    auto ctb = rest.get<F32>(first++);
+    if (!ctb.has_value()) return Invalid("log_prob_vjp: cotangent of lp missing");
+    ChainStorage cs;
+    if (auto e = BuildChainFromLeaves(program, bounds, margin, s.D, s.C, rest, first, &cs); e.failure()) return e;
+    auto gx = rets.get<F32>(0);
+    if (!gx.has_value()) return Invalid("result gx missing");
+    float* gc = nullptr;
+    if (cdim > 0) {
+        auto g = rets.get<F32>(1);
+        if (!g.has_value()) return Invalid("result gc missing");
+        gc = g.value()->typed_data();
+    }
+    if (auto e = BindGradients(rets, cdim > 0 ? 2 : 1, &cs); e.failure()) return e;
+    ZeroGradients(cs, s.D, s.C, stream);
+    const size_t bytes = zf_flow_log_prob_vjp_workspace_bytes(&cs.chain, s.M, micro_batch);
+    if (bytes == 0) return FromStatus(ZF_ERR_INVALID);
+    auto ws = scratch.Allocate(bytes, 256);
+    if (!ws.has_value()) return ffi::Error(ffi::ErrorCode::kResourceExhausted, "zenflow_b200: scratch allocation failed");
+    return FromStatus(zf_flow_log_prob_vjp(stream, &cs.chain, cs.grads.empty() ? nullptr : cs.grads.data(), latent, peakness,
+                                           x.typed_data(), c, s.M, ctb.value().typed_data(), nullptr,
+                                           gx.value()->typed_data(), gc, *ws, bytes, micro_batch));
 }
 
 // ---- optimizer.update + optax.apply_updates on the flattened pytree, train.py:84-85 ------------------------------
@@ -314,6 +353,17 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfFlowTrain, TrainImpl,
                                   .Attr<float>("peakness")
                                   .Attr<double>("global_count")
                                   .Attr<int32_t>("with_grads")
+                                  .Attr<int64_t>("micro_batch"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfFlowLogProbVjp, LogProbVjpImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Ctx<ffi::ScratchAllocator>()
+                                  .Arg<F32>()
+                                  .RemainingArgs()
+                                  .RemainingRets() ZF_CHAIN_ATTRS()
+                                  .Attr<int32_t>("latent")
+                                  .Attr<float>("peakness")
                                   .Attr<int64_t>("micro_batch"));
 
 XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfNadamwUpdate, NadamwImpl,

@@ -8,7 +8,8 @@ of the reference's modules; everything that touches jax is imported lazily insid
 Calling convention = the header comment of ffi/zenflow_b200_xla.cc.
 
 reference call site                                   -> handler
-  Flow.__call__(x, c, train=False)   flow.py:45-47    -> ZfFlowLogProb      (flow_log_prob)
+  Flow.__call__(x, c, train=False)   flow.py:45-47    -> ZfFlowLogProb      (flow_log_prob, a jax.custom_vjp)
+  jax.grad of it (wrt x, c, params)                   -> ZfFlowLogProbVjp   (its backward rule)
   Chain.inverse(z, c)         bijectors.py:113-116    -> ZfChainInverse     (chain_inverse)
   Flow.sample                        flow.py:50-78    -> ZfFlowSample       (flow_sample; Philox mode) or
                                                          latent.sample (jax.random) + chain_inverse (parity mode)
@@ -31,6 +32,7 @@ LATENT = {"Beta": 0, "Normal": 1, "TruncatedNormal": 2, "Uniform": 3}
 
 _TARGETS = {
     "zf_flow_log_prob": "ZfFlowLogProb",
+    "zf_flow_log_prob_vjp": "ZfFlowLogProbVjp",
     "zf_chain_inverse": "ZfChainInverse",
     "zf_flow_sample": "ZfFlowSample",
     "zf_flow_train": "ZfFlowTrain",
@@ -192,15 +194,44 @@ def _latent(flow):
     return dict(latent=np.int32(LATENT[type(lat).__name__]), peakness=np.float32(getattr(lat, "peakness", 12.0)))
 
 
-def flow_log_prob(flow, variables, x, c=None):
-    """Flow.__call__(x, c, train=False), flow.py:45-47: one fused launch (chain + latent + nan_to_num)."""
+def flow_log_prob(flow, variables, x, c=None, *, micro_batch: int = 1 << 18):
+    """Flow.__call__(x, c, train=False), flow.py:45-47: one fused launch (chain + latent + nan_to_num).
+
+    A jax.custom_vjp: jax.grad wrt x, c and the params leaves runs ZfFlowLogProbVjp (one zf_flow_log_prob_vjp call,
+    the conditioner recomputed in micro-batches of ``micro_batch`` events) with the running statistics held fixed;
+    the statistics leaves get zero cotangents, as in make_flow_log_prob_train."""
     import jax
     import jax.numpy as jnp
+    import numpy as np
 
     register()
-    head, leaves, _, _, attrs = _operands(flow, variables, x, c)
-    call = jax.ffi.ffi_call("zf_flow_log_prob", jax.ShapeDtypeStruct((x.shape[0],), jnp.float32))
-    return call(*head, *leaves, **attrs, **_latent(flow))
+    _, leaves, is_stat, _, attrs = _operands(flow, variables, x, c)
+    latent = _latent(flow)
+
+    def _head(x, c):
+        return [x] if c is None else [x, c]
+
+    @jax.custom_vjp
+    def f(x, c, leaves):
+        call = jax.ffi.ffi_call("zf_flow_log_prob", jax.ShapeDtypeStruct((x.shape[0],), jnp.float32))
+        return call(*_head(x, c), *leaves, **attrs, **latent)
+
+    def f_fwd(x, c, leaves):
+        return f(x, c, leaves), (x, c, leaves)
+
+    def f_bwd(saved, ct_lp):
+        x, c, leaves = saved
+        outs = [jax.ShapeDtypeStruct(v.shape, jnp.float32) for v in _head(x, c)]
+        outs += [jax.ShapeDtypeStruct(v.shape, jnp.float32) for v, s in zip(leaves, is_stat) if not s]
+        call = jax.ffi.ffi_call("zf_flow_log_prob_vjp", outs)
+        res = call(*_head(x, c), ct_lp, *leaves, **attrs, **latent, micro_batch=np.int64(micro_batch))
+        n_in = len(_head(x, c))
+        gp = iter(res[n_in:])
+        gl = [jnp.zeros_like(v) if s else next(gp) for v, s in zip(leaves, is_stat)]
+        return res[0], (res[1] if c is not None else None), gl
+
+    f.defvjp(f_fwd, f_bwd)
+    return f(x, c, list(leaves))
 
 
 def chain_inverse(flow, variables, z, c=None):

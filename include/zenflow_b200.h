@@ -274,10 +274,11 @@ int zf_flow_loss_grad_ct(void* stream, int32_t latent_kind, float peakness, cons
  * input path: recomputes the conditioner in micro-batches, then
  *   gx (M,D)   = d/dx_in through the spline (transformed columns) and the pass-through columns,
  *   gh0 (M,F)  = d/d(BatchNorm output),
- *   grads      += d/d(Dense kernels and biases),
- *   bn_sums[0..F) = sum gh0, [F..2F) = sum gh0*xhat  (for BatchNorm's own VJP).
- * cp->bn_mean/bn_var must hold the BATCH statistics used in the forward.  gy is the cotangent of
- * the coupling output; its column j is read at (j + gy_rot) % D (folds the following Rolls). */
+ *   grads      += d/d(Dense kernels and biases)   (NULL: skipped, only the products toward the inputs run),
+ *   bn_sums[0..F) = sum gh0, [F..2F) = sum gh0*xhat  (for BatchNorm's own VJP; NULL: skipped).
+ * cp->bn_mean/bn_var must hold the statistics used in the forward (the BATCH statistics in train
+ * mode, the running ones in eval mode).  gy is the cotangent of the coupling output; its column j
+ * is read at (j + gy_rot) % D (folds the following Rolls). */
 size_t zf_coupling_backward_workspace_bytes(const zf_coupling* cp, int32_t D, int32_t C, int64_t micro_batch);
 int zf_coupling_backward(void* stream, const zf_coupling* cp, const zf_coupling_grads* grads, int32_t D, int32_t C,
                          const float* x_in, const float* c, const float* gy, int32_t gy_rot, const float* glp,
@@ -353,6 +354,22 @@ int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_chain* chain
                            double global_count, const float* lp_cotangent, float* lp, double* lp_sum, float* gc,
                            void* dp_comm, void* dp_grad_comm, float* grad_flat, const int64_t* bucket_off,
                            void* workspace, size_t workspace_bytes, int64_t micro_batch);
+
+/* ---- VJP of the eval-mode log-density (flow.py:22-48: jax.grad of Flow.__call__(x, c, train=False)) -----------
+ * The running statistics (the couplings' bn_mean / bn_var, the ShiftBounds' xmin / xmax) are read, never written.
+ * Same plan and loop as zf_flow_value_and_grad without the statistics phases: the BatchNorm input VJP is the
+ * diagonal one of fixed statistics, and the backward continues through a leading ShiftBounds into gx.
+ *   chain         layout as for zf_flow_value_and_grad; a chain with no coupling ([ShiftBounds] Roll*) is accepted too
+ *   grads         one zf_coupling_grads per coupling op, in op order; accumulated into (+=).  NULL: input cotangents
+ *                 only (no grad-weight products, no BatchNorm parameter sums)
+ *   lp_cotangent  (M,) required: the cotangent of lp (ones = per-event gradients of log p, the events being
+ *                 independent in eval mode); events whose lp is not finite (nan_to_num) get zero gradients
+ *   lp (M,)       optional output: the log-density as recomputed by this call
+ *   gx (M,D), gc (M,C)  optional outputs, overwritten: d/dx and d/dc */
+size_t zf_flow_log_prob_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch);
+int zf_flow_log_prob_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, int32_t latent_kind,
+                         float peakness, const float* x, const float* c, int64_t M, const float* lp_cotangent,
+                         float* lp, float* gx, float* gc, void* workspace, size_t workspace_bytes, int64_t micro_batch);
 
 /* ---- Deep-Set conditioner Phi (examples/deep_set.ipynb:138-160; SURVEY.md 8f-4) ---------------------------
  * The FLAX module on the other side of the flow's conditions in the deep_set config:

@@ -1,13 +1,14 @@
-"""Host-side assembly of the native chain description (zf_chain) and the three eval calls.
+"""Host-side assembly of the native chain description (zf_chain), the eval calls and the VJP of the eval log-density.
 
 A ``ChainSpec`` is what the bijector modules emit: the op list of a Chain with device
 pointers to the FLAX variable leaves.  It owns the torch tensors behind those pointers for
-the duration of the call.  No arithmetic happens here.
+the duration of the call, and remembers which original leaf object each coupling's parameter
+pointer came from (so gradients can be handed back to those objects).  No arithmetic happens here.
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -25,6 +26,10 @@ class ChainSpec:
         self.device = require_cuda()
         self._ops: List[_lib.ZfOp] = []
         self._keep: list = []  # tensors and ctypes structs that must outlive the call
+        # per coupling, in op order: the original params leaves (BatchNorm scale, bias, then kernel_j, bias_j per Dense)
+        # and the float32 device tensors the zf_coupling points at, in zf_coupling_grads order
+        self.coupling_params: List[Tuple[list, List[torch.Tensor]]] = []
+        self.param_slots: List[Tuple[int, int]] = []   # (coupling, slot) of each torch leaf a differentiable call takes
 
     # -- emitters used by the bijectors -------------------------------------------------------
     def leaf(self, a) -> torch.Tensor:
@@ -64,8 +69,10 @@ class ChainSpec:
         cp.act = int(act)
         for i, w in enumerate(hidden):
             cp.hidden[i] = int(w)
-        cp.bn_scale = ptr(self.leaf(bn_scale))
-        cp.bn_bias = ptr(self.leaf(bn_bias))
+        scale_t, bias_t = self.leaf(bn_scale), self.leaf(bn_bias)
+        cp.bn_scale = ptr(scale_t)
+        cp.bn_bias = ptr(bias_t)
+        src, dev = [bn_scale, bn_bias], [scale_t, bias_t]
         cp.bn_mean = ptr(self.leaf(bn_mean))
         cp.bn_var = ptr(self.leaf(bn_var))
         d = self.dim // 2
@@ -78,8 +85,11 @@ class ChainSpec:
                                  f"the expected ({fan_in}, {widths[i]})")
             cp.kernel[i] = ptr(kt)
             cp.bias[i] = ptr(bt)
+            src += [k, b]
+            dev += [kt, bt]
             fan_in = widths[i]
         self._keep.append(cp)
+        self.coupling_params.append((src, dev))
         op = _lib.ZfOp()
         op.kind = _lib.OP_COUPLING
         op.coupling = C.pointer(cp)
@@ -163,6 +173,42 @@ class ChainSpec:
                                         ptr(cd), M, ptr(lp), ptr(ws), nbytes), "zf_flow_log_prob")
         return lp
 
+    def log_prob_vjp(self, x, c, latent_kind: int, peakness: float, lp_cotangent, *, want_gx: bool = True,
+                     want_gc: bool = True, want_params: bool = True, micro_batch: int = 1 << 18, want_lp: bool = False):
+        """VJP of the eval-mode log-density (zf_flow_log_prob_vjp) for the cotangent ``lp_cotangent`` (M,).
+
+        Returns ``(gx, gc, param_grads, lp)``: float32 device tensors, None where not asked for;
+        ``param_grads[k]`` lists coupling k's gradients in the order of ``coupling_params[k]``."""
+        lib = _lib.load()
+        xd, cd = self._inputs(x, c)
+        M = xd.shape[0]
+        ch = self._chain()
+        ct = to_device_f32(lp_cotangent, self.device).reshape(-1)
+        if ct.shape[0] != M:
+            raise ValueError(f"lp_cotangent must have shape ({M},), got {tuple(ct.shape)}")
+        nbytes = int(lib.zf_flow_log_prob_vjp_workspace_bytes(C.byref(ch), M, int(micro_batch)))
+        if nbytes == 0:
+            _lib.check(1, "zf_flow_log_prob_vjp_workspace_bytes")
+        ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
+        base = (ws.data_ptr() + 255) & ~255
+        gx = torch.empty_like(xd) if want_gx else None
+        gc = torch.empty_like(cd) if (want_gc and cd is not None) else None
+        lp = torch.empty(M, dtype=torch.float32, device=self.device) if want_lp else None
+        grads, arr = None, None
+        if want_params and self.coupling_params:
+            grads = [[torch.zeros_like(t) for t in dev] for _, dev in self.coupling_params]
+            arr = (_lib.ZfCouplingGrads * len(grads))()
+            for k, gl in enumerate(grads):
+                arr[k].bn_scale, arr[k].bn_bias = ptr(gl[0]), ptr(gl[1])
+                for j in range((len(gl) - 2) // 2):
+                    arr[k].kernel[j] = ptr(gl[2 + 2 * j])
+                    arr[k].bias[j] = ptr(gl[3 + 2 * j])
+        _lib.check(lib.zf_flow_log_prob_vjp(stream_ptr(), C.byref(ch), arr, int(latent_kind), float(peakness), ptr(xd),
+                                            ptr(cd), M, ptr(ct), ptr(lp), ptr(gx), ptr(gc), base,
+                                            ws.numel() - (base - ws.data_ptr()), int(micro_batch)),
+                   "zf_flow_log_prob_vjp")
+        return gx, gc, grads, lp
+
     def sample(self, n: int, c, latent_kind: int, peakness: float, seed: int):
         """Flow.sample: latent draw inside the inverse chain kernel (zf_flow_sample)."""
         lib = _lib.load()
@@ -182,3 +228,52 @@ class ChainSpec:
                                       int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(cd), n, ptr(x), ptr(ws), nbytes),
                    "zf_flow_sample")
         return x
+
+
+def _wants_grad(a) -> bool:
+    return isinstance(a, torch.Tensor) and a.requires_grad
+
+
+def _grad_like(g: Optional[torch.Tensor], like) -> Optional[torch.Tensor]:
+    """A float32 device gradient in the device, dtype and shape of the tensor it belongs to."""
+    if g is None:
+        return None
+    return g.to(device=like.device, dtype=like.dtype).reshape(like.shape)
+
+
+class _FlowLogProb(torch.autograd.Function):
+    """Flow.__call__(x, c, train=False) as a differentiable op: forward = zf_flow_log_prob (the non-grad call, so lp is
+    bit-identical to it), backward = one zf_flow_log_prob_vjp with the incoming gradient as the cotangent of lp.
+    ``leaves`` are the torch tensors among the couplings' params leaves, in ``spec.param_slots`` order."""
+
+    @staticmethod
+    def forward(ctx, spec, latent_kind, peakness, x, c, *leaves):
+        xd, cd = spec._inputs(x, c)
+        ctx.spec, ctx.latent = spec, (latent_kind, peakness)
+        ctx.x_like = x.detach() if isinstance(x, torch.Tensor) else None
+        ctx.c_like = c.detach() if isinstance(c, torch.Tensor) else None
+        ctx.save_for_backward(xd, cd)
+        return spec.log_prob(xd, cd, latent_kind, peakness)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_lp):
+        xd, cd = ctx.saved_tensors
+        spec = ctx.spec
+        need = ctx.needs_input_grad
+        want_p = any(need[5:])
+        gx, gc, grads, _ = spec.log_prob_vjp(xd, cd, *ctx.latent, g_lp, want_gx=need[3], want_gc=need[4],
+                                             want_params=want_p)
+        out_p = []
+        for i, (k, j) in enumerate(spec.param_slots):
+            out_p.append(_grad_like(grads[k][j], spec.coupling_params[k][0][j]) if need[5 + i] else None)
+        return (None, None, None, _grad_like(gx, ctx.x_like) if need[3] else None,
+                _grad_like(gc, ctx.c_like) if need[4] else None, *out_p)
+
+
+def flow_log_prob_differentiable(spec: ChainSpec, x, c, latent_kind: int, peakness: float) -> torch.Tensor:
+    """The eval log-density with a grad_fn wrt every torch tensor among x, c and the couplings' params leaves."""
+    spec.param_slots = [(k, j) for k, (src, _) in enumerate(spec.coupling_params)
+                        for j, leaf in enumerate(src) if isinstance(leaf, torch.Tensor)]
+    leaves = [spec.coupling_params[k][0][j] for k, j in spec.param_slots]
+    return _FlowLogProb.apply(spec, latent_kind, peakness, x, c, *leaves)

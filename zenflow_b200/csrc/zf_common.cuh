@@ -102,6 +102,20 @@ int launch_img_tn(cudaStream_t st, const void* A, const void* B, int WB, float* 
 // In-place all-reduce over the data-parallel ranks of `comm` (zf_dp.cu); op 0 = sum, 1 = min.  A null comm is a no-op.
 int dp_allreduce(cudaStream_t st, void* comm, void* buf, long long n, int is_f64, int op);
 
+// Eval-mode pieces of the step loop (zf_train.cu, sequenced by zf_step.cu).
+// zf_flow_loss_grad_ct; zero_dead = 1 also zeroes gz on rows whose cotangent is 0 (nan_to_num rows), where the latent's
+// derivative may be infinite: eval batches may hold events outside the running ShiftBounds range.
+int flow_loss_grad(cudaStream_t st, int latent_kind, float peakness, const float* z, const float* log_det, long long M, int D,
+                   double global_count, const float* lp_cotangent, float* lp, float* gz, float* glp, double* lp_sum,
+                   int zero_dead);
+// Eval-mode BatchNorm VJP into its inputs (running statistics are constants): gx[:, D/2 + f] += dh_f,
+// gc[:, f - (D - D/2)] += dh_f, dh = gh0 * scale * rstd(cp->bn_var).
+int bn_backward_eval(cudaStream_t st, const zf_coupling* cp, int D, int C, const float* gh0, long long M, float* gx, float* gc);
+// Eval-mode ShiftBounds VJP: gx (M, D) = d/dx of the ShiftBounds output (cotangent gz, column i read at (i + gz_rot) % D)
+// and of its log-det (cotangent glp), with the running sb->xmin / sb->xmax.
+int shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* x, const float* gz, int gz_rot,
+                          const float* glp, long long M, float* gx);
+
 // ---- PTX wrappers ----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return (uint32_t)__cvta_generic_to_shared(p);

@@ -1,4 +1,6 @@
-// zf_flow_value_and_grad: the whole `loss_fn` + `jax.grad` of train.py:64-86 as ONE C-ABI call.
+// zf_flow_value_and_grad: the whole `loss_fn` + `jax.grad` of train.py:64-86 as ONE C-ABI call, and
+// zf_flow_log_prob_vjp: the VJP of Flow.__call__(x, c, train=False), flow.py:22-48 (what jax.grad of the eval-mode
+// log-density gives: the score d/dx, d/dc and the parameter gradients with the running statistics held fixed).
 //
 // Train mode couples the events of a batch (ShiftBounds batch min/max, bijectors.py:250-260; BatchNorm batch
 // moments, bijectors.py:342), so the step is a sequence of phases, each a kernel (or a few) of zf_train.cu /
@@ -9,6 +11,9 @@
 //   loss      lp = nan_to_num(latent.log_prob(z) + log_det), cotangents of z and of the log-dets
 //   backward  per coupling in reverse: recompute + spline VJP + Dense VJPs -> [all-reduce BatchNorm sums] ->
 //             BatchNorm VJP into x and c; the coupling's gradient bucket is all-reduced behind it
+// Eval mode runs the same plan and the same loop (run_step) with three differences: no statistics phase (the
+// couplings and the ShiftBounds read their running statistics), the diagonal BatchNorm VJP instead of the
+// batch-coupled one, and the backward continues through a leading ShiftBounds into d/dx.
 #include "zf_common.cuh"
 
 #include <algorithm>
@@ -30,7 +35,7 @@ struct StepPlan {
     int Fmax = 1;
     // workspace carve-up in bytes
     size_t off_states = 0, off_ld = 0, off_glp = 0, off_ga = 0, off_gb = 0, off_gh0 = 0, off_stats = 0, off_chain = 0,
-           off_bwd = 0, total = 0;
+           off_bwd = 0, off_lp_sum = 0, total = 0;
     size_t stats_stride = 0, chain_bytes = 0, bwd_bytes = 0;
 };
 
@@ -38,34 +43,37 @@ static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // Per-coupling statistics block: bmean[F] bvar[F] (float) | fwd sums 2F (double) | bwd sums 2F (double);
 // the ShiftBounds group uses the same block for minmax[2D] (float) | scratch[2D] (uint32).
-static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, StepPlan& p) {
-    ZF_REQUIRE(chain && chain->n_ops >= 1 && chain->ops, "value_and_grad: empty chain");
+// Eval mode uses only the bwd sums (parameter gradients of the BatchNorm) and adds a slot for the lp sum the loss
+// kernel keeps; it also accepts a chain with no coupling, whose only derivative is d/dx through the ShiftBounds.
+static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, bool train, StepPlan& p) {
+    const char* who = train ? "value_and_grad" : "log_prob_vjp";
+    ZF_REQUIRE(chain && chain->n_ops >= 1 && chain->ops, "%s: empty chain", who);
     const int D = chain->dim, C = chain->cdim;
-    ZF_REQUIRE(D >= 2 && D <= ZF_MAX_DIM, "value_and_grad: dim must be in [2, %d]", ZF_MAX_DIM);
-    ZF_REQUIRE(M >= 1 && micro_batch >= 1, "value_and_grad: bad batch");
+    ZF_REQUIRE(D >= (train ? 2 : 1) && D <= ZF_MAX_DIM, "%s: dim must be in [%d, %d]", who, train ? 2 : 1, ZF_MAX_DIM);
+    ZF_REQUIRE(M >= 1 && micro_batch >= 1, "%s: bad batch", who);
     for (int i = 0; i < chain->n_ops; ++i) {
         const zf_op& op = chain->ops[i];
         if (op.kind == ZF_OP_ROLL) {
             if (p.groups.empty())
-                return fail(ZF_ERR_UNSUPPORTED, "value_and_grad: a chain that starts with Roll is not supported");
+                return fail(ZF_ERR_UNSUPPORTED, "%s: a chain that starts with Roll is not supported", who);
             p.groups.back().ops.push_back(op);
             p.groups.back().rot += op.shift;
         } else if (op.kind == ZF_OP_SHIFT_BOUNDS) {
             if (!p.groups.empty())
-                return fail(ZF_ERR_UNSUPPORTED, "value_and_grad: ShiftBounds after another bijector is not supported");
-            ZF_REQUIRE(op.shift_bounds, "value_and_grad: op %d: shift_bounds is NULL", i);
+                return fail(ZF_ERR_UNSUPPORTED, "%s: ShiftBounds after another bijector is not supported", who);
+            ZF_REQUIRE(op.shift_bounds, "%s: op %d: shift_bounds is NULL", who, i);
             p.groups.push_back(StepGroup{ZF_OP_SHIFT_BOUNDS, i, -1, 0, {op}});
         } else if (op.kind == ZF_OP_COUPLING) {
-            ZF_REQUIRE(op.coupling, "value_and_grad: op %d: coupling is NULL", i);
+            ZF_REQUIRE(op.coupling, "%s: op %d: coupling is NULL", who, i);
             p.groups.push_back(StepGroup{ZF_OP_COUPLING, i, p.n_couplings++, 0, {op}});
         } else {
-            return fail(ZF_ERR_INVALID, "value_and_grad: op %d: unknown kind %d", i, op.kind);
+            return fail(ZF_ERR_INVALID, "%s: op %d: unknown kind %d", who, i, op.kind);
         }
     }
-    ZF_REQUIRE(p.n_couplings >= 1, "value_and_grad: the chain has no coupling (nothing to differentiate)");
+    ZF_REQUIRE(!train || p.n_couplings >= 1, "value_and_grad: the chain has no coupling (nothing to differentiate)");
     const int F = D - D / 2 + C;
     p.Fmax = F;
-    ZF_REQUIRE(F <= 256, "value_and_grad: at most 256 conditioner inputs");
+    ZF_REQUIRE(F <= 256, "%s: at most 256 conditioner inputs", who);
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     p.off_states = take(p.groups.size() * (size_t)M * D * 4);
@@ -87,6 +95,7 @@ static int build_step_plan(const zf_chain* chain, long long M, long long micro_b
     }
     p.off_chain = take(p.chain_bytes);
     p.off_bwd = take(p.bwd_bytes);
+    if (!train) p.off_lp_sum = take(sizeof(double));
     p.total = off;
     return ZF_OK;
 }
@@ -108,34 +117,41 @@ static int aux_events(AuxEvents** out) {
     return ZF_OK;
 }
 
-}  // namespace zf
+// The arguments of either entry point.  Train-only fields (global_count, lp_sum, the communicators and buckets) are
+// unused in eval mode; gx (d/dx) is eval-only.
+struct StepCall {
+    bool train;
+    cudaStream_t st, aux;
+    const zf_chain* chain;
+    const zf_coupling_grads* grads;
+    int latent_kind;
+    float peakness;
+    const float* x;
+    const float* c;
+    long long M;
+    double global_count;
+    const float* lp_cotangent;
+    float* lp;
+    double* lp_sum;
+    float* gx;
+    float* gc;
+    void* dp_comm;
+    void* dp_grad_comm;
+    float* grad_flat;
+    const int64_t* bucket_off;
+    char* ws;
+    long long micro_batch;
+};
 
-using namespace zf;
-
-extern "C" size_t zf_flow_value_and_grad_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
-    StepPlan p;
-    if (build_step_plan(chain, M, micro_batch, p) != ZF_OK) return 0;
-    return p.total;
-}
-
-extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_chain* chain, const zf_coupling_grads* grads,
-                                      int32_t latent_kind, float peakness, const float* x, const float* c, int64_t M,
-                                      double global_count, const float* lp_cotangent, float* lp, double* lp_sum, float* gc,
-                                      void* dp_comm, void* dp_grad_comm, float* grad_flat, const int64_t* bucket_off,
-                                      void* workspace, size_t workspace_bytes, int64_t micro_batch) {
-    StepPlan p;
-    if (int rc = build_step_plan(chain, M, micro_batch, p)) return rc;
-    ZF_REQUIRE(x && lp_sum && workspace, "value_and_grad: null argument");
-    const bool fwd_only = (grads == nullptr);   // train-mode forward only: lp, lp_sum and the statistics updates
-    ZF_REQUIRE(chain->cdim == 0 || c, "value_and_grad: chain has cdim=%d but c is NULL", chain->cdim);
-    ZF_REQUIRE(global_count >= 1, "value_and_grad: global_count must be >= 1");
-    ZF_REQUIRE(!grad_flat || bucket_off, "value_and_grad: grad_flat needs bucket_off");
-    ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "value_and_grad: workspace must be 256-byte aligned");
-    if (workspace_bytes < p.total)
-        return fail(ZF_ERR_WORKSPACE, "value_and_grad: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
-    const int D = chain->dim, C = chain->cdim, F = D - D / 2 + C;
-    cudaStream_t st = (cudaStream_t)stream, aux = (cudaStream_t)aux_stream;
-    char* ws = static_cast<char*>(workspace);
+// One plan, one loop: the forward per group, the loss cotangents, the backward per group in reverse.
+static int run_step(StepPlan& p, const StepCall& a) {
+    const bool train = a.train;
+    const int D = a.chain->dim, C = a.chain->cdim, F = D - D / 2 + C;
+    cudaStream_t st = a.st;
+    char* ws = a.ws;
+    const long long M = a.M;
+    const float* x = a.x;
+    const float* c = a.c;
     float* ld = reinterpret_cast<float*>(ws + p.off_ld);
     float* glp = reinterpret_cast<float*>(ws + p.off_glp);
     float* gy = reinterpret_cast<float*>(ws + p.off_ga);
@@ -143,25 +159,27 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
     float* gh0 = reinterpret_cast<float*>(ws + p.off_gh0);
     void* chain_ws = ws + p.off_chain;
     void* bwd_ws = ws + p.off_bwd;
-    const long long mb = std::min<long long>(micro_batch, M);
+    const long long mb = std::min<long long>(a.micro_batch, M);
     auto state = [&](size_t g) { return reinterpret_cast<float*>(ws + p.off_states + g * (size_t)M * D * 4); };
     auto stats = [&](size_t g) { return ws + p.off_stats + g * p.stats_stride; };
 
     ZF_CUDA_CHECK(cudaMemsetAsync(ld, 0, (size_t)M * 4, st));
-    if (gc && C) ZF_CUDA_CHECK(cudaMemsetAsync(gc, 0, (size_t)M * C * 4, st));
+    if (a.gc && C) ZF_CUDA_CHECK(cudaMemsetAsync(a.gc, 0, (size_t)M * C * 4, st));
 
-    // ---- forward, one bijector group at a time (the batch statistics couple the events)
-    std::vector<zf_coupling> batch_cp(p.groups.size());   // couplings reading the BATCH statistics
+    // ---- forward, one bijector group at a time (in train mode the batch statistics couple the events)
+    std::vector<zf_coupling> batch_cp(p.groups.size());   // couplings reading the BATCH statistics (train mode)
     const float* cur = x;
     for (size_t gi = 0; gi < p.groups.size(); ++gi) {
         StepGroup& g = p.groups[gi];
         float* nxt = state(gi);
-        if (g.kind == ZF_OP_SHIFT_BOUNDS) {
+        if (!train) {
+            // the chain's own ShiftBounds and couplings: running statistics, read only
+        } else if (g.kind == ZF_OP_SHIFT_BOUNDS) {
             const zf_shift_bounds* sb = g.ops[0].shift_bounds;
             float* mm = reinterpret_cast<float*>(stats(gi));
             void* scratch = mm + 2 * D;
             if (int rc = zf_shift_bounds_minmax(st, sb, cur, M, D, mm, scratch)) return rc;
-            if (int rc = zf_dp_allreduce_minmax_f32(st, dp_comm, mm, D)) return rc;
+            if (int rc = zf_dp_allreduce_minmax_f32(st, a.dp_comm, mm, D)) return rc;
             if (int rc = zf_shift_bounds_update(st, sb, D, mm)) return rc;
         } else {
             const zf_coupling* cp = g.ops[0].coupling;
@@ -169,8 +187,8 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
             float* bvar = bmean + F;
             double* sums = reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8));
             if (int rc = zf_bn_moments(st, cur, c, M, D, C, sums)) return rc;
-            if (int rc = dp_allreduce(st, dp_comm, sums, 2 * F, 1, 0)) return rc;
-            if (int rc = zf_bn_finalize(st, sums, global_count, F, 0.99f /* flax BatchNorm momentum */, bmean, bvar,
+            if (int rc = dp_allreduce(st, a.dp_comm, sums, 2 * F, 1, 0)) return rc;
+            if (int rc = zf_bn_finalize(st, sums, a.global_count, F, 0.99f /* flax BatchNorm momentum */, bmean, bvar,
                                         cp->bn_mean, cp->bn_var))
                 return rc;
             batch_cp[gi] = *cp;
@@ -184,44 +202,112 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
     }
 
     // ---- loss and the cotangents of z and of the log-dets (flow.py:46-47, train.py:73)
-    if (int rc = zf_flow_loss_grad_ct(st, latent_kind, peakness, cur, ld, M, D, global_count, lp_cotangent, lp, gy, glp, lp_sum))
+    double* lp_sum = train ? a.lp_sum : reinterpret_cast<double*>(ws + p.off_lp_sum);
+    if (int rc = flow_loss_grad(st, a.latent_kind, a.peakness, cur, ld, M, D, a.global_count, a.lp_cotangent, a.lp, gy, glp,
+                                lp_sum, train ? 0 : 1))
         return rc;
-    if (fwd_only) return ZF_OK;
+    if (train && !a.grads) return ZF_OK;
 
     // ---- backward
-    const bool bucketed = dp_comm && grad_flat;
-    const bool overlap = bucketed && aux && dp_grad_comm;
+    const bool bucketed = a.dp_comm && a.grad_flat;
+    const bool overlap = bucketed && a.aux && a.dp_grad_comm;
     AuxEvents* ev = nullptr;
     if (overlap)
         if (int rc = aux_events(&ev)) return rc;
     for (size_t gi = p.groups.size(); gi-- > 0;) {
         StepGroup& g = p.groups[gi];
-        if (g.kind != ZF_OP_COUPLING) break;   // a leading ShiftBounds has no parameters; x needs no cotangent
-        const zf_coupling* cp = &batch_cp[gi];
-        const zf_coupling_grads* gr = &grads[g.coupling_index];
         const float* x_in = gi == 0 ? x : state(gi - 1);
-        double* bsums = reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8)) + 2 * F;
-        if (int rc = zf_coupling_backward(st, cp, gr, D, C, x_in, c, gy, g.rot, glp, M, gx, gh0, bsums, bwd_ws, p.bwd_bytes, mb))
+        float* dst = (gi == 0 && a.gx) ? a.gx : gx;   // the cotangent of x goes straight to the caller's buffer
+        if (g.kind != ZF_OP_COUPLING) {
+            // a leading ShiftBounds has no parameters: in train mode x needs no cotangent
+            if (train || !a.gx) break;
+            if (int rc = shift_bounds_backward(st, g.ops[0].shift_bounds, D, x, gy, g.rot, glp, M, a.gx)) return rc;
+            break;
+        }
+        const zf_coupling* cp = train ? &batch_cp[gi] : g.ops[0].coupling;
+        const zf_coupling_grads* gr = a.grads ? &a.grads[g.coupling_index] : nullptr;
+        // sum gh0 and sum gh0 xhat: the BatchNorm's parameter gradients, and in train mode also its input VJP
+        double* bsums = gr ? reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8)) + 2 * F : nullptr;
+        if (int rc = zf_coupling_backward(st, cp, gr, D, C, x_in, c, gy, g.rot, glp, M, dst, gh0, bsums, bwd_ws, p.bwd_bytes, mb))
             return rc;
-        if (int rc = zf_bn_param_grads(st, bsums, F, gr->bn_scale, gr->bn_bias)) return rc;
+        if (gr)
+            if (int rc = zf_bn_param_grads(st, bsums, F, gr->bn_scale, gr->bn_bias)) return rc;
+        if (!train) {
+            if (int rc = bn_backward_eval(st, cp, D, C, gh0, M, dst, a.gc)) return rc;
+            std::swap(gy, gx);
+            continue;
+        }
         if (bucketed) {   // this coupling's parameter gradients are complete: reduce them behind the next backward
-            float* b0 = grad_flat + bucket_off[g.coupling_index];
-            const long long bn = bucket_off[g.coupling_index + 1] - bucket_off[g.coupling_index];
+            float* b0 = a.grad_flat + a.bucket_off[g.coupling_index];
+            const long long bn = a.bucket_off[g.coupling_index + 1] - a.bucket_off[g.coupling_index];
             if (overlap) {
                 ZF_CUDA_CHECK(cudaEventRecord(ev->main_done, st));
-                ZF_CUDA_CHECK(cudaStreamWaitEvent(aux, ev->main_done, 0));
-                if (int rc = dp_allreduce(aux, dp_grad_comm, b0, bn, 0, 0)) return rc;
+                ZF_CUDA_CHECK(cudaStreamWaitEvent(a.aux, ev->main_done, 0));
+                if (int rc = dp_allreduce(a.aux, a.dp_grad_comm, b0, bn, 0, 0)) return rc;
             } else {
-                if (int rc = dp_allreduce(st, dp_comm, b0, bn, 0, 0)) return rc;
+                if (int rc = dp_allreduce(st, a.dp_comm, b0, bn, 0, 0)) return rc;
             }
         }
-        if (int rc = dp_allreduce(st, dp_comm, bsums, 2 * F, 1, 0)) return rc;
-        if (int rc = zf_bn_backward_apply(st, cp, D, C, x_in, c, gh0, bsums, global_count, M, gx, gc)) return rc;
+        if (int rc = dp_allreduce(st, a.dp_comm, bsums, 2 * F, 1, 0)) return rc;
+        if (int rc = zf_bn_backward_apply(st, cp, D, C, x_in, c, gh0, bsums, a.global_count, M, dst, a.gc)) return rc;
         std::swap(gy, gx);
     }
     if (overlap) {
-        ZF_CUDA_CHECK(cudaEventRecord(ev->aux_done, aux));
+        ZF_CUDA_CHECK(cudaEventRecord(ev->aux_done, a.aux));
         ZF_CUDA_CHECK(cudaStreamWaitEvent(st, ev->aux_done, 0));
     }
     return ZF_OK;
+}
+
+}  // namespace zf
+
+using namespace zf;
+
+extern "C" size_t zf_flow_value_and_grad_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
+    StepPlan p;
+    if (build_step_plan(chain, M, micro_batch, true, p) != ZF_OK) return 0;
+    return p.total;
+}
+
+extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_chain* chain, const zf_coupling_grads* grads,
+                                      int32_t latent_kind, float peakness, const float* x, const float* c, int64_t M,
+                                      double global_count, const float* lp_cotangent, float* lp, double* lp_sum, float* gc,
+                                      void* dp_comm, void* dp_grad_comm, float* grad_flat, const int64_t* bucket_off,
+                                      void* workspace, size_t workspace_bytes, int64_t micro_batch) {
+    StepPlan p;
+    if (int rc = build_step_plan(chain, M, micro_batch, true, p)) return rc;
+    ZF_REQUIRE(x && lp_sum && workspace, "value_and_grad: null argument");
+    ZF_REQUIRE(chain->cdim == 0 || c, "value_and_grad: chain has cdim=%d but c is NULL", chain->cdim);
+    ZF_REQUIRE(global_count >= 1, "value_and_grad: global_count must be >= 1");
+    ZF_REQUIRE(!grad_flat || bucket_off, "value_and_grad: grad_flat needs bucket_off");
+    ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "value_and_grad: workspace must be 256-byte aligned");
+    if (workspace_bytes < p.total)
+        return fail(ZF_ERR_WORKSPACE, "value_and_grad: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
+    StepCall a{true, (cudaStream_t)stream, (cudaStream_t)aux_stream, chain, grads, latent_kind, peakness, x, c, M,
+               global_count, lp_cotangent, lp, lp_sum, nullptr, gc, dp_comm, dp_grad_comm, grad_flat, bucket_off,
+               static_cast<char*>(workspace), micro_batch};
+    return run_step(p, a);
+}
+
+extern "C" size_t zf_flow_log_prob_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
+    StepPlan p;
+    if (build_step_plan(chain, M, micro_batch, false, p) != ZF_OK) return 0;
+    return p.total;
+}
+
+extern "C" int zf_flow_log_prob_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, int32_t latent_kind,
+                                    float peakness, const float* x, const float* c, int64_t M, const float* lp_cotangent,
+                                    float* lp, float* gx, float* gc, void* workspace, size_t workspace_bytes,
+                                    int64_t micro_batch) {
+    StepPlan p;
+    if (int rc = build_step_plan(chain, M, micro_batch, false, p)) return rc;
+    ZF_REQUIRE(x && lp_cotangent && workspace, "log_prob_vjp: null argument");
+    ZF_REQUIRE(chain->cdim == 0 || c, "log_prob_vjp: chain has cdim=%d but c is NULL", chain->cdim);
+    ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "log_prob_vjp: workspace must be 256-byte aligned");
+    if (workspace_bytes < p.total)
+        return fail(ZF_ERR_WORKSPACE, "log_prob_vjp: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
+    // the cotangent is given, so the count that scales the train loss plays no part
+    StepCall a{false, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, x, c, M, 1.0, lp_cotangent, lp,
+               nullptr, gx, gc, nullptr, nullptr, nullptr, nullptr, static_cast<char*>(workspace), micro_batch};
+    return run_step(p, a);
 }

@@ -267,6 +267,84 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float* __restri
     for (; m < M; m += step) apply(m, cond_feature(x, c, m, f, D, d, C), g[m * F + f]);
 }
 
+// Eval-mode BatchNorm VJP: the running statistics are constants, so dh = scale * rstd * g with no batch terms (rstd as in
+// bn_bwd_apply_kernel); gx[:, d+f] += dh (f < D-d), gc[:, f-(D-d)] += dh.  Reads only g: x and c are not needed.
+__global__ void __launch_bounds__(256) bn_bwd_eval_kernel(const float* __restrict__ g, long long M, int D, int C,
+                                                          const float* __restrict__ scale, const float* __restrict__ var,
+                                                          float* __restrict__ gx, float* __restrict__ gc) {
+    const int d = D / 2, F = D - d + C;
+    extern __shared__ float sha[];
+    for (int f = threadIdx.x; f < F; f += blockDim.x) {
+        const float rstd = __fdiv_rn(1.0f, __fsqrt_rn(__fadd_rn(var[f], 1e-5f)));
+        sha[f] = scale[f] * rstd;
+    }
+    __syncthreads();
+    const long long n = M * F;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+        const long long m = e / F;
+        const int f = (int)(e - m * F);
+        const float dh = sha[f] * g[e];
+        if (f < D - d) gx[m * D + d + f] += dh;
+        else if (gc) gc[m * C + (f - (D - d))] += dh;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Eval-mode ShiftBounds VJP (forward: shift_bounds_row in zf_chain.cu, bijectors.py:183-207 / :262-273)
+//   both bounds   z = (x - a) mul                         dz/dx = mul = 1 / (b - a)
+//   otherwise     z = clip((u - xmin) mul, 0, 1)          dz/du = mul strictly inside (0, 1), else 0 (zf_vjp.cuh)
+//                 u = x | log(x - a + tiny) | log(b - x + tiny),  du/dx = 1 | 1/(x - a + tiny) | -1/(b - x + tiny)
+//                 the one-sided log-det log(mul) - u adds -glp du/dx
+// ---------------------------------------------------------------------------------------------
+struct SbVjpCols {
+    SbCols c;
+    float mul_both[ZF_MAX_DIM];   // (float)(1 / (b - a)) of ZF_BOUND_BOTH columns, in double as the chain's pack_step_kernel
+};
+
+__global__ void __launch_bounds__(256) sb_bwd_kernel(const __grid_constant__ SbVjpCols cols, const float* __restrict__ xmin,
+                                                     const float* __restrict__ xmax, const float* __restrict__ x,
+                                                     const float* __restrict__ gz, int rot, const float* __restrict__ glp,
+                                                     long long M, int D, float* __restrict__ gx) {
+    __shared__ float smul[ZF_MAX_DIM], smin[ZF_MAX_DIM];
+    for (int i = threadIdx.x; i < D; i += blockDim.x) {
+        if (cols.c.kind[i] == ZF_BOUND_BOTH) {
+            smul[i] = cols.mul_both[i];
+            smin[i] = 0.f;
+        } else {
+            smul[i] = __fdiv_rn(1.0f, __fsub_rn(xmax[i], xmin[i]));   // as the chain's pack_step_kernel
+            smin[i] = xmin[i];
+        }
+    }
+    __syncthreads();
+    const long long n = M * D;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+        const long long m = e / D;
+        const int i = (int)(e - m * D);
+        const int kind = cols.c.kind[i];
+        const float v = x[e], g = gz[m * D + (i + rot) % D], mul = smul[i];
+        float r;
+        if (kind == ZF_BOUND_BOTH) {
+            r = g * mul;
+        } else {
+            float u = v, dudx = 1.f;
+            if (kind == ZF_BOUND_LOWER) {
+                const float s = __fadd_rn(__fsub_rn(v, cols.c.lo[i]), FLT_MIN);
+                u = logf(s);
+                dudx = 1.f / s;
+            } else if (kind == ZF_BOUND_UPPER) {
+                const float s = __fadd_rn(__fsub_rn(cols.c.hi[i], v), FLT_MIN);
+                u = logf(s);
+                dudx = -1.f / s;
+            }
+            const float t = __fmul_rn(__fsub_rn(u, smin[i]), mul);
+            const float dzdu = (t > 0.f && t < 1.f) ? mul : 0.f;
+            r = (g * dzdu) * dudx;
+            if (kind != ZF_BOUND_NONE) r -= glp[m] * dudx;
+        }
+        gx[e] = r;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // loss and latent gradient
 // ---------------------------------------------------------------------------------------------
@@ -274,7 +352,7 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
                                                         const float* __restrict__ log_det, long long M, int D,
                                                         float wgt, const float* __restrict__ cot,
                                                         float* __restrict__ lp_out, float* __restrict__ gz,
-                                                        float* __restrict__ glp, double* lp_sum) {
+                                                        float* __restrict__ glp, double* lp_sum, int zero_dead) {
     __shared__ double red[256];
     double local = 0.0;
     for (long long m = blockIdx.x * (long long)blockDim.x + threadIdx.x; m < M; m += (long long)gridDim.x * blockDim.x) {
@@ -293,7 +371,7 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
             if (lc.kind == kLatentBeta) dl = (v > 1.f || v < 0.f) ? 0.f : (lc.p1 / v - lc.p1 / (1.f - v));
             else if (lc.kind == kLatentNormal) dl = -(v - 0.5f) / 0.01f;
             else if (lc.kind == kLatentTruncNormal) dl = (v > 1.f || v < 0.f) ? 0.f : -(v - 0.5f) / 0.01f;
-            gz[m * D + j] = w * dl;
+            gz[m * D + j] = (zero_dead && w == 0.f) ? 0.f : w * dl;   // 0 * inf at a latent boundary
         }
     }
     red[threadIdx.x] = local;
@@ -590,9 +668,9 @@ extern "C" int zf_bn_finalize(void* stream, const double* sums, double count, in
     return ZF_OK;
 }
 
-extern "C" int zf_flow_loss_grad_ct(void* stream, int32_t latent_kind, float peakness, const float* z, const float* log_det,
-                                    int64_t M, int32_t D, double global_count, const float* lp_cotangent, float* lp,
-                                    float* gz, float* glp, double* lp_sum) {
+int zf::flow_loss_grad(cudaStream_t st, int latent_kind, float peakness, const float* z, const float* log_det, long long M,
+                       int D, double global_count, const float* lp_cotangent, float* lp, float* gz, float* glp,
+                       double* lp_sum, int zero_dead) {
     ZF_REQUIRE(z && log_det && gz && glp && lp_sum && M >= 1 && D >= 1 && global_count >= 1, "flow_loss_grad: bad argument");
     LatentConst lc{};
     lc.kind = latent_kind;
@@ -600,12 +678,18 @@ extern "C" int zf_flow_loss_grad_ct(void* stream, int32_t latent_kind, float pea
     lc.betaln = (float)(2.0 * lgamma((double)peakness) - lgamma(2.0 * (double)peakness));
     lc.lognorm = (float)log(2.0 * M_PI * 0.1 * 0.1);
     lc.logmass = (float)log(0.5 * (erf(5.0 / sqrt(2.0)) - erf(-5.0 / sqrt(2.0))));
-    loss_grad_kernel<<<grid_for(M, 256, 148 * 8), 256, 0, (cudaStream_t)stream>>>(lc, z, log_det, M, D,
-                                                                                  (float)(-1.0 / global_count),
-                                                                                  lp_cotangent, lp, gz, glp, lp_sum);
+    loss_grad_kernel<<<grid_for(M, 256, 148 * 8), 256, 0, st>>>(lc, z, log_det, M, D, (float)(-1.0 / global_count),
+                                                                lp_cotangent, lp, gz, glp, lp_sum, zero_dead);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;
+}
+
+extern "C" int zf_flow_loss_grad_ct(void* stream, int32_t latent_kind, float peakness, const float* z, const float* log_det,
+                                    int64_t M, int32_t D, double global_count, const float* lp_cotangent, float* lp,
+                                    float* gz, float* glp, double* lp_sum) {
+    return flow_loss_grad((cudaStream_t)stream, latent_kind, peakness, z, log_det, M, D, global_count, lp_cotangent, lp, gz,
+                          glp, lp_sum, 0);
 }
 
 extern "C" int zf_flow_loss_grad(void* stream, int32_t latent_kind, float peakness, const float* z, const float* log_det,
@@ -697,7 +781,7 @@ static int coupling_backward_fused(cudaStream_t st, const zf_coupling* cp, const
         }
         if (int rc = pack_w_images(st, jobs, L + 1)) return rc;
     }
-    ZF_CUDA_CHECK(cudaMemsetAsync(gWp, 0, lay.fixed_bytes - lay.off_gwp, st));
+    if (gr) ZF_CUDA_CHECK(cudaMemsetAsync(gWp, 0, lay.fixed_bytes - lay.off_gwp, st));
     char* wb = ws + lay.fixed_bytes;
     for (long long m0 = 0; m0 < M; m0 += micro_batch) {
         const long long Mb = std::min<long long>(micro_batch, M - m0);
@@ -717,26 +801,36 @@ static int coupling_backward_fused(cudaStream_t st, const zf_coupling* cp, const
                                       gx + m0 * D, img_h0, lay.WH, img_act, act_g, img_dt))
             return rc;
         // last Dense (padded column space): dW_L, db_L, dZ_L = (dTheta W_L^T) swish'(Z_L)
-        if (int rc = launch_img_tn(st, img_act[L - 1], img_dt, TW, gWp, TW, 1, 128, TW, gbp, nullptr, -1, Mb)) return rc;
+        if (gr)
+            if (int rc = launch_img_tn(st, img_act[L - 1], img_dt, TW, gWp, TW, 1, 128, TW, gbp, nullptr, -1, Mb)) return rc;
         if (int rc = launch_img_nt(st, img_dt, TW, ws + lay.off_wimg[L], 128, act_g[L - 1], -1, img_dz[0], nullptr, 0, 0, Mb)) return rc;
         int cur = 0;
         for (int l = L - 1; l >= 1; --l) {   // hidden Dense_l: input swish(Z_l), output cotangent dZ_{l+1}
-            if (int rc = launch_img_tn(st, img_act[l - 1], img_dz[cur], 128, gr->kernel[l], 128, 1, 128, 128, gr->bias[l], nullptr, -1, Mb))
-                return rc;
+            if (gr)
+                if (int rc = launch_img_tn(st, img_act[l - 1], img_dz[cur], 128, gr->kernel[l], 128, 1, 128, 128, gr->bias[l], nullptr, -1,
+                                           Mb))
+                    return rc;
             if (int rc = launch_img_nt(st, img_dz[cur], 128, ws + lay.off_wimg[l], 128, act_g[l - 1], -1, img_dz[cur ^ 1], nullptr, 0, 0, Mb))
                 return rc;
             cur ^= 1;
         }
         // first Dense: dW_0[f][h] = sum_e H0[e][f] dZ_1[e][h] (transposed product; H0's bias column gives db_0), d/dH0
-        if (int rc = launch_img_tn(st, img_dz[cur], img_h0, lay.WH, gr->kernel[0], 1, 128, 128, F, nullptr, gr->bias[0], F, Mb)) return rc;
+        if (gr)
+            if (int rc = launch_img_tn(st, img_dz[cur], img_h0, lay.WH, gr->kernel[0], 1, 128, 128, F, nullptr, gr->bias[0], F, Mb))
+                return rc;
         if (int rc = launch_img_nt(st, img_dz[cur], 128, ws + lay.off_wimg[0], lay.WF0, nullptr, 0, nullptr, gh0 + m0 * F, F, F, Mb)) return rc;
-        const int R = 256 / F;
-        bn_bwd_sums_kernel<<<grid_for(Mb, R * small_batch_rows(Mb, 64), 148 * 4), 256, 2 * F * sizeof(double), st>>>(
-            x_in + m0 * D, c ? c + m0 * C : nullptr, gh0 + m0 * F, Mb, D, C, cp->bn_mean, cp->bn_var, bn_sums);
+        if (bn_sums) {
+            const int R = 256 / F;
+            bn_bwd_sums_kernel<<<grid_for(Mb, R * small_batch_rows(Mb, 64), 148 * 4), 256, 2 * F * sizeof(double), st>>>(
+                x_in + m0 * D, c ? c + m0 * C : nullptr, gh0 + m0 * F, Mb, D, C, cp->bn_mean, cp->bn_var, bn_sums);
+            count_launch();
+        }
+    }
+    if (gr) {
+        unpad_add_kernel<<<grid_for((long long)(128 + 1) * d * P, 256, 148 * 4), 256, 0, st>>>(gWp, gbp, 128, d, P, NL, gr->kernel[L],
+                                                                                               gr->bias[L]);
         count_launch();
     }
-    unpad_add_kernel<<<grid_for((long long)(128 + 1) * d * P, 256, 148 * 4), 256, 0, st>>>(gWp, gbp, 128, d, P, NL, gr->kernel[L], gr->bias[L]);
-    count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;
 }
@@ -745,7 +839,7 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
                                     const float* x_in, const float* c, const float* gy, int32_t gy_rot, const float* glp,
                                     int64_t M, float* gx, float* gh0, double* bn_sums, void* workspace,
                                     size_t workspace_bytes, int64_t micro_batch) {
-    ZF_REQUIRE(cp && gr && x_in && gy && glp && gx && gh0 && bn_sums && workspace, "coupling_backward: null argument");
+    ZF_REQUIRE(cp && x_in && gy && glp && gx && gh0 && workspace, "coupling_backward: null argument");
     const int d = D / 2, F = D - d + C;
     ZF_REQUIRE(d > 0 && d < D && (C == 0 || c) && M >= 1 && micro_batch >= 1, "coupling_backward: bad shape");
     ZF_REQUIRE(F <= 256, "coupling_backward: at most 256 conditioner inputs");
@@ -754,7 +848,7 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
     if (workspace_bytes < lay.fixed_bytes + cpl_bwd_batch_bytes(cp, lay, D, C, std::min<long long>(micro_batch, M)))
         return fail(ZF_ERR_WORKSPACE, "coupling_backward: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
-    ZF_CUDA_CHECK(cudaMemsetAsync(bn_sums, 0, 2 * F * sizeof(double), st));
+    if (bn_sums) ZF_CUDA_CHECK(cudaMemsetAsync(bn_sums, 0, 2 * F * sizeof(double), st));
     if (lay.fused) {
         ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "coupling_backward: workspace must be 256-byte aligned");
         return coupling_backward_fused(st, cp, gr, D, C, x_in, c, gy, gy_rot, glp, M, gx, gh0, bn_sums, static_cast<char*>(workspace),
@@ -818,14 +912,16 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
         }
         // backward through the dense layers
         for (int l = L; l >= 0; --l) {
-            GemmArgs gw{};  // dW_l += act(Z_l)^T dZ_{l+1}; db_l += colsum(dZ_{l+1})
-            gw.A = act[l]; gw.lda = widths[l];
-            gw.B = act[l + 1]; gw.ldb = widths[l + 1];
-            gw.C = gr->kernel[l]; gw.ldc = widths[l + 1];
-            gw.colsum = gr->bias[l];
-            gw.a_swish = l > 0; gw.act = cp->act;
-            gw.I = widths[l]; gw.J = widths[l + 1]; gw.R = Mb; gw.r_slab = 2048;
-            if (int rc = launch_gemm(st, 2, gw)) return rc;
+            if (gr) {
+                GemmArgs gw{};  // dW_l += act(Z_l)^T dZ_{l+1}; db_l += colsum(dZ_{l+1})
+                gw.A = act[l]; gw.lda = widths[l];
+                gw.B = act[l + 1]; gw.ldb = widths[l + 1];
+                gw.C = gr->kernel[l]; gw.ldc = widths[l + 1];
+                gw.colsum = gr->bias[l];
+                gw.a_swish = l > 0; gw.act = cp->act;
+                gw.I = widths[l]; gw.J = widths[l + 1]; gw.R = Mb; gw.r_slab = 2048;
+                if (int rc = launch_gemm(st, 2, gw)) return rc;
+            }
             GemmArgs ga{};  // dZ_l = (dZ_{l+1} W_l^T) * swish'(Z_l)   (l = 0: d/d(BN output), no activation)
             ga.A = act[l + 1]; ga.lda = widths[l + 1];
             ga.B = cp->kernel[l]; ga.ldb = widths[l + 1];
@@ -834,10 +930,12 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
             ga.I = Mb; ga.J = widths[l]; ga.R = widths[l + 1];
             if (int rc = launch_gemm(st, 1, ga)) return rc;
         }
-        const int R = 256 / F;
-        bn_bwd_sums_kernel<<<grid_for(Mb, R * small_batch_rows(Mb, 64), 148 * 4), 256, 2 * F * sizeof(double), st>>>(
-            x_in + m0 * D, c ? c + m0 * C : nullptr, gh0 + m0 * F, Mb, D, C, cp->bn_mean, cp->bn_var, bn_sums);
-        count_launch();
+        if (bn_sums) {
+            const int R = 256 / F;
+            bn_bwd_sums_kernel<<<grid_for(Mb, R * small_batch_rows(Mb, 64), 148 * 4), 256, 2 * F * sizeof(double), st>>>(
+                x_in + m0 * D, c ? c + m0 * C : nullptr, gh0 + m0 * F, Mb, D, C, cp->bn_mean, cp->bn_var, bn_sums);
+            count_launch();
+        }
     }
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;
@@ -867,6 +965,35 @@ extern "C" int zf_bn_backward_apply(void* stream, const zf_coupling* cp, int32_t
     const int R = 256 / F;
     bn_bwd_apply_kernel<<<grid_for(M, R * small_batch_rows(M, 16), 148 * 16), 256, 5 * F * sizeof(float), (cudaStream_t)stream>>>(
         x_in, c, gh0, M, D, C, cp->bn_scale, cp->bn_mean, cp->bn_var, bn_sums, global_count, gx, gc);
+    count_launch();
+    ZF_CUDA_CHECK(cudaGetLastError());
+    return ZF_OK;
+}
+
+int zf::bn_backward_eval(cudaStream_t st, const zf_coupling* cp, int D, int C, const float* gh0, long long M, float* gx,
+                         float* gc) {
+    ZF_REQUIRE(cp && gh0 && gx && M >= 1, "bn_backward_eval: bad argument");
+    const int F = D - D / 2 + C;
+    bn_bwd_eval_kernel<<<grid_for(M * F, 256 * 8, 148 * 16), 256, F * sizeof(float), st>>>(gh0, M, D, C, cp->bn_scale,
+                                                                                           cp->bn_var, gx, gc);
+    count_launch();
+    ZF_CUDA_CHECK(cudaGetLastError());
+    return ZF_OK;
+}
+
+int zf::shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* x, const float* gz, int gz_rot,
+                              const float* glp, long long M, float* gx) {
+    ZF_REQUIRE(sb && x && gz && glp && gx && M >= 1 && D >= 1 && D <= ZF_MAX_DIM, "shift_bounds_backward: bad argument");
+    SbVjpCols cols{};
+    fill_cols(sb, D, cols.c);
+    bool running = false;
+    for (int i = 0; i < D; ++i) {
+        if (sb->kind[i] == ZF_BOUND_BOTH) cols.mul_both[i] = (float)(1.0 / (sb->hi[i] - sb->lo[i]));
+        else running = true;
+    }
+    ZF_REQUIRE(!running || (sb->xmin && sb->xmax), "shift_bounds_backward: xmin / xmax are NULL");
+    sb_bwd_kernel<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(cols, sb->xmin, sb->xmax, x, gz, ((gz_rot % D) + D) % D,
+                                                                       glp, M, D, gx);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;

@@ -2,7 +2,9 @@
 
 ``Flow.__call__`` (eval) is a single fused kernel launch: ShiftBounds, every coupling's
 conditioner MLP and spline, the Roll renamings, the latent log-pdf and nan_to_num
-(zf_flow_log_prob).  ``Flow.sample`` draws the latent on the device and runs the fused
+(zf_flow_log_prob).  When torch grad mode is on and x, c or a params leaf is a tensor that
+requires grad, the result is differentiable: its backward is one zf_flow_log_prob_vjp call
+(the running statistics stay fixed, as under jax.grad of the reference's eval call).  ``Flow.sample`` draws the latent on the device and runs the fused
 inverse chain (zf_chain_inverse).
 """
 from __future__ import annotations
@@ -12,7 +14,7 @@ from typing import Optional, Union
 import numpy as np
 import torch
 
-from ._chain import ChainSpec
+from ._chain import ChainSpec, _wants_grad, flow_log_prob_differentiable
 from ._device import like_input
 from .bijectors import Bijector, Chain, _cdim, _shape2
 from .distributions import Beta, Distribution
@@ -30,6 +32,12 @@ def _normalize_c(c):
     return c
 
 
+def _any_wants_grad(tree) -> bool:
+    if isinstance(tree, dict):
+        return any(_any_wants_grad(v) for v in tree.values())
+    return _wants_grad(tree)
+
+
 class Flow(Module):
     """A conditional normalizing flow (flow.py:16-95)."""
 
@@ -38,7 +46,11 @@ class Flow(Module):
         self.latent = latent
 
     def __call__(self, x, c=None, *, train: bool = False):
-        """Return log-likelihood of the samples: x (N, D), c (N, K) / (N,) / None -> (N,)."""
+        """Return log-likelihood of the samples: x (N, D), c (N, K) / (N,) / None -> (N,).
+
+        With ``train=False``, torch grad mode on, and x, c or a ``params`` leaf a tensor that requires grad, the result
+        is a CUDA tensor with a grad_fn (whatever the type of x): backward gives each of them its gradient in its own
+        device, dtype and shape, with the running statistics held fixed (the reference's jax.grad of this call)."""
         c = _normalize_c(c)
         D = _shape2(x)[1]
         self.latent._latch_dim(D)  # distributions.py:31-32 via latent.log_prob
@@ -49,8 +61,13 @@ class Flow(Module):
             return np.zeros(x.shape[0], np.float32)
         if not train:
             spec = ChainSpec(D, _cdim(c))
-            self.bijector._emit(spec, child)
             kind, peak = self.latent._native()
+            if torch.is_grad_enabled() and (_wants_grad(x) or _wants_grad(c) or _any_wants_grad(self.scope.subtree("params"))):
+                # differentiable: a CUDA tensor with a grad_fn whatever the type of x
+                with torch.no_grad():
+                    self.bijector._emit(spec, child)
+                return flow_log_prob_differentiable(spec, x, c, kind, peak)
+            self.bijector._emit(spec, child)
             return like_input(spec.log_prob(x, c, kind, peak), x)
         from . import _train
 
