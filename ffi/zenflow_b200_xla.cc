@@ -296,6 +296,47 @@ ffi::Error LogProbVjpImpl(cudaStream_t stream, ffi::ScratchAllocator scratch, F3
                                            gx.value()->typed_data(), gc, *ws, bytes, micro_batch));
 }
 
+// ---- jax.grad of Chain.inverse(z, c) (bijectors.py:113-116) or of Flow.sample's inverse pass (flow.py:76-77) -------
+// The backward rule of chain_inverse (sample = 0) and flow_sample (sample = 1).  Operands: z (M, D) (sample: a shape
+// carrier whose values are not read) [, c], the cotangent of x (M, D), the leaves.  Results: gz (M, D) (not when
+// sampling: the draw is a constant) [, gc (M, C)], then one cotangent per trainable leaf in op order.  The running
+// statistics are read, never written.
+ffi::Error InverseVjpImpl(cudaStream_t stream, ffi::ScratchAllocator scratch, F32 z, ffi::RemainingArgs rest,
+                          ffi::RemainingRets rets, ffi::Span<const int32_t> program, ffi::Span<const double> bounds,
+                          double margin, int32_t cdim, int32_t latent, float peakness, int64_t seed, int32_t sample,
+                          int64_t micro_batch) {
+    Shapes s;
+    const float* c;
+    if (auto e = ReadShapes(z, cdim, rest, &s, &c); e.failure()) return e;
+    int first = cdim > 0 ? 1 : 0;
+    auto ctb = rest.get<F32>(first++);
+    if (!ctb.has_value()) return Invalid("inverse_vjp: cotangent of x missing");
+    ChainStorage cs;
+    if (auto e = BuildChainFromLeaves(program, bounds, margin, s.D, s.C, rest, first, &cs); e.failure()) return e;
+    int r = 0;
+    float* gz = nullptr;
+    if (!sample) {
+        auto g = rets.get<F32>(r++);
+        if (!g.has_value()) return Invalid("result gz missing");
+        gz = g.value()->typed_data();
+    }
+    float* gc = nullptr;
+    if (cdim > 0) {
+        auto g = rets.get<F32>(r++);
+        if (!g.has_value()) return Invalid("result gc missing");
+        gc = g.value()->typed_data();
+    }
+    if (auto e = BindGradients(rets, r, &cs); e.failure()) return e;
+    ZeroGradients(cs, s.D, s.C, stream);
+    const size_t bytes = zf_chain_inverse_vjp_workspace_bytes(&cs.chain, s.M, micro_batch);
+    if (bytes == 0) return FromStatus(ZF_ERR_INVALID);
+    auto ws = scratch.Allocate(bytes, 256);
+    if (!ws.has_value()) return ffi::Error(ffi::ErrorCode::kResourceExhausted, "zenflow_b200: scratch allocation failed");
+    return FromStatus(zf_chain_inverse_vjp(stream, &cs.chain, cs.grads.empty() ? nullptr : cs.grads.data(),
+                                           sample ? nullptr : z.typed_data(), latent, peakness, (uint64_t)seed, c, s.M,
+                                           ctb.value().typed_data(), nullptr, gz, gc, *ws, bytes, micro_batch));
+}
+
 // ---- optimizer.update + optax.apply_updates on the flattened pytree, train.py:84-85 ------------------------------
 // params / mu / nu are aliased to the results (updated in place).
 ffi::Error NadamwImpl(cudaStream_t stream, F32 params, F32 grads, F32 mu, F32 nu, ffi::Result<F32> params_out, ffi::Result<F32> mu_out,
@@ -364,6 +405,19 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfFlowLogProbVjp, LogProbVjpImpl,
                                   .RemainingRets() ZF_CHAIN_ATTRS()
                                   .Attr<int32_t>("latent")
                                   .Attr<float>("peakness")
+                                  .Attr<int64_t>("micro_batch"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfChainInverseVjp, InverseVjpImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Ctx<ffi::ScratchAllocator>()
+                                  .Arg<F32>()
+                                  .RemainingArgs()
+                                  .RemainingRets() ZF_CHAIN_ATTRS()
+                                  .Attr<int32_t>("latent")
+                                  .Attr<float>("peakness")
+                                  .Attr<int64_t>("seed")
+                                  .Attr<int32_t>("sample")
                                   .Attr<int64_t>("micro_batch"));
 
 XLA_FFI_DEFINE_HANDLER_SYMBOL(ZfNadamwUpdate, NadamwImpl,

@@ -10,9 +10,10 @@ Calling convention = the header comment of ffi/zenflow_b200_xla.cc.
 reference call site                                   -> handler
   Flow.__call__(x, c, train=False)   flow.py:45-47    -> ZfFlowLogProb      (flow_log_prob, a jax.custom_vjp)
   jax.grad of it (wrt x, c, params)                   -> ZfFlowLogProbVjp   (its backward rule)
-  Chain.inverse(z, c)         bijectors.py:113-116    -> ZfChainInverse     (chain_inverse)
-  Flow.sample                        flow.py:50-78    -> ZfFlowSample       (flow_sample; Philox mode) or
-                                                         latent.sample (jax.random) + chain_inverse (parity mode)
+  Chain.inverse(z, c)         bijectors.py:113-116    -> ZfChainInverse     (chain_inverse, a jax.custom_vjp)
+  Flow.sample                        flow.py:50-78    -> ZfFlowSample       (flow_sample, a jax.custom_vjp; Philox mode)
+                                                         or latent.sample (jax.random) + chain_inverse (parity mode)
+  jax.grad of either (wrt z, c, params)               -> ZfChainInverseVjp  (their backward rule)
   Flow.__call__(train=True, mutable=["batch_stats"]) + jax.grad(loss_fn)   train.py:64-86
                                                       -> ZfFlowTrain        (flow_log_prob_train, a jax.custom_vjp)
   optimizer.update + apply_updates  train.py:84-85    -> ZfNadamwUpdate     (nadamw_update)
@@ -35,6 +36,7 @@ _TARGETS = {
     "zf_flow_log_prob_vjp": "ZfFlowLogProbVjp",
     "zf_chain_inverse": "ZfChainInverse",
     "zf_flow_sample": "ZfFlowSample",
+    "zf_chain_inverse_vjp": "ZfChainInverseVjp",
     "zf_flow_train": "ZfFlowTrain",
     "zf_nadamw_update": "ZfNadamwUpdate",
 }
@@ -234,21 +236,59 @@ def flow_log_prob(flow, variables, x, c=None, *, micro_batch: int = 1 << 18):
     return f(x, c, list(leaves))
 
 
-def chain_inverse(flow, variables, z, c=None):
-    """Chain.inverse(z, c), bijectors.py:113-116 (Flow.sample after latent.sample: bit-parity mode)."""
+def _inverse_custom_vjp(target, z_or_like, c, leaves, is_stat, attrs, extra, sample, micro_batch):
+    """The forward ffi call ``target`` wrapped in a jax.custom_vjp whose backward runs ZfChainInverseVjp (one
+    zf_chain_inverse_vjp call) with the running statistics held fixed; the statistics leaves get zero cotangents, and
+    z gets none when sampling (the draw is a constant)."""
     import jax
     import jax.numpy as jnp
+    import numpy as np
 
+    def _head(z, c):
+        return [z] if c is None else [z, c]
+
+    @jax.custom_vjp
+    def f(z, c, leaves):
+        call = jax.ffi.ffi_call(target, jax.ShapeDtypeStruct(z.shape, jnp.float32))
+        return call(*_head(z, c), *leaves, **attrs, **extra)
+
+    def f_fwd(z, c, leaves):
+        return f(z, c, leaves), (z, c, leaves)
+
+    def f_bwd(saved, ct_x):
+        z, c, leaves = saved
+        outs = [] if sample else [jax.ShapeDtypeStruct(z.shape, jnp.float32)]
+        outs += [] if c is None else [jax.ShapeDtypeStruct(c.shape, jnp.float32)]
+        outs += [jax.ShapeDtypeStruct(v.shape, jnp.float32) for v, s in zip(leaves, is_stat) if not s]
+        call = jax.ffi.ffi_call("zf_chain_inverse_vjp", outs)
+        lat = dict(latent=np.int32(0), peakness=np.float32(1.0), seed=np.int64(0))
+        lat.update(extra)
+        res = call(*_head(z, c), ct_x, *leaves, **attrs, **lat, sample=np.int32(1 if sample else 0),
+                   micro_batch=np.int64(micro_batch))
+        res = iter(res)
+        gz = jnp.zeros_like(z) if sample else next(res)
+        gc = None if c is None else next(res)
+        gp = res
+        gl = [jnp.zeros_like(v) if s else next(gp) for v, s in zip(leaves, is_stat)]
+        return gz, gc, gl
+
+    f.defvjp(f_fwd, f_bwd)
+    return f(z_or_like, c, list(leaves))
+
+
+def chain_inverse(flow, variables, z, c=None, *, micro_batch: int = 1 << 18):
+    """Chain.inverse(z, c), bijectors.py:113-116 (Flow.sample after latent.sample: bit-parity mode).
+
+    A jax.custom_vjp: jax.grad wrt z, c and the params leaves runs ZfChainInverseVjp (one zf_chain_inverse_vjp call)."""
     register()
-    head, leaves, _, _, attrs = _operands(flow, variables, z, c)
-    call = jax.ffi.ffi_call("zf_chain_inverse", jax.ShapeDtypeStruct(z.shape, jnp.float32))
-    return call(*head, *leaves, **attrs)
+    _, leaves, is_stat, _, attrs = _operands(flow, variables, z, c)
+    return _inverse_custom_vjp("zf_chain_inverse", z, c, leaves, is_stat, attrs, {}, False, micro_batch)
 
 
-def flow_sample(flow, variables, conditions_or_size, dim: int, *, seed: int = 0):
+def flow_sample(flow, variables, conditions_or_size, dim: int, *, seed: int = 0, micro_batch: int = 1 << 18):
     """Flow.sample, flow.py:50-78, with the latent drawn inside the kernel (Philox4x32-10; same distribution, not
-    the jax.random stream)."""
-    import jax
+    the jax.random stream).  A jax.custom_vjp: jax.grad wrt c and the params leaves (reparameterised samples) runs
+    ZfChainInverseVjp, which redraws the same latent."""
     import jax.numpy as jnp
     import numpy as np
 
@@ -260,9 +300,9 @@ def flow_sample(flow, variables, conditions_or_size, dim: int, *, seed: int = 0)
         c = c.reshape(-1, 1) if c.ndim == 1 else c  # flow.py:100-108 _normalize_c
         n = c.shape[0]
     like = jnp.zeros((n, dim), jnp.float32)  # shape carrier (values unread)
-    head, leaves, _, _, attrs = _operands(flow, variables, like, c)
-    call = jax.ffi.ffi_call("zf_flow_sample", jax.ShapeDtypeStruct((n, dim), jnp.float32))
-    return call(*head, *leaves, **attrs, **_latent(flow), seed=np.int64(seed))
+    _, leaves, is_stat, _, attrs = _operands(flow, variables, like, c)
+    extra = dict(_latent(flow), seed=np.int64(seed))
+    return _inverse_custom_vjp("zf_flow_sample", like, c, leaves, is_stat, attrs, extra, True, micro_batch)
 
 
 def make_flow_log_prob_train(flow, dim: int, cdim: int, *, global_count=None, micro_batch: int = 0):

@@ -371,6 +371,24 @@ int zf_flow_log_prob_vjp(void* stream, const zf_chain* chain, const zf_coupling_
                          float peakness, const float* x, const float* c, int64_t M, const float* lp_cotangent,
                          float* lp, float* gx, float* gc, void* workspace, size_t workspace_bytes, int64_t micro_batch);
 
+/* ---- VJP of Chain.inverse (bijectors.py:113-116) and of Flow.sample's inverse pass (flow.py:76-77) --------------
+ * What jax.grad through flow.apply(v, u, c, method="inverse") or method="sample" gives: the inverse is always eval-mode,
+ * so the running statistics are read, never written.  Same plan and loop as zf_flow_log_prob_vjp in inverse mode: the
+ * groups' inverses are recomputed last to first (one zf_chain_inverse per Roll run and per group), then the VJPs run first
+ * to last; the spline's is that of the analytic inverse as written (utils.py:191-201: no EPS, no clip).
+ *   chain         layout as for zf_flow_log_prob_vjp ([ShiftBounds]? (Coupling Roll*)*)
+ *   z (M,D)       the inverse's input; NULL: sample it from (latent_kind, peakness, seed) exactly as zf_flow_sample does
+ *   grads         as for zf_flow_log_prob_vjp (+=; NULL = input cotangents only)
+ *   x_cotangent   (M,D) required: the cotangent of the inverse's output x
+ *   x (M,D)       optional output: the inverse as recomputed by this call
+ *   gz (M,D)      optional output, overwritten: d/dz; must be NULL when z is NULL (the latent draw is a constant)
+ *   gc (M,C)      optional output, overwritten: d/dc */
+size_t zf_chain_inverse_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch);
+int zf_chain_inverse_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, const float* z,
+                         int32_t latent_kind, float peakness, uint64_t seed, const float* c, int64_t M,
+                         const float* x_cotangent, float* x, float* gz, float* gc,
+                         void* workspace, size_t workspace_bytes, int64_t micro_batch);
+
 /* ---- Deep-Set conditioner Phi (examples/deep_set.ipynb:138-160; SURVEY.md 8f-4) ---------------------------
  * The FLAX module on the other side of the flow's conditions in the deep_set config:
  *   BatchNorm_0 -> NNBlock_0 = (Dense_l + swish) x n_hidden, Dense_{n_hidden} (out_dim) -> Dropout(rate) -> sum_matrix @ .

@@ -1,4 +1,5 @@
-"""Host-side assembly of the native chain description (zf_chain), the eval calls and the VJP of the eval log-density.
+"""Host-side assembly of the native chain description (zf_chain), the eval calls and the VJPs of the eval log-density
+and of the inverse / sample pass.
 
 A ``ChainSpec`` is what the bijector modules emit: the op list of a Chain with device
 pointers to the FLAX variable leaves.  It owns the torch tensors behind those pointers for
@@ -194,24 +195,63 @@ class ChainSpec:
         gx = torch.empty_like(xd) if want_gx else None
         gc = torch.empty_like(cd) if (want_gc and cd is not None) else None
         lp = torch.empty(M, dtype=torch.float32, device=self.device) if want_lp else None
-        grads, arr = None, None
-        if want_params and self.coupling_params:
-            grads = [[torch.zeros_like(t) for t in dev] for _, dev in self.coupling_params]
-            arr = (_lib.ZfCouplingGrads * len(grads))()
-            for k, gl in enumerate(grads):
-                arr[k].bn_scale, arr[k].bn_bias = ptr(gl[0]), ptr(gl[1])
-                for j in range((len(gl) - 2) // 2):
-                    arr[k].kernel[j] = ptr(gl[2 + 2 * j])
-                    arr[k].bias[j] = ptr(gl[3 + 2 * j])
+        grads, arr = self._grads_array(want_params)
         _lib.check(lib.zf_flow_log_prob_vjp(stream_ptr(), C.byref(ch), arr, int(latent_kind), float(peakness), ptr(xd),
                                             ptr(cd), M, ptr(ct), ptr(lp), ptr(gx), ptr(gc), base,
                                             ws.numel() - (base - ws.data_ptr()), int(micro_batch)),
                    "zf_flow_log_prob_vjp")
         return gx, gc, grads, lp
 
-    def sample(self, n: int, c, latent_kind: int, peakness: float, seed: int):
-        """Flow.sample: latent draw inside the inverse chain kernel (zf_flow_sample)."""
+    def _grads_array(self, want_params: bool):
+        """Zeroed float32 gradient tensors of every coupling's parameters and the zf_coupling_grads array over them."""
+        if not (want_params and self.coupling_params):
+            return None, None
+        grads = [[torch.zeros_like(t) for t in dev] for _, dev in self.coupling_params]
+        arr = (_lib.ZfCouplingGrads * len(grads))()
+        for k, gl in enumerate(grads):
+            arr[k].bn_scale, arr[k].bn_bias = ptr(gl[0]), ptr(gl[1])
+            for j in range((len(gl) - 2) // 2):
+                arr[k].kernel[j] = ptr(gl[2 + 2 * j])
+                arr[k].bias[j] = ptr(gl[3 + 2 * j])
+        return grads, arr
+
+    def inverse_vjp(self, z, c, x_cotangent, *, draw=None, want_gz: bool = True, want_gc: bool = True,
+                    want_params: bool = True, micro_batch: int = 1 << 18, want_x: bool = False):
+        """VJP of Chain.inverse(z, c) (zf_chain_inverse_vjp) for the cotangent ``x_cotangent`` (M, D) of its output.
+        ``draw = (n, latent_kind, peakness, seed)`` differentiates Flow.sample's inverse pass instead: z is then the
+        latent draw zf_flow_sample makes (pass z=None; there is no gz).
+
+        Returns ``(gz, gc, param_grads, x)``: float32 device tensors, None where not asked for;
+        ``param_grads[k]`` lists coupling k's gradients in the order of ``coupling_params[k]``."""
         lib = _lib.load()
+        if draw is None:
+            zd, cd = self._inputs(z, c)
+            kind, peak, seed = 0, 1.0, 0
+        else:
+            n, kind, peak, seed = draw
+            zd, cd = None, self._conditions(int(n), c)
+            want_gz = False
+        M = int(zd.shape[0]) if zd is not None else int(draw[0])
+        ch = self._chain()
+        ct = to_device_f32(x_cotangent, self.device)
+        if tuple(ct.shape) != (M, self.dim):
+            raise ValueError(f"x_cotangent must have shape ({M}, {self.dim}), got {tuple(ct.shape)}")
+        nbytes = int(lib.zf_chain_inverse_vjp_workspace_bytes(C.byref(ch), M, int(micro_batch)))
+        if nbytes == 0:
+            _lib.check(1, "zf_chain_inverse_vjp_workspace_bytes")
+        ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
+        base = (ws.data_ptr() + 255) & ~255
+        gz = torch.empty((M, self.dim), dtype=torch.float32, device=self.device) if want_gz else None
+        gc = torch.empty_like(cd) if (want_gc and cd is not None) else None
+        x = torch.empty((M, self.dim), dtype=torch.float32, device=self.device) if want_x else None
+        grads, arr = self._grads_array(want_params)
+        _lib.check(lib.zf_chain_inverse_vjp(stream_ptr(), C.byref(ch), arr, ptr(zd), int(kind), float(peak),
+                                            int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(cd), M, ptr(ct), ptr(x), ptr(gz), ptr(gc),
+                                            base, ws.numel() - (base - ws.data_ptr()), int(micro_batch)),
+                   "zf_chain_inverse_vjp")
+        return gz, gc, grads, x
+
+    def _conditions(self, n: int, c):
         cd = None
         if self.cdim:
             if c is None:
@@ -221,6 +261,12 @@ class ChainSpec:
                 cd = cd.reshape(-1, 1)
             if cd.shape != (n, self.cdim):
                 raise ValueError(f"c must have shape ({n}, {self.cdim}), got {tuple(cd.shape)}")
+        return cd
+
+    def sample(self, n: int, c, latent_kind: int, peakness: float, seed: int):
+        """Flow.sample: latent draw inside the inverse chain kernel (zf_flow_sample)."""
+        lib = _lib.load()
+        cd = self._conditions(n, c)
         ch = self._chain()
         ws, nbytes = self._workspace(lib, ch, n)
         x = torch.empty((n, self.dim), dtype=torch.float32, device=self.device)
@@ -273,7 +319,55 @@ class _FlowLogProb(torch.autograd.Function):
 
 def flow_log_prob_differentiable(spec: ChainSpec, x, c, latent_kind: int, peakness: float) -> torch.Tensor:
     """The eval log-density with a grad_fn wrt every torch tensor among x, c and the couplings' params leaves."""
+    return _FlowLogProb.apply(spec, latent_kind, peakness, x, c, *_param_leaves(spec))
+
+
+class _FlowInverse(torch.autograd.Function):
+    """Chain.inverse(z, c) (``draw`` None) or Flow.sample's inverse pass (``draw = (n, latent_kind, peakness, seed)``,
+    z None) as a differentiable op: forward = zf_chain_inverse / zf_flow_sample (the non-grad calls, so x is
+    bit-identical to them), backward = one zf_chain_inverse_vjp with the incoming gradient as the cotangent of x.
+    ``leaves`` are the torch tensors among the couplings' params leaves, in ``spec.param_slots`` order."""
+
+    @staticmethod
+    def forward(ctx, spec, draw, z, c, *leaves):
+        if draw is None:
+            zd, cd = spec._inputs(z, c)
+            x = spec.inverse(zd, cd)
+        else:
+            zd, cd = None, spec._conditions(int(draw[0]), c)
+            x = spec.sample(int(draw[0]), cd, *draw[1:])
+        ctx.spec, ctx.draw = spec, draw
+        ctx.z_like = z.detach() if isinstance(z, torch.Tensor) else None
+        ctx.c_like = c.detach() if isinstance(c, torch.Tensor) else None
+        ctx.save_for_backward(zd, cd)
+        return x
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_x):
+        zd, cd = ctx.saved_tensors
+        spec = ctx.spec
+        need = ctx.needs_input_grad
+        gz, gc, grads, _ = spec.inverse_vjp(zd, cd, g_x, draw=ctx.draw, want_gz=need[2], want_gc=need[3],
+                                            want_params=any(need[4:]))
+        out_p = []
+        for i, (k, j) in enumerate(spec.param_slots):
+            out_p.append(_grad_like(grads[k][j], spec.coupling_params[k][0][j]) if need[4 + i] else None)
+        return (None, None, _grad_like(gz, ctx.z_like) if need[2] else None,
+                _grad_like(gc, ctx.c_like) if need[3] else None, *out_p)
+
+
+def _param_leaves(spec: ChainSpec) -> list:
     spec.param_slots = [(k, j) for k, (src, _) in enumerate(spec.coupling_params)
                         for j, leaf in enumerate(src) if isinstance(leaf, torch.Tensor)]
-    leaves = [spec.coupling_params[k][0][j] for k, j in spec.param_slots]
-    return _FlowLogProb.apply(spec, latent_kind, peakness, x, c, *leaves)
+    return [spec.coupling_params[k][0][j] for k, j in spec.param_slots]
+
+
+def flow_inverse_differentiable(spec: ChainSpec, z, c) -> torch.Tensor:
+    """Chain.inverse(z, c) with a grad_fn wrt every torch tensor among z, c and the couplings' params leaves."""
+    return _FlowInverse.apply(spec, None, z, c, *_param_leaves(spec))
+
+
+def flow_sample_differentiable(spec: ChainSpec, n: int, c, latent_kind: int, peakness: float, seed: int) -> torch.Tensor:
+    """Flow.sample's draw and inverse pass with a grad_fn wrt c and the couplings' params leaves (the draw is a constant)."""
+    return _FlowInverse.apply(spec, (int(n), int(latent_kind), float(peakness), int(seed)), None, c, *_param_leaves(spec))

@@ -169,6 +169,10 @@ SIGNATURES = {
     "zf_flow_log_prob_vjp": (C.c_int, [C.c_void_p, C.POINTER(ZfChain), C.POINTER(ZfCouplingGrads), C.c_int32, C.c_float,
                                        C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_size_t, C.c_int64]),
+    "zf_chain_inverse_vjp_workspace_bytes": (C.c_size_t, [C.POINTER(ZfChain), C.c_int64, C.c_int64]),
+    "zf_chain_inverse_vjp": (C.c_int, [C.c_void_p, C.POINTER(ZfChain), C.POINTER(ZfCouplingGrads), C.c_void_p, C.c_int32,
+                                       C.c_float, C.c_uint64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_size_t, C.c_int64]),
     "zf_phi_workspace_bytes": (C.c_size_t, [C.POINTER(ZfPhi), C.c_int64]),
     "zf_phi_forward": (C.c_int, [C.c_void_p, C.POINTER(ZfPhi), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
                                  C.c_int64, C.c_int32, C.c_float, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -787,38 +787,55 @@ __device__ __forceinline__ void vjp_activation(const ChainArgs& a, int layer, lo
 // ---- VJP row of the fused train kernel: theta from tensor memory -> cotangent of theta in this thread's row buffer
 // (row[0, 3 KT - 1), row[3 KT - 1] = 0).  Fast path: theta stays in registers (rqs_row_vjp_regs); rows with
 // |theta| >= kThetaFastBound, inf or NaN go through the IEEE path on the row buffer (rqs_row_backward).
-template <int KT, class Release>
+// INVERSE: the VJP of the spline inverse at y = x (no log-det), always on the row buffer (rqs_row_inverse_backward).
+template <int KT, bool INVERSE, class Release>
 __device__ __forceinline__ float vjp_row_tmem(uint32_t dbase, const float* __restrict__ bias, float* row, float x, float gy,
                                               float gld, Release release) {
     const KnotNorm kn = make_knot_norm(KT);
-    float pa[KT], pb[KT], wa[KT], wb[KT];
-    theta_block_issue<KT>(dbase, TC_XOFF, 0, pa, wa);
-    theta_block_issue<KT>(dbase, TC_XOFF, KT, pb, wb);
-    umma::wait_ld();
-    const float amax_w = theta_block_finish<KT>(0, bias, pa, wa);
-    const float amax_h = theta_block_finish<KT>(KT, bias, pb, wb);
-    theta_block_issue<KT>(dbase, TC_XOFF, 2 * KT, wa, wb);       // slopes: main in wa, cross in wb
-    umma::wait_ld();
-    release();                                                    // every TMEM read of this row is done
-    float amax_s = 0.f;
+    if constexpr (INVERSE) {
+        // the inverse row works on the row buffer: theta goes there one block at a time (three blocks of KT columns)
+        float p[KT], w[KT];
 #pragma unroll
-    for (int j = 0; j < KT; ++j) {
-        wa[j] = fmaf(wb[j], umma::kF16LoUnscale, wa[j]) + bias[2 * KT + j];
-        if (j < KT - 1) amax_s = fmaxf(amax_s, fabsf(wa[j]));
-    }
-    const bool slow = !(fmaxf(fmaxf(amax_w, amax_h), amax_s) < kThetaFastBound) || !(amax_s == amax_s);
-    if (__any_sync(0xffffffffu, slow)) {
+        for (int blk = 0; blk < 3; ++blk) {
+            theta_block_issue<KT>(dbase, TC_XOFF, blk * KT, p, w);
+            umma::wait_ld();
+            if (blk == 2) release();                                  // every TMEM read of this row is done
 #pragma unroll
-        for (int j = 0; j < KT; ++j) { row[j] = pa[j]; row[KT + j] = pb[j]; row[2 * KT + j] = wa[j]; }
-        const float g = rqs_row_backward<KT>(row, KT, x, gy, gld, kn);
+            for (int j = 0; j < KT; ++j) row[blk * KT + j] = fmaf(w[j], umma::kF16LoUnscale, p[j]) + bias[blk * KT + j];
+        }
+        const float g = rqs_row_inverse_backward<KT>(row, KT, x, gy, kn);
+        row[3 * KT - 1] = 0.f;
+        return g;
+    } else {
+        float pa[KT], pb[KT], wa[KT], wb[KT];
+        theta_block_issue<KT>(dbase, TC_XOFF, 0, pa, wa);
+        theta_block_issue<KT>(dbase, TC_XOFF, KT, pb, wb);
+        umma::wait_ld();
+        const float amax_w = theta_block_finish<KT>(0, bias, pa, wa);
+        const float amax_h = theta_block_finish<KT>(KT, bias, pb, wb);
+        theta_block_issue<KT>(dbase, TC_XOFF, 2 * KT, wa, wb);       // slopes: main in wa, cross in wb
+        umma::wait_ld();
+        release();                                                    // every TMEM read of this row is done
+        float amax_s = 0.f;
+#pragma unroll
+        for (int j = 0; j < KT; ++j) {
+            wa[j] = fmaf(wb[j], umma::kF16LoUnscale, wa[j]) + bias[2 * KT + j];
+            if (j < KT - 1) amax_s = fmaxf(amax_s, fabsf(wa[j]));
+        }
+        const bool slow = !(fmaxf(fmaxf(amax_w, amax_h), amax_s) < kThetaFastBound) || !(amax_s == amax_s);
+        if (__any_sync(0xffffffffu, slow)) {
+#pragma unroll
+            for (int j = 0; j < KT; ++j) { row[j] = pa[j]; row[KT + j] = pb[j]; row[2 * KT + j] = wa[j]; }
+            const float g = rqs_row_backward<KT>(row, KT, x, gy, gld, kn);
+            row[3 * KT - 1] = 0.f;
+            return g;
+        }
+#pragma unroll
+        for (int j = 0; j < KT - 1; ++j) row[j] = wa[j];
+        const float g = rqs_row_vjp_regs<KT>(pa, pb, row, x, gy, gld, kn);
         row[3 * KT - 1] = 0.f;
         return g;
     }
-#pragma unroll
-    for (int j = 0; j < KT - 1; ++j) row[j] = wa[j];
-    const float g = rqs_row_vjp_regs<KT>(pa, pb, row, x, gy, gld, kn);
-    row[3 * KT - 1] = 0.f;
-    return g;
 }
 
 // ---- the epilogue / SIMT role of the tensor-core chain kernel ------------------------------------------------
@@ -861,7 +878,6 @@ __device__ __forceinline__ void activation_store(uint32_t tb, uint32_t lane_base
 
 template <bool INVERSE, bool VJP = false>
 __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
-    static_assert(!(INVERSE && VJP), "the VJP kernel recomputes the forward conditioner");
     constexpr int NG = 2;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int q = warp & 3, half = warp >> 2, m = q * 32 + lane;   // half = column group g in [0, NG)
@@ -1177,7 +1193,7 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                 float* wrows = reinterpret_cast<float*>(cx.scratch) + ((size_t)half * UM + q * 32) * VJP_ROW;   // this warp's 32 rows
                 float* row = wrows + lane * VJP_ROW;
                 const KnotNorm kn = make_knot_norm(K);
-                const float gld = m < nm ? a.glp[m0 + m] : 0.f;
+                const float gld = (!INVERSE && m < nm) ? a.glp[m0 + m] : 0.f;   // the inverse has no log-det
                 float gy_next = (half < d && m < nm) ? a.gy[(m0 + m) * D + pmod(half + a.gy_rot, D)] : 0.f;
                 for (int jj = half; jj < d; jj += 2) {
                     const float gyv = gy_next;
@@ -1194,8 +1210,8 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                     };
                     const float xv = xs[pmod(jj - rot, D) * UM + m];
                     float g_x;
-                    if (K == 16) g_x = vjp_row_tmem<16>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
-                    else g_x = vjp_row_tmem<32>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
+                    if (K == 16) g_x = vjp_row_tmem<16, INVERSE>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
+                    else g_x = vjp_row_tmem<32, INVERSE>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
                     ZF_TR(trs);   // row cotangent done
                     if (m < nm) a.gx[(m0 + m) * D + jj] = g_x;
                     {   // this thread's row -> the event-row image: 16-byte units of 8 columns, hi and lo parts; the 32 lanes of a
@@ -1922,7 +1938,9 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         if (l == 1 && nslots == 2) {
                             // While the first hidden GEMM finishes: the BatchNorm of the next occurrence.  It belongs
                             // to the other tile of the pair (or to the next pair), whose state does not depend on
-                            // anything this occurrence still has to produce, so waiting for it here cannot deadlock.
+                            // anything this occurrence still has to produce, so waiting for it here cannot deadlock
+                            // (the row warps publish a tile of the next pair as soon as they are through the first
+                            // coupling of the tile it replaces).
                             long long pn = p;
                             int cjn = cj, sn = 1;
                             if (slot == 1) { sn = 0; if (++cjn == ncoup) { cjn = 0; ++pn; } }
@@ -2076,6 +2094,10 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                     }
                     // as soon as this tile's state is complete for its next coupling, tell the activation warps
                     if (si + 1 < a.n_steps && step_at(si + 1).kind == kStepKindCoupling) signal_ready(k);
+                    // the tile that takes this slot in the next pair: its buffers were released two pairs ago.  It is
+                    // published here, not after both slots: the activation warps may wait for it while they still owe
+                    // this pair's other slot (in a chain of one coupling, before that slot's spline rows can run).
+                    if (si == fc) preamble(k + 2);
                     if (si == a.n_steps - 1) {
                         // ---- store this tile
                         if (a.mode == kModeLogProb) {
@@ -2098,10 +2120,6 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                             s2_barrier();
                         }
                     }
-                }
-                if (si == fc) {   // the next pair's tiles: their buffers were released two pairs ago
-                    preamble(2 * (p + 1));
-                    preamble(2 * (p + 1) + 1);
                 }
             }
         }
@@ -2308,8 +2326,10 @@ struct ChainLaunch {
 //   !tc, impl == umma                                                                ZF_ERR_UNSUPPORTED
 //   fits(FFMA tile)        (a tc chain beyond the single-tile kernel's memory too)   chain_kernel
 //   otherwise                                                                        ZF_ERR_UNSUPPORTED
-// and the VJP of one coupling (vjp, the plan of vjp_plan):
-//   tc, fits(single-tile VJP)   chain_umma_kernel<false, true>;   otherwise kNone (zf_coupling_backward's unfused path)
+// and the VJP of one coupling (vjp, the plan of vjp_plan), of its forward or of its inverse (the same plan, packing and
+// shared memory; only the spline row differs):
+//   tc, fits(single-tile VJP)   chain_umma_kernel<false, true> (forward) / <true, true> (inverse);
+//   otherwise                   kNone (the unfused path of coupling_backward: spline_bwd_kernel<K, false | true>)
 // The constant blocks are laid out by build_plan, before the device is known: for tc couplings with Fmax <= 16 they carry
 // the first Dense's operand image (Plan::w0img: first Dense on the tensor cores), except in the eval passes of flows
 // whose couplings all transform one dim.  Those take the two-tile kernel, whose first Dense is FFMA, and keep the FFMA
@@ -2431,7 +2451,8 @@ static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int l
 }
 
 // ---- fused conditioner recompute + spline VJP of ONE coupling (tensor-core path of zf_coupling_backward) ---------
-// The coupling is planned and packed as a chain of one op; the kernel is chain_umma_kernel<false, true>.
+// The coupling is planned and packed as a chain of one op; the kernel is chain_umma_kernel<false, true>, or
+// chain_umma_kernel<true, true> for the VJP of the coupling's inverse (x_in is then the inverse's input, glp unused).
 static int vjp_plan(const zf_coupling* cp, int D, int C, Plan& plan, zf_op& op, zf_chain& chain) {
     op = zf_op{};
     op.kind = ZF_OP_COUPLING;
@@ -2469,7 +2490,7 @@ int coupling_vjp_pack(cudaStream_t stream, const zf_coupling* cp, int D, int C, 
 
 int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, const float* ws, const float* x_in, const float* c,
                      const float* gy, int gy_rot, const float* glp, long long M, float* gx, void* img_h0, int wh0, void* const* img_act,
-                     float* const* act_g, void* img_dtheta) {
+                     float* const* act_g, void* img_dtheta, bool inverse) {
     Plan plan;
     zf_op op;
     zf_chain chain;
@@ -2498,10 +2519,11 @@ int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, c
     ChainLaunch k;
     if (int rc = choose_chain_kernel(plan, di, true, impl_switch().chain, &k)) return rc;
     ZF_REQUIRE(k.kernel == ChainKernel::kUmmaVjp, "coupling_vjp: the coupling does not take the fused kernel (coupling_vjp_ws_floats is 0)");
-    if (int rc = smem_optin((const void*)chain_umma_kernel<false, true>, k.smem)) return rc;
+    auto kern = inverse ? chain_umma_kernel<true, true> : chain_umma_kernel<false, true>;
+    if (int rc = smem_optin((const void*)kern, k.smem)) return rc;
     const long long tiles = (M + UM - 1) / UM;
     if (tiles == 0) return ZF_OK;
-    chain_umma_kernel<false, true><<<(unsigned)std::min<long long>(tiles, (long long)di.sm_count), 320, k.smem, stream>>>(a);
+    kern<<<(unsigned)std::min<long long>(tiles, (long long)di.sm_count), 320, k.smem, stream>>>(a);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;

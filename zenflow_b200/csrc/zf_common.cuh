@@ -73,13 +73,21 @@ struct GemmArgs {
 // Runs one product; the only place that chooses between the three GEMM kernels (the table is at its definition).
 int launch_gemm(cudaStream_t st, int mode, const GemmArgs& g);
 
-// Fused conditioner recompute + spline VJP of one coupling (zf_chain.cu).  ws_floats is 0 when the coupling or the
-// device does not take the fused kernel.
+// Fused conditioner recompute + spline VJP of one coupling (zf_chain.cu), of its forward or (inverse) of its inverse.
+// ws_floats is 0 when the coupling or the device does not take the fused kernel.
 size_t coupling_vjp_ws_floats(const zf_coupling* cp, int D, int C);
 int coupling_vjp_pack(cudaStream_t stream, const zf_coupling* cp, int D, int C, float* ws);
 int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, const float* ws, const float* x_in, const float* c,
                      const float* gy, int gy_rot, const float* glp, long long M, float* gx, void* img_h0, int wh0, void* const* img_act,
-                     float* const* act_g, void* img_dtheta);
+                     float* const* act_g, void* img_dtheta, bool inverse);
+
+// zf_coupling_backward (zf_train.cu) for either direction.  inverse = false: the VJP of the coupling's forward, as the
+// public entry.  inverse = true: the VJP of NeuralSplineCoupling.inverse (bijectors.py:367-371) with x_in its input (the
+// forward's output), gy the cotangent of its output read at column (j + gy_rot) % D, glp unused (no log-det); gx is the
+// cotangent of x_in.  The BatchNorm running statistics are constants either way (the inverse is always eval-mode).
+int coupling_backward(cudaStream_t st, const zf_coupling* cp, const zf_coupling_grads* gr, int D, int C, const float* x_in,
+                      const float* c, const float* gy, int gy_rot, const float* glp, long long M, float* gx, float* gh0,
+                      double* bn_sums, void* workspace, size_t workspace_bytes, long long micro_batch, bool inverse);
 
 // One weight image of pack_w_images (zf_img_gemm.cu): Wimg(n, k) = W[n * ldw + (k / NL) * P + k % NL] for n < n_valid and
 // k % NL < P, else 0, as the bf16x2 hi | lo operand image of img_nt_kernel.  block0 / blocks are filled by the launcher.
@@ -115,6 +123,11 @@ int bn_backward_eval(cudaStream_t st, const zf_coupling* cp, int D, int C, const
 // and of its log-det (cotangent glp), with the running sb->xmin / sb->xmax.
 int shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* x, const float* gz, int gz_rot,
                           const float* glp, long long M, float* gx);
+// VJP of ShiftBounds.inverse (bijectors.py:210-240) with the running sb->xmin / sb->xmax: gz (M, D) = d/dz for the
+// cotangent gx of its output x.  dx/dz is b - a (both bounds), xmax - xmin (running statistics), exp(t) (xmax - xmin)
+// (lower bound) or -exp(t) (xmax - xmin) (upper bound), t = z xmax + (1 - z) xmin.
+int shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* z, const float* gx, long long M,
+                                  float* gz);
 
 // ---- PTX wrappers ----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

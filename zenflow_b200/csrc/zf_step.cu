@@ -14,6 +14,15 @@
 // Eval mode runs the same plan and the same loop (run_step) with three differences: no statistics phase (the
 // couplings and the ShiftBounds read their running statistics), the diagonal BatchNorm VJP instead of the
 // batch-coupled one, and the backward continues through a leading ShiftBounds into d/dx.
+//
+// zf_chain_inverse_vjp: the VJP of Chain.inverse (bijectors.py:113-116) and of Flow.sample's inverse pass (flow.py:76-77),
+// the inverse mode of the same plan and loop.  Chain.inverse walks the groups last to first, a group's inverse being its
+// Rolls' inverses and then the coupling's (or the ShiftBounds') inverse, always with the running statistics:
+//   forward   per group, last to first: u_g = Roll^-1(input) (zf_chain_inverse on the Rolls; in sample mode the first
+//             pass draws the latent, zf_flow_sample), then the group's own inverse from u_g; u_g is kept
+//   backward  per group, first to last (the cotangent travels from x toward z): the ShiftBounds' inverse VJP, or the
+//             coupling's (conditioner recompute + spline-inverse VJP + Dense VJPs) and the diagonal BatchNorm VJP;
+//             the cotangent of u_g reaches the next group's output through its Rolls by index arithmetic.
 #include "zf_common.cuh"
 
 #include <algorithm>
@@ -29,13 +38,16 @@ struct StepGroup {
     std::vector<zf_op> ops;   // the group's sub-chain
 };
 
+// train: value_and_grad; eval: log_prob_vjp; inverse: chain_inverse_vjp
+enum StepMode { kStepTrain, kStepEval, kStepInverse };
+
 struct StepPlan {
     std::vector<StepGroup> groups;
     int n_couplings = 0;
     int Fmax = 1;
     // workspace carve-up in bytes
     size_t off_states = 0, off_ld = 0, off_glp = 0, off_ga = 0, off_gb = 0, off_gh0 = 0, off_stats = 0, off_chain = 0,
-           off_bwd = 0, off_lp_sum = 0, total = 0;
+           off_bwd = 0, off_lp_sum = 0, off_xtmp = 0, total = 0;
     size_t stats_stride = 0, chain_bytes = 0, bwd_bytes = 0;
 };
 
@@ -45,8 +57,11 @@ static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // the ShiftBounds group uses the same block for minmax[2D] (float) | scratch[2D] (uint32).
 // Eval mode uses only the bwd sums (parameter gradients of the BatchNorm) and adds a slot for the lp sum the loss
 // kernel keeps; it also accepts a chain with no coupling, whose only derivative is d/dx through the ShiftBounds.
-static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, bool train, StepPlan& p) {
-    const char* who = train ? "value_and_grad" : "log_prob_vjp";
+// Inverse mode uses the states for u_g, the input of group g's own inverse, and adds one (M, D) buffer for the outputs
+// that are not states (x_g when group g-1 has Rolls, and x when the caller does not ask for it).
+static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, StepMode mode, StepPlan& p) {
+    const bool train = mode == kStepTrain;
+    const char* who = train ? "value_and_grad" : mode == kStepEval ? "log_prob_vjp" : "chain_inverse_vjp";
     ZF_REQUIRE(chain && chain->n_ops >= 1 && chain->ops, "%s: empty chain", who);
     const int D = chain->dim, C = chain->cdim;
     ZF_REQUIRE(D >= (train ? 2 : 1) && D <= ZF_MAX_DIM, "%s: dim must be in [%d, %d]", who, train ? 2 : 1, ZF_MAX_DIM);
@@ -95,7 +110,8 @@ static int build_step_plan(const zf_chain* chain, long long M, long long micro_b
     }
     p.off_chain = take(p.chain_bytes);
     p.off_bwd = take(p.bwd_bytes);
-    if (!train) p.off_lp_sum = take(sizeof(double));
+    if (mode == kStepEval) p.off_lp_sum = take(sizeof(double));
+    if (mode == kStepInverse) p.off_xtmp = take((size_t)M * D * 4);
     p.total = off;
     return ZF_OK;
 }
@@ -117,10 +133,11 @@ static int aux_events(AuxEvents** out) {
     return ZF_OK;
 }
 
-// The arguments of either entry point.  Train-only fields (global_count, lp_sum, the communicators and buckets) are
-// unused in eval mode; gx (d/dx) is eval-only.
+// The arguments of the three entry points.  Train-only fields (global_count, lp_sum, the communicators and buckets) are
+// unused in eval mode; gx (d/dx) is eval-only.  Inverse mode reads x as z (NULL: sample with latent_kind, peakness, seed),
+// x_ct as the cotangent of its output, writes x_out (optional) and gz (optional), and uses none of the loss fields.
 struct StepCall {
-    bool train;
+    StepMode mode;
     cudaStream_t st, aux;
     const zf_chain* chain;
     const zf_coupling_grads* grads;
@@ -141,11 +158,19 @@ struct StepCall {
     const int64_t* bucket_off;
     char* ws;
     long long micro_batch;
+    const float* x_ct;
+    float* x_out;
+    float* gz;
+    unsigned long long seed;
 };
 
-// One plan, one loop: the forward per group, the loss cotangents, the backward per group in reverse.
+static int pmod_rot(int r, int D) { return ((r % D) + D) % D; }
+
+// One plan, one loop: the forward per group, the loss cotangents, the backward per group in reverse.  In inverse mode the
+// forward visits the groups last to first, there is no loss, and the backward visits them first to last.
 static int run_step(StepPlan& p, const StepCall& a) {
-    const bool train = a.train;
+    const bool train = a.mode == kStepTrain, inv = a.mode == kStepInverse;
+    const size_t G = p.groups.size();
     const int D = a.chain->dim, C = a.chain->cdim, F = D - D / 2 + C;
     cudaStream_t st = a.st;
     char* ws = a.ws;
@@ -163,15 +188,38 @@ static int run_step(StepPlan& p, const StepCall& a) {
     auto state = [&](size_t g) { return reinterpret_cast<float*>(ws + p.off_states + g * (size_t)M * D * 4); };
     auto stats = [&](size_t g) { return ws + p.off_stats + g * p.stats_stride; };
 
-    ZF_CUDA_CHECK(cudaMemsetAsync(ld, 0, (size_t)M * 4, st));
+    if (!inv) ZF_CUDA_CHECK(cudaMemsetAsync(ld, 0, (size_t)M * 4, st));
     if (a.gc && C) ZF_CUDA_CHECK(cudaMemsetAsync(a.gc, 0, (size_t)M * C * 4, st));
 
     // ---- forward, one bijector group at a time (in train mode the batch statistics couple the events)
-    std::vector<zf_coupling> batch_cp(p.groups.size());   // couplings reading the BATCH statistics (train mode)
+    std::vector<zf_coupling> batch_cp(G);    // couplings reading the BATCH statistics (train mode)
+    std::vector<const float*> u_in(G);       // inverse mode: the input of each group's own inverse
+    float* xtmp = reinterpret_cast<float*>(ws + p.off_xtmp);
     const float* cur = x;
-    for (size_t gi = 0; gi < p.groups.size(); ++gi) {
+    for (size_t k = 0; k < G; ++k) {
+        const size_t gi = inv ? G - 1 - k : k;
         StepGroup& g = p.groups[gi];
         float* nxt = state(gi);
+        if (inv) {
+            // Roll^-1 of the group's input (the latent draw for the first pass when sampling) into u_g, then the group's
+            // own inverse into the next state (x_g is u_{g-1} when group g-1 has no Rolls) or into the output buffer
+            zf_chain rolls{D, 0, (int32_t)g.ops.size() - 1, g.ops.data() + 1};
+            if (!x && k == 0) {
+                if (int rc = zf_flow_sample(st, &rolls, a.latent_kind, a.peakness, a.seed, nullptr, M, nxt, chain_ws, p.chain_bytes))
+                    return rc;
+                u_in[gi] = nxt;
+            } else if (pmod_rot(g.rot, D) != 0) {
+                if (int rc = zf_chain_inverse(st, &rolls, cur, nullptr, M, nxt, chain_ws, p.chain_bytes)) return rc;
+                u_in[gi] = nxt;
+            } else {
+                u_in[gi] = cur;
+            }
+            float* out = gi == 0 ? (a.x_out ? a.x_out : xtmp) : pmod_rot(p.groups[gi - 1].rot, D) != 0 ? xtmp : state(gi - 1);
+            zf_chain own{D, C, 1, g.ops.data()};
+            if (int rc = zf_chain_inverse(st, &own, u_in[gi], c, M, out, chain_ws, p.chain_bytes)) return rc;
+            cur = out;
+            continue;
+        }
         if (!train) {
             // the chain's own ShiftBounds and couplings: running statistics, read only
         } else if (g.kind == ZF_OP_SHIFT_BOUNDS) {
@@ -202,11 +250,13 @@ static int run_step(StepPlan& p, const StepCall& a) {
     }
 
     // ---- loss and the cotangents of z and of the log-dets (flow.py:46-47, train.py:73)
-    double* lp_sum = train ? a.lp_sum : reinterpret_cast<double*>(ws + p.off_lp_sum);
-    if (int rc = flow_loss_grad(st, a.latent_kind, a.peakness, cur, ld, M, D, a.global_count, a.lp_cotangent, a.lp, gy, glp,
-                                lp_sum, train ? 0 : 1))
-        return rc;
-    if (train && !a.grads) return ZF_OK;
+    if (!inv) {
+        double* lp_sum = train ? a.lp_sum : reinterpret_cast<double*>(ws + p.off_lp_sum);
+        if (int rc = flow_loss_grad(st, a.latent_kind, a.peakness, cur, ld, M, D, a.global_count, a.lp_cotangent, a.lp, gy, glp,
+                                    lp_sum, train ? 0 : 1))
+            return rc;
+        if (train && !a.grads) return ZF_OK;
+    }
 
     // ---- backward
     const bool bucketed = a.dp_comm && a.grad_flat;
@@ -214,8 +264,38 @@ static int run_step(StepPlan& p, const StepCall& a) {
     AuxEvents* ev = nullptr;
     if (overlap)
         if (int rc = aux_events(&ev)) return rc;
-    for (size_t gi = p.groups.size(); gi-- > 0;) {
+    const float* g_in = a.x_ct;   // inverse mode: the cotangent of the current group's output, read at (j + g_rot) % D
+    int g_rot = 0;
+    for (size_t k = 0; k < G; ++k) {
+        const size_t gi = inv ? k : G - 1 - k;
         StepGroup& g = p.groups[gi];
+        if (inv) {
+            // the cotangent of u_g; the last group's goes straight to gz when its Rolls are the identity
+            const bool last = gi + 1 == G;
+            float* dst = (last && a.gz && pmod_rot(g.rot, D) == 0) ? a.gz : gy;
+            if (g.kind == ZF_OP_SHIFT_BOUNDS) {
+                if (int rc = shift_bounds_inverse_backward(st, g.ops[0].shift_bounds, D, u_in[gi], g_in, M, dst)) return rc;
+            } else {
+                const zf_coupling* cp = g.ops[0].coupling;
+                const zf_coupling_grads* gr = a.grads ? &a.grads[g.coupling_index] : nullptr;
+                double* bsums = gr ? reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8)) + 2 * F : nullptr;
+                if (int rc = coupling_backward(st, cp, gr, D, C, u_in[gi], c, g_in, g_rot, nullptr, M, dst, gh0, bsums, bwd_ws,
+                                               p.bwd_bytes, mb, true))
+                    return rc;
+                if (gr)
+                    if (int rc = zf_bn_param_grads(st, bsums, F, gr->bn_scale, gr->bn_bias)) return rc;
+                if (int rc = bn_backward_eval(st, cp, D, C, gh0, M, dst, a.gc)) return rc;
+            }
+            // the group's output u_g is rolled into the next group's input: its cotangent is read back through the Rolls
+            if (last && a.gz && dst != a.gz) {
+                zf_chain rolls{D, 0, (int32_t)g.ops.size() - 1, g.ops.data() + 1};
+                if (int rc = zf_chain_forward(st, &rolls, dst, nullptr, M, a.gz, nullptr, chain_ws, p.chain_bytes)) return rc;
+            }
+            g_in = dst;
+            g_rot = pmod_rot(-g.rot, D);
+            std::swap(gy, gx);
+            continue;
+        }
         const float* x_in = gi == 0 ? x : state(gi - 1);
         float* dst = (gi == 0 && a.gx) ? a.gx : gx;   // the cotangent of x goes straight to the caller's buffer
         if (g.kind != ZF_OP_COUPLING) {
@@ -228,7 +308,7 @@ static int run_step(StepPlan& p, const StepCall& a) {
         const zf_coupling_grads* gr = a.grads ? &a.grads[g.coupling_index] : nullptr;
         // sum gh0 and sum gh0 xhat: the BatchNorm's parameter gradients, and in train mode also its input VJP
         double* bsums = gr ? reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8)) + 2 * F : nullptr;
-        if (int rc = zf_coupling_backward(st, cp, gr, D, C, x_in, c, gy, g.rot, glp, M, dst, gh0, bsums, bwd_ws, p.bwd_bytes, mb))
+        if (int rc = coupling_backward(st, cp, gr, D, C, x_in, c, gy, g.rot, glp, M, dst, gh0, bsums, bwd_ws, p.bwd_bytes, mb, false))
             return rc;
         if (gr)
             if (int rc = zf_bn_param_grads(st, bsums, F, gr->bn_scale, gr->bn_bias)) return rc;
@@ -265,7 +345,7 @@ using namespace zf;
 
 extern "C" size_t zf_flow_value_and_grad_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
     StepPlan p;
-    if (build_step_plan(chain, M, micro_batch, true, p) != ZF_OK) return 0;
+    if (build_step_plan(chain, M, micro_batch, kStepTrain, p) != ZF_OK) return 0;
     return p.total;
 }
 
@@ -275,7 +355,7 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
                                       void* dp_comm, void* dp_grad_comm, float* grad_flat, const int64_t* bucket_off,
                                       void* workspace, size_t workspace_bytes, int64_t micro_batch) {
     StepPlan p;
-    if (int rc = build_step_plan(chain, M, micro_batch, true, p)) return rc;
+    if (int rc = build_step_plan(chain, M, micro_batch, kStepTrain, p)) return rc;
     ZF_REQUIRE(x && lp_sum && workspace, "value_and_grad: null argument");
     ZF_REQUIRE(chain->cdim == 0 || c, "value_and_grad: chain has cdim=%d but c is NULL", chain->cdim);
     ZF_REQUIRE(global_count >= 1, "value_and_grad: global_count must be >= 1");
@@ -283,7 +363,7 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
     ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "value_and_grad: workspace must be 256-byte aligned");
     if (workspace_bytes < p.total)
         return fail(ZF_ERR_WORKSPACE, "value_and_grad: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
-    StepCall a{true, (cudaStream_t)stream, (cudaStream_t)aux_stream, chain, grads, latent_kind, peakness, x, c, M,
+    StepCall a{kStepTrain, (cudaStream_t)stream, (cudaStream_t)aux_stream, chain, grads, latent_kind, peakness, x, c, M,
                global_count, lp_cotangent, lp, lp_sum, nullptr, gc, dp_comm, dp_grad_comm, grad_flat, bucket_off,
                static_cast<char*>(workspace), micro_batch};
     return run_step(p, a);
@@ -291,7 +371,7 @@ extern "C" int zf_flow_value_and_grad(void* stream, void* aux_stream, const zf_c
 
 extern "C" size_t zf_flow_log_prob_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
     StepPlan p;
-    if (build_step_plan(chain, M, micro_batch, false, p) != ZF_OK) return 0;
+    if (build_step_plan(chain, M, micro_batch, kStepEval, p) != ZF_OK) return 0;
     return p.total;
 }
 
@@ -300,14 +380,42 @@ extern "C" int zf_flow_log_prob_vjp(void* stream, const zf_chain* chain, const z
                                     float* lp, float* gx, float* gc, void* workspace, size_t workspace_bytes,
                                     int64_t micro_batch) {
     StepPlan p;
-    if (int rc = build_step_plan(chain, M, micro_batch, false, p)) return rc;
+    if (int rc = build_step_plan(chain, M, micro_batch, kStepEval, p)) return rc;
     ZF_REQUIRE(x && lp_cotangent && workspace, "log_prob_vjp: null argument");
     ZF_REQUIRE(chain->cdim == 0 || c, "log_prob_vjp: chain has cdim=%d but c is NULL", chain->cdim);
     ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "log_prob_vjp: workspace must be 256-byte aligned");
     if (workspace_bytes < p.total)
         return fail(ZF_ERR_WORKSPACE, "log_prob_vjp: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
     // the cotangent is given, so the count that scales the train loss plays no part
-    StepCall a{false, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, x, c, M, 1.0, lp_cotangent, lp,
+    StepCall a{kStepEval, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, x, c, M, 1.0, lp_cotangent, lp,
                nullptr, gx, gc, nullptr, nullptr, nullptr, nullptr, static_cast<char*>(workspace), micro_batch};
+    return run_step(p, a);
+}
+
+extern "C" size_t zf_chain_inverse_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
+    StepPlan p;
+    if (build_step_plan(chain, M, micro_batch, kStepInverse, p) != ZF_OK) return 0;
+    return p.total;
+}
+
+extern "C" int zf_chain_inverse_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, const float* z,
+                                    int32_t latent_kind, float peakness, uint64_t seed, const float* c, int64_t M,
+                                    const float* x_cotangent, float* x, float* gz, float* gc, void* workspace,
+                                    size_t workspace_bytes, int64_t micro_batch) {
+    StepPlan p;
+    if (int rc = build_step_plan(chain, M, micro_batch, kStepInverse, p)) return rc;
+    ZF_REQUIRE(x_cotangent && workspace, "chain_inverse_vjp: null argument");
+    ZF_REQUIRE(chain->cdim == 0 || c, "chain_inverse_vjp: chain has cdim=%d but c is NULL", chain->cdim);
+    ZF_REQUIRE(z || !gz, "chain_inverse_vjp: gz must be NULL when sampling (z is NULL): the latent draw is a constant");
+    if (!z) {
+        ZF_REQUIRE(latent_kind >= 0 && latent_kind <= 3, "chain_inverse_vjp: unknown latent kind %d", latent_kind);
+        ZF_REQUIRE(latent_kind != ZF_LATENT_BETA || peakness >= 1.f, "chain_inverse_vjp: peakness must be at least 1");
+    }
+    ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "chain_inverse_vjp: workspace must be 256-byte aligned");
+    if (workspace_bytes < p.total)
+        return fail(ZF_ERR_WORKSPACE, "chain_inverse_vjp: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
+    StepCall a{kStepInverse, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, z, c, M, 1.0, nullptr, nullptr,
+               nullptr, nullptr, gc, nullptr, nullptr, nullptr, nullptr, static_cast<char*>(workspace), micro_batch,
+               x_cotangent, x, gz, (unsigned long long)seed};
     return run_step(p, a);
 }

@@ -10,7 +10,8 @@
 //   zf_shift_bounds_minmax / _update   <- bijectors.py:250-260
 //   zf_bn_moments / zf_bn_finalize      <- flax BatchNorm(use_running_average=False), bijectors.py:342
 //   zf_flow_loss_grad                   <- flow.py:46-47 + train.py:73 (-mean) and d/dz of the latent
-//   zf_coupling_backward                <- VJP of bijectors.py:329-365 (conditioner recompute + spline VJP)
+//   zf_coupling_backward                <- VJP of bijectors.py:329-365 (conditioner recompute + spline VJP), and
+//                                          of the coupling's inverse, bijectors.py:367-371 (coupling_backward)
 //   zf_bn_backward_apply                <- VJP of train-mode BatchNorm into x and c
 //   zf_nadamw_update                    <- optax.nadamw / adamw (train.py:12-15,84-85)
 #include "zf_common.cuh"
@@ -345,6 +346,32 @@ __global__ void __launch_bounds__(256) sb_bwd_kernel(const __grid_constant__ SbV
     }
 }
 
+// VJP of ShiftBounds.inverse (forward: shift_bounds_row<true> in zf_chain.cu, bijectors.py:210-240); cols.mul_both holds
+// (float)(b - a) of the ZF_BOUND_BOTH columns here
+__global__ void __launch_bounds__(256) sb_inv_bwd_kernel(const __grid_constant__ SbVjpCols cols, const float* __restrict__ xmin,
+                                                         const float* __restrict__ xmax, const float* __restrict__ z,
+                                                         const float* __restrict__ gx, long long M, int D, float* __restrict__ gz) {
+    const long long n = M * D;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+        const int i = (int)(e % D);
+        const int kind = cols.c.kind[i];
+        const float g = gx[e];
+        float r;
+        if (kind == ZF_BOUND_BOTH) {
+            r = g * cols.mul_both[i];
+        } else {
+            const float lo = xmin[i], hi = xmax[i], span = hi - lo;
+            r = g * span;
+            if (kind != ZF_BOUND_NONE) {
+                const float v = z[e];
+                const float t = __fadd_rn(__fmul_rn(v, hi), __fmul_rn(__fsub_rn(1.f, v), lo));   // as the chain's inverse
+                r *= (kind == ZF_BOUND_LOWER) ? expf(t) : -expf(t);
+            }
+        }
+        gz[e] = r;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // loss and latent gradient
 // ---------------------------------------------------------------------------------------------
@@ -385,7 +412,8 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
 
 // ---------------------------------------------------------------------------------------------
 // spline VJP: theta row -> d(theta) row in place; d/dx of the transformed columns; pass-through
-// of the conditioning columns' cotangent
+// of the conditioning columns' cotangent.  INVERSE: the VJP of the spline inverse, x_in is the inverse's input y and
+// glp is not read.
 // ---------------------------------------------------------------------------------------------
 struct SplineBwdArgs {
     float* theta;          // (Mb, d, P) in: raw params, out: their cotangent
@@ -411,7 +439,7 @@ __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.w
 
 // theta tiles stream HBM -> smem ring (bulk copies) -> in-place VJP, one thread per (sample, dim) row ->
 // HBM (bulk store); same pipeline shape as rqs_stage_kernel.
-template <int KT>
+template <int KT, bool INVERSE>
 __global__ void __launch_bounds__(256) spline_bwd_kernel(const __grid_constant__ SplineBwdArgs a) {
     extern __shared__ __align__(128) float sm[];
     const int tid = threadIdx.x;
@@ -464,7 +492,8 @@ __global__ void __launch_bounds__(256) spline_bwd_kernel(const __grid_constant__
             const long long m = a.m0 + s0 + sidx;
             const float x = a.x_in[m * D + jj];
             const float gy = a.gy[m * D + (jj + a.rot) % D];
-            a.gx[m * D + jj] = rqs_row_backward<KT>(buf + (size_t)r * P, K, x, gy, a.glp[m], kn);
+            a.gx[m * D + jj] = INVERSE ? rqs_row_inverse_backward<KT>(buf + (size_t)r * P, K, x, gy, kn)
+                                       : rqs_row_backward<KT>(buf + (size_t)r * P, K, x, gy, a.glp[m], kn);
         }
         // conditioning columns pass through unchanged: d y[:, j] / d x[:, j] = 1   (bijectors.py:364)
         for (int e = tid; e < ns * (D - d); e += 256) {
@@ -766,7 +795,7 @@ __global__ void __launch_bounds__(256) unpad_add_kernel(const float* __restrict_
 // Fused path of zf_coupling_backward (see CplBwdLayout).
 static int coupling_backward_fused(cudaStream_t st, const zf_coupling* cp, const zf_coupling_grads* gr, int D, int C, const float* x_in,
                                    const float* c, const float* gy, int gy_rot, const float* glp, long long M, float* gx, float* gh0,
-                                   double* bn_sums, char* ws, long long micro_batch, const CplBwdLayout& lay) {
+                                   double* bn_sums, char* ws, long long micro_batch, const CplBwdLayout& lay, bool inverse) {
     const int d = D / 2, F = D - d + C, K = cp->knots, P = 3 * K - 1, L = cp->n_hidden, NL = lay.NL, TW = lay.TW;
     float* pack = reinterpret_cast<float*>(ws);
     float* gWp = reinterpret_cast<float*>(ws + lay.off_gwp);
@@ -797,8 +826,8 @@ static int coupling_backward_fused(cudaStream_t st, const zf_coupling* cp, const
             act_g[l] = reinterpret_cast<float*>(take(img_bytes(Mb, 128)));   // fp32 tile image: whole tiles
         }
         // BatchNorm, conditioner (theta in tensor memory), spline VJP: writes gx and the images
-        if (int rc = coupling_vjp_run(st, cp, D, C, pack, x_in + m0 * D, c ? c + m0 * C : nullptr, gy + m0 * D, gy_rot, glp + m0, Mb,
-                                      gx + m0 * D, img_h0, lay.WH, img_act, act_g, img_dt))
+        if (int rc = coupling_vjp_run(st, cp, D, C, pack, x_in + m0 * D, c ? c + m0 * C : nullptr, gy + m0 * D, gy_rot,
+                                      glp ? glp + m0 : nullptr, Mb, gx + m0 * D, img_h0, lay.WH, img_act, act_g, img_dt, inverse))
             return rc;
         // last Dense (padded column space): dW_L, db_L, dZ_L = (dTheta W_L^T) swish'(Z_L)
         if (gr)
@@ -835,11 +864,10 @@ static int coupling_backward_fused(cudaStream_t st, const zf_coupling* cp, const
     return ZF_OK;
 }
 
-extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const zf_coupling_grads* gr, int32_t D, int32_t C,
-                                    const float* x_in, const float* c, const float* gy, int32_t gy_rot, const float* glp,
-                                    int64_t M, float* gx, float* gh0, double* bn_sums, void* workspace,
-                                    size_t workspace_bytes, int64_t micro_batch) {
-    ZF_REQUIRE(cp && x_in && gy && glp && gx && gh0 && workspace, "coupling_backward: null argument");
+int zf::coupling_backward(cudaStream_t st, const zf_coupling* cp, const zf_coupling_grads* gr, int D, int C, const float* x_in,
+                          const float* c, const float* gy, int gy_rot, const float* glp, long long M, float* gx, float* gh0,
+                          double* bn_sums, void* workspace, size_t workspace_bytes, long long micro_batch, bool inverse) {
+    ZF_REQUIRE(cp && x_in && gy && (glp || inverse) && gx && gh0 && workspace, "coupling_backward: null argument");
     const int d = D / 2, F = D - d + C;
     ZF_REQUIRE(d > 0 && d < D && (C == 0 || c) && M >= 1 && micro_batch >= 1, "coupling_backward: bad shape");
     ZF_REQUIRE(F <= 256, "coupling_backward: at most 256 conditioner inputs");
@@ -847,12 +875,11 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
     const CplBwdLayout lay = cpl_bwd_layout(cp, D, C);
     if (workspace_bytes < lay.fixed_bytes + cpl_bwd_batch_bytes(cp, lay, D, C, std::min<long long>(micro_batch, M)))
         return fail(ZF_ERR_WORKSPACE, "coupling_backward: workspace too small");
-    cudaStream_t st = (cudaStream_t)stream;
     if (bn_sums) ZF_CUDA_CHECK(cudaMemsetAsync(bn_sums, 0, 2 * F * sizeof(double), st));
     if (lay.fused) {
         ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "coupling_backward: workspace must be 256-byte aligned");
         return coupling_backward_fused(st, cp, gr, D, C, x_in, c, gy, gy_rot, glp, M, gx, gh0, bn_sums, static_cast<char*>(workspace),
-                                       micro_batch, lay);
+                                       micro_batch, lay, inverse);
     }
     DeviceInfo di;
     if (int rc = get_device_info(&di)) return rc;
@@ -866,7 +893,8 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
     if (2 * (2 * tile_bytes + 256) + 2048 <= (size_t)di.max_smem_optin) { sp_stages = 2; sp_bps = 2; }
     if (sp_stages < 1) return fail(ZF_ERR_UNSUPPORTED, "coupling_backward: spline tile does not fit shared memory");
     const size_t sp_smem = (size_t)sp_stages * tile_bytes + 64;
-    auto sp_kernel = (K == 16) ? spline_bwd_kernel<16> : (K == 32) ? spline_bwd_kernel<32> : spline_bwd_kernel<0>;
+    auto sp_kernel = inverse ? ((K == 16) ? spline_bwd_kernel<16, true> : (K == 32) ? spline_bwd_kernel<32, true> : spline_bwd_kernel<0, true>)
+                             : ((K == 16) ? spline_bwd_kernel<16, false> : (K == 32) ? spline_bwd_kernel<32, false> : spline_bwd_kernel<0, false>);
     if (int rc = smem_optin((const void*)sp_kernel, sp_smem)) return rc;
 
     float* ws = static_cast<float*>(workspace);
@@ -941,6 +969,14 @@ extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const z
     return ZF_OK;
 }
 
+extern "C" int zf_coupling_backward(void* stream, const zf_coupling* cp, const zf_coupling_grads* gr, int32_t D, int32_t C,
+                                    const float* x_in, const float* c, const float* gy, int32_t gy_rot, const float* glp,
+                                    int64_t M, float* gx, float* gh0, double* bn_sums, void* workspace,
+                                    size_t workspace_bytes, int64_t micro_batch) {
+    return coupling_backward((cudaStream_t)stream, cp, gr, D, C, x_in, c, gy, gy_rot, glp, M, gx, gh0, bn_sums, workspace,
+                             workspace_bytes, micro_batch, false);
+}
+
 __global__ void bn_param_grads_kernel(const double* sums, int F, float* gscale, float* gbias) {
     int f = threadIdx.x;
     if (f < F) {
@@ -994,6 +1030,23 @@ int zf::shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D,
     ZF_REQUIRE(!running || (sb->xmin && sb->xmax), "shift_bounds_backward: xmin / xmax are NULL");
     sb_bwd_kernel<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(cols, sb->xmin, sb->xmax, x, gz, ((gz_rot % D) + D) % D,
                                                                        glp, M, D, gx);
+    count_launch();
+    ZF_CUDA_CHECK(cudaGetLastError());
+    return ZF_OK;
+}
+
+int zf::shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* z, const float* gx,
+                                      long long M, float* gz) {
+    ZF_REQUIRE(sb && z && gx && gz && M >= 1 && D >= 1 && D <= ZF_MAX_DIM, "shift_bounds_inverse_backward: bad argument");
+    SbVjpCols cols{};
+    fill_cols(sb, D, cols.c);
+    bool running = false;
+    for (int i = 0; i < D; ++i) {
+        if (sb->kind[i] == ZF_BOUND_BOTH) cols.mul_both[i] = cols.c.hi[i] - cols.c.lo[i];
+        else running = true;
+    }
+    ZF_REQUIRE(!running || (sb->xmin && sb->xmax), "shift_bounds_inverse_backward: xmin / xmax are NULL");
+    sb_inv_bwd_kernel<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(cols, sb->xmin, sb->xmax, z, gx, M, D, gz);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;

@@ -1,6 +1,6 @@
-// VJP of normalize_spline_params + rational_quadratic_spline_forward (utils.py:37-141) for one (event, dim) row:
-// shared by the stage-style kernel of zf_train.cu (theta from HBM) and the fused conditioner-recompute kernel of
-// zf_chain.cu (theta from tensor memory).  Derivation: SURVEY.md Appendix A.
+// VJP of normalize_spline_params + rational_quadratic_spline_forward (utils.py:37-141) and of the analytic inverse
+// (utils.py:144-202) for one (event, dim) row: shared by the stage-style kernel of zf_train.cu (theta from HBM) and the
+// fused conditioner-recompute kernel of zf_chain.cu (theta from tensor memory).  Derivation: SURVEY.md Appendix A.
 #pragma once
 #include "zf_math.cuh"
 
@@ -65,24 +65,13 @@ __device__ __forceinline__ void rqs_scalar_adjoints(float x, float gy, float gld
     g_w -= g_s * s / w;
 }
 
-// row: raw theta (3K-1) in shared memory, overwritten by its cotangent.  Returns d/dx.
-// KT > 0: K known at compile time (loops unrolled); KT == 0: runtime K.
+// Cotangent of raw theta from the cotangents of what one bin gathers (normalize_spline_params, utils.py:37-62): the
+// widths block gets g_xk (knots left of the bin) and g_w (the bin), the heights block g_yk and g_h, the slopes g_d0 and
+// g_d1 at the bin's two inner knots.  idx < K is the bin.  row: raw theta (3K-1) in, its cotangent out.
 template <int KT>
-__device__ __forceinline__ float rqs_row_backward(float* row, int K_rt, float x, float gy, float gld, const KnotNorm& kn) {
+__device__ __forceinline__ void rqs_theta_adjoints(float* row, int K_rt, int idx, const KnotNorm& kn, float g_xk, float g_w,
+                                                   float g_yk, float g_h, float g_d0, float g_d1) {
     const int K = KT > 0 ? KT : K_rt;
-    RqsBin b;
-    rqs_locate<KT>(row, K, true, x, kn, b);
-    const int P = 3 * K - 1;
-    const bool oob = (x < 0.f) || (x >= 1.f);
-    const int idx = b.idx;
-    if (oob || idx >= K || !(x == x)) {  // identity branch (or the reference's NaN corner): no parameter gradient
-        for (int p = 0; p < P; ++p) row[p] = 0.f;
-        return oob ? gy : 0.f;
-    }
-    const float xk = b.ks, w = b.bs, h = b.bo, d0 = b.dk, d1 = b.dkp1;
-    float g_x, g_xk, g_w, g_yk, g_h, g_d0, g_d1;
-    rqs_scalar_adjoints(x, gy, gld, xk, w, h, d0, d1, g_x, g_xk, g_w, g_yk, g_h, g_d0, g_d1);
-
     // slopes first (their raw values are needed before the row is overwritten)
     const float c_lo = (idx >= 1) ? row[2 * K + idx - 1] : 0.f;
     const float c_hi = (idx + 1 <= K - 1) ? row[2 * K + idx] : 0.f;
@@ -134,7 +123,93 @@ __device__ __forceinline__ float rqs_row_backward(float* row, int K_rt, float x,
     for (int j = 0; j < K - 1; ++j) row[2 * K + j] = 0.f;
     if (idx >= 1) row[2 * K + idx - 1] = g_d0 * squareplus_grad(c_lo);
     if (idx + 1 <= K - 1) row[2 * K + idx] = g_d1 * squareplus_grad(c_hi);
+}
+
+// row: raw theta (3K-1) in shared memory, overwritten by its cotangent.  Returns d/dx.
+// KT > 0: K known at compile time (loops unrolled); KT == 0: runtime K.
+template <int KT>
+__device__ __forceinline__ float rqs_row_backward(float* row, int K_rt, float x, float gy, float gld, const KnotNorm& kn) {
+    const int K = KT > 0 ? KT : K_rt;
+    RqsBin b;
+    rqs_locate<KT>(row, K, true, x, kn, b);
+    const int P = 3 * K - 1;
+    const bool oob = (x < 0.f) || (x >= 1.f);
+    const int idx = b.idx;
+    if (oob || idx >= K || !(x == x)) {  // identity branch (or the reference's NaN corner): no parameter gradient
+        for (int p = 0; p < P; ++p) row[p] = 0.f;
+        return oob ? gy : 0.f;
+    }
+    const float xk = b.ks, w = b.bs, h = b.bo, d0 = b.dk, d1 = b.dkp1;
+    float g_x, g_xk, g_w, g_yk, g_h, g_d0, g_d1;
+    rqs_scalar_adjoints(x, gy, gld, xk, w, h, d0, d1, g_x, g_xk, g_w, g_yk, g_h, g_d0, g_d1);
+    rqs_theta_adjoints<KT>(row, K, idx, kn, g_xk, g_w, g_yk, g_h, g_d0, g_d1);
     return g_x;
+}
+
+// Adjoints of the analytic inverse (utils.py:191-201, rqs_eval_inverse): y -> x inside bin [yk, yk + h) x [xk, xk + w)
+// with knot derivatives d0, d1; gx is the cotangent of x.  The formula is differentiated as written (a quadratic root,
+// no EPS, no clip), which is what jax.grad of the reference's inverse gives; it is not 1 / (dy/dx) of the forward.
+__device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, float yk, float h, float xk, float w, float d0,
+                                                            float d1, float& g_y, float& g_yk, float& g_h, float& g_xk, float& g_w,
+                                                            float& g_d0, float& g_d1) {
+    const float s = h / w;
+    const float dy = y - yk;
+    const float beta = d1 + d0 - 2.0f * s;
+    const float a = h * (s - d0) + dy * beta;
+    const float bq = h * d0 - dy * beta;
+    const float c = -s * dy;
+    const float sq = sqrtf(bq * bq - 4.0f * a * c);
+    const float Dq = -bq - sq;
+    const float z = 2.0f * c / Dq;
+    // x = z w + xk,  z = 2c / Dq,  Dq = -bq - sqrt(bq^2 - 4ac)
+    g_xk = gx;
+    g_w = gx * z;
+    const float g_z = gx * w;
+    float g_c = g_z * 2.0f / Dq;
+    const float g_Dq = -g_z * z / Dq;
+    const float g_disc = -g_Dq * 0.5f / sq;
+    const float g_bq = -g_Dq + g_disc * 2.0f * bq;
+    const float g_a = -g_disc * 4.0f * c;
+    g_c -= g_disc * 4.0f * a;
+    // c = -s dy;  bq = h d0 - dy beta;  a = h (s - d0) + dy beta;  beta = d1 + d0 - 2 s
+    float g_s = -g_c * dy;
+    float g_dy = -g_c * s;
+    g_h = g_bq * d0 + g_a * (s - d0);
+    g_d0 = g_bq * h - g_a * h;
+    g_dy += (g_a - g_bq) * beta;
+    const float g_beta = (g_a - g_bq) * dy;
+    g_s += g_a * h;
+    g_d1 = g_beta;
+    g_d0 += g_beta;
+    g_s -= 2.0f * g_beta;
+    // dy = y - yk;  s = h / w
+    g_y = g_dy;
+    g_yk = -g_dy;
+    g_h += g_s / w;
+    g_w -= g_s * s / w;
+}
+
+// The VJP of normalize_spline_params + rational_quadratic_spline_inverse (utils.py:144-202) on a row: raw theta (3K-1)
+// in shared memory, overwritten by its cotangent; gx is the cotangent of x.  Returns d/dy.  The bin is searched in the
+// heights, as the eval inverse searches it.  Conventions as rqs_row_backward: identity branch (y outside [0, 1)):
+// d/dy = gx and no parameter gradient; the reference's NaN corner (past the last knot, NaN input): zero gradients.
+template <int KT>
+__device__ __forceinline__ float rqs_row_inverse_backward(float* row, int K_rt, float y, float gx, const KnotNorm& kn) {
+    const int K = KT > 0 ? KT : K_rt;
+    RqsBin b;
+    rqs_locate<KT>(row, K, false, y, kn, b);
+    const int P = 3 * K - 1;
+    const bool oob = (y < 0.f) || (y >= 1.f);
+    const int idx = b.idx;
+    if (oob || idx >= K || !(y == y)) {
+        for (int p = 0; p < P; ++p) row[p] = 0.f;
+        return oob ? gx : 0.f;
+    }
+    const float yk = b.ks, h = b.bs, xk = b.ko, w = b.bo, d0 = b.dk, d1 = b.dkp1;
+    float g_y, g_yk, g_h, g_xk, g_w, g_d0, g_d1;
+    rqs_scalar_inverse_adjoints(y, gx, yk, h, xk, w, d0, d1, g_y, g_yk, g_h, g_xk, g_w, g_d0, g_d1);
+    rqs_theta_adjoints<KT>(row, K, idx, kn, g_xk, g_w, g_yk, g_h, g_d0, g_d1);
+    return g_y;
 }
 
 // The same VJP with theta in registers (the fused conditioner-recompute kernel reads it from tensor memory) and the

@@ -4,8 +4,10 @@
 conditioner MLP and spline, the Roll renamings, the latent log-pdf and nan_to_num
 (zf_flow_log_prob).  When torch grad mode is on and x, c or a params leaf is a tensor that
 requires grad, the result is differentiable: its backward is one zf_flow_log_prob_vjp call
-(the running statistics stay fixed, as under jax.grad of the reference's eval call).  ``Flow.sample`` draws the latent on the device and runs the fused
-inverse chain (zf_chain_inverse).
+(the running statistics stay fixed, as under jax.grad of the reference's eval call).  ``Flow.sample`` draws the latent
+on the device and runs the fused inverse chain (zf_flow_sample); ``Flow.inverse`` runs it on a given draw
+(zf_chain_inverse).  Both are differentiable in the same way, wrt c and the params leaves (and u for ``inverse``): the
+backward is one zf_chain_inverse_vjp call.
 """
 from __future__ import annotations
 
@@ -14,7 +16,8 @@ from typing import Optional, Union
 import numpy as np
 import torch
 
-from ._chain import ChainSpec, _wants_grad, flow_log_prob_differentiable
+from ._chain import (ChainSpec, _wants_grad, flow_inverse_differentiable, flow_log_prob_differentiable,
+                     flow_sample_differentiable)
 from ._device import like_input
 from .bijectors import Bijector, Chain, _cdim, _shape2
 from .distributions import Beta, Distribution
@@ -80,7 +83,12 @@ class Flow(Module):
         Return type: like every entry point of the package the result mirrors the input - numpy conditions give a
         numpy array, torch conditions a CUDA tensor.  An int size has nothing to mirror: the samples stay on the
         device (CUDA ``torch.Tensor``), as for ``Distribution.sample``.  ``as_numpy=True`` / ``False`` overrides
-        either way (``flow.apply(v, 1000, method="sample", as_numpy=True)`` for host-side plotting code)."""
+        either way (``flow.apply(v, 1000, method="sample", as_numpy=True)`` for host-side plotting code).
+
+        With torch grad mode on and c or a ``params`` leaf a tensor that requires grad, the samples are differentiable
+        (reparameterised: x = T^-1(z; c, params) with the draw z a constant): the result is then a CUDA tensor with a
+        grad_fn whatever the type of the conditions, unless ``as_numpy=True``, which still returns a detached host
+        array."""
         if isinstance(conditions_or_size, (int, np.integer)):
             size = int(conditions_or_size)
             c = None
@@ -92,8 +100,13 @@ class Flow(Module):
         from .distributions import _seed_of
 
         spec = ChainSpec(self.latent.dim, _cdim(c))
-        self.bijector._emit(spec, self.scope.child("bijector"))
         kind, peak = self.latent._native()
+        if as_numpy is not True and torch.is_grad_enabled() and (
+                _wants_grad(c) or _any_wants_grad(self.scope.subtree("params"))):
+            with torch.no_grad():
+                self.bijector._emit(spec, self.scope.child("bijector"))
+            return flow_sample_differentiable(spec, size, c, kind, peak, _seed_of(seed))
+        self.bijector._emit(spec, self.scope.child("bijector"))
         # latent.sample(size, PRNGKey(seed)) and bijector.inverse in one fused pass (flow.py:76-77)
         x = spec.sample(size, c, kind, peak, _seed_of(seed))
         if as_numpy is None:
@@ -102,9 +115,16 @@ class Flow(Module):
 
     def inverse(self, u, c=None):
         """bijector.inverse(u, c) with the latent draw given (flow.py:77); the parity-mode
-        counterpart of ``sample`` since jax.random streams cannot be reproduced here."""
+        counterpart of ``sample`` since jax.random streams cannot be reproduced here.
+
+        With torch grad mode on and u, c or a ``params`` leaf a tensor that requires grad, the result is a CUDA tensor
+        with a grad_fn (whatever the type of u), differentiable wrt each of them with the running statistics fixed."""
         c = _normalize_c(c)
         spec = ChainSpec(_shape2(u)[1], _cdim(c))
+        if torch.is_grad_enabled() and (_wants_grad(u) or _wants_grad(c) or _any_wants_grad(self.scope.subtree("params"))):
+            with torch.no_grad():
+                self.bijector._emit(spec, self.scope.child("bijector"))
+            return flow_inverse_differentiable(spec, u, c)
         self.bijector._emit(spec, self.scope.child("bijector"))
         return like_input(spec.inverse(u, c), u)
 
