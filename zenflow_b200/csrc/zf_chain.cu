@@ -610,7 +610,7 @@ constexpr int USTEPS = 40;   // step descriptors kept in shared memory (longer p
 constexpr int VJP_ROW = 97;   // floats per theta row of the VJP kernel (odd: one thread per row without bank conflicts)
 __host__ __device__ inline size_t umma_hs_floats(int Fmax) { return (size_t)Fmax * UM; }   // x - mean, [Fmax][UM]
 __host__ __device__ inline size_t umma_smem_floats(int D, int C, int Fmax, int Hmax, int BLmax, bool vjp = false, bool img = false) {
-    return 2 * (size_t)UM * (D + C) + umma_hs_floats(Fmax) + (vjp ? 1 : 2) * (size_t)ucst_layout(Fmax, Hmax, BLmax, img).total + 11 * UM +
+    return 2 * (size_t)UM * (D + C) + umma_hs_floats(Fmax) + (vjp ? 1 : 2) * (size_t)ucst_layout(Fmax, Hmax, BLmax, img).total + 3 * UM +
            (vjp ? 2 * UM * VJP_ROW : 2 * 8 * UM * 4) +
            (size_t)URING * URING_FLOATS + 2 * B_COUNT + 32 + USTEPS * sizeof(StepDesc) / sizeof(float);
 }
@@ -660,9 +660,9 @@ __device__ __forceinline__ float theta_block_finish(int col, const float* __rest
 // (rows are issue-bound: ~1.3k instead of ~1.9k instructions for K = 32).  The three raw blocks are loaded in a software
 // pipeline (the next block's TMEM load is in flight while the current one is processed) and the D buffer is handed
 // back to the MMA warp (release()) right after the last load.  Bins are bit-identical to the IEEE path
-// (rqs_block_search<KT, true>); the other-axis knot, the bin height / width and the knot derivatives are
+// (rqs_block_search<KT>); the other-axis knot, the bin height / width and the knot derivatives are
 // fp32-tolerance quantities either way.  scr: this thread's scratch column (float4, stride apart, KT / 4 entries).
-// Rows with |theta| >= kThetaFastBound (or inf) take the IEEE path (rqs_block_search / rqs_block_other<KT, true>).
+// Rows with |theta| >= kThetaFastBound (or inf) take the IEEE path (rqs_block_search / rqs_block_other).
 template <int KT>
 __device__ __forceinline__ float theta_block_finish_lean(int col, const float* __restrict__ bias, float (&p)[KT],
                                                          const float (&w)[KT]) {
@@ -685,66 +685,16 @@ __device__ __forceinline__ void spline_row_tmem_lean(uint32_t dbase, uint32_t cr
     const float amax_s = theta_block_finish_lean<KT>(cs_, bias, pa, wa);
     theta_block_issue<KT>(dbase, cross_off, co_, pb, wb);          // in flight during the search pass
     const bool slow_s = __any_sync(0xffffffffu, !(amax_s < kThetaFastBound));
-    RqsCheck chk;
-    if (slow_s) rqs_block_search<KT, true>(pa, v, kn, b.idx, b.ks, b.bs, chk);
+    if (slow_s) rqs_block_search<KT>(pa, v, kn, b.idx, b.ks, b.bs);
     else rqs_block_search_lean<KT>(pa, v, kn, b.idx, b.ks, b.bs);
     umma::wait_ld();
     const float amax_o = theta_block_finish_lean<KT>(co_, bias, pb, wb);
     theta_block_issue<KT>(dbase, cross_off, 2 * KT, pa, wa);       // raw slopes reuse the searched block's registers
     umma::wait_ld();
     release();                                          // every TMEM read of this row is done
-    if (__any_sync(0xffffffffu, !(amax_o < kThetaFastBound))) rqs_block_other<KT>(pb, b.idx, kn, b.ko, b.bo, chk);
+    if (__any_sync(0xffffffffu, !(amax_o < kThetaFastBound))) rqs_block_other<KT>(pb, b.idx, kn, b.ko, b.bo);
     else rqs_block_other_lean<KT>(pb, b.idx, kn, scr, stride, b.ko, b.bo);
     rqs_block_slopes_lean<KT>(pa, wa, umma::kF16LoUnscale, bias + 2 * KT, b.idx, scr, stride, b.dk, b.dkp1);
-}
-
-// One spline row shared by two threads (the same event in column groups 0 and 1), for couplings that transform a
-// single dim and would otherwise leave group 1 idle: group 0 normalises the searched axis and finds the bin while
-// group 1 normalises the other axis; the bin goes over through shared memory, group 1 selects the other-axis knot
-// and the slopes and hands them back; then group 0 evaluates y (or x) while group 1 evaluates log|dy/dx|.
-// Operation for operation the same arithmetic as the IEEE and exact-fast block forms (rqs_block_search<KT, SAFE> +
-// rqs_block_other_pre / _post<KT, SAFE>) + rqs_eval_*.
-__device__ __forceinline__ void pair_barrier(int id) { asm volatile("bar.sync %0, 256;" ::"r"(id) : "memory"); }
-
-template <int KT, bool INVERSE>
-__device__ __forceinline__ void spline_row_search_half(uint32_t dbase, uint32_t cross_off, const float* __restrict__ bias,
-                                                       float v, RqsBin& b) {
-    constexpr int cs_ = INVERSE ? KT : 0;
-    const KnotNorm kn = make_knot_norm(KT);
-    float pa[KT], wa[KT];
-    RqsCheck chk;
-    theta_block_issue<KT>(dbase, cross_off, cs_, pa, wa);
-    umma::wait_ld();
-    const float amax_s = theta_block_finish<KT>(cs_, bias, pa, wa);
-    if (__any_sync(0xffffffffu, !(amax_s < kThetaFastBound)))
-        rqs_block_search<KT, true>(pa, v, kn, b.idx, b.ks, b.bs, chk);
-    else
-        rqs_block_search<KT, false>(pa, v, kn, b.idx, b.ks, b.bs, chk);
-}
-
-// group 1: loads of the other-axis and slope blocks, squareplus + sum of the other axis while group 0 searches; then
-// (pair barrier 3) the bin index arrives through ex[0..2], and the other-axis knot and the slopes are selected
-template <int KT, bool INVERSE>
-__device__ __forceinline__ void spline_row_other_half(uint32_t dbase, uint32_t cross_off, const float* __restrict__ bias,
-                                                      const float* ex, int m, RqsBin& b) {
-    constexpr int co_ = INVERSE ? 0 : KT;
-    const KnotNorm kn = make_knot_norm(KT);
-    float pb[KT], ps[KT], wb[KT], ws[KT];
-    RqsCheck chk;
-    theta_block_issue<KT>(dbase, cross_off, co_, pb, wb);
-    theta_block_issue<KT>(dbase, cross_off, 2 * KT, ps, ws);
-    umma::wait_ld();                                    // every TMEM read of this thread is done
-    const float amax_o = theta_block_finish<KT>(co_, bias, pb, wb);
-    (void)theta_block_finish<KT>(2 * KT, bias, ps, ws);
-    float sum;
-    const bool safe = __any_sync(0xffffffffu, !(amax_o < kThetaFastBound));
-    if (safe) rqs_block_other_pre<KT, true>(pb, sum, chk);
-    else rqs_block_other_pre<KT, false>(pb, sum, chk);
-    pair_barrier(3);
-    b.idx = __float_as_int(ex[0 * UM + m]); b.ks = ex[1 * UM + m]; b.bs = ex[2 * UM + m];
-    if (safe) rqs_block_other_post<KT, true>(pb, sum, b.idx, kn, b.ko, b.bo);
-    else rqs_block_other_post<KT, false>(pb, sum, b.idx, kn, b.ko, b.bo);
-    rqs_block_slopes<KT>(ps, b.idx, b.dk, b.dkp1);
 }
 
 // Activation phase of the VJP kernel: swish for the next GEMM (fp16 x 3 split into tensor memory, as in the eval
@@ -841,10 +791,11 @@ __device__ __forceinline__ float vjp_row_tmem(uint32_t dbase, const float* __res
 // ---- the epilogue / SIMT role of the tensor-core chain kernel ------------------------------------------------
 // NG column groups of 4 warps each (group g = warp / 4 owns CW = 32 / NG columns of every 32-column K-chunk and
 // every NG-th feature / bounded column); TMEM lane quarter = warp % 4 (hardware rule).  Spline rows are run by
-// groups 0 and 1 (one transformed dim each, alternating accumulator buffers).
+// groups 0 and 1 (one transformed dim each, alternating accumulator buffers; one thread per row, so a single-dim
+// coupling's row runs on group 0 alone).
 struct UCtx {
     const ChainArgs& a;
-    float *xs, *cs, *xraw, *hs, *cst, *ldx, *pairx;
+    float *xs, *cs, *xraw, *hs, *cst, *ldx;
     float4* scratch;   // per-thread scratch columns of the lean spline row: [2][8][UM] float4 (32 KB)
     uint64_t* bars;
     const StepDesc* steps;
@@ -874,6 +825,173 @@ __device__ __forceinline__ void activation_store(uint32_t tb, uint32_t lane_base
     static_assert(CW == 16, "one tcgen05.st.x8 per part");
     umma::st8u(umma::taddr(tb, lane_base, n0 >> 1), hi);
     umma::st8u(umma::taddr(tb, lane_base, TC_ALO + (n0 >> 1)), lo);
+}
+
+// Act: the activation of one chunk, act(layer, n0, z, hi, lo) - swish + split (activation_compute) in the eval passes,
+// vjp_activation in the VJP kernel.
+// FFMA first Dense (K = F), output straight into tensor memory: K-chunk c of the next GEMM = columns [32c, 32c+32), of
+// which column group `half` owns CW.  The event's first four inputs stay in registers for all chunks, the rest are read
+// from hs ([F][UM], x - mean) in a loop.  before_store() runs once, ahead of the first tcgen05.st.
+template <int CW, class Act, class BeforeStore>
+__device__ __forceinline__ void first_dense_ffma(const float* hs, int F, int m, int half, const float* w0s, const float* b0s,
+                                                 uint32_t tb, uint32_t lane_base, uint64_t* aready, Act act,
+                                                 BeforeStore before_store) {
+    float hreg[4];
+#pragma unroll
+    for (int f = 0; f < 4; ++f) hreg[f] = f < F ? hs[f * UM + m] : 0.f;
+#pragma unroll 1
+    for (int c = 0; c < 4; ++c) {
+        const int n0 = c * 32 + half * CW;
+        float acc[CW];
+        uint32_t ahi[CW / 2], alo[CW / 2];
+        {
+            const float4* bv = reinterpret_cast<const float4*>(b0s + n0);
+#pragma unroll
+            for (int g4 = 0; g4 < CW / 4; ++g4) {
+                const float4 t = bv[g4];
+                acc[g4 * 4 + 0] = t.x; acc[g4 * 4 + 1] = t.y; acc[g4 * 4 + 2] = t.z; acc[g4 * 4 + 3] = t.w;
+            }
+        }
+        auto fma_row = [&](float h, int f) {
+            const float4* w = reinterpret_cast<const float4*>(w0s + f * 128 + n0);
+#pragma unroll
+            for (int g4 = 0; g4 < CW / 4; ++g4) {
+                const float4 wv = w[g4];
+                acc[g4 * 4 + 0] = fmaf(h, wv.x, acc[g4 * 4 + 0]);
+                acc[g4 * 4 + 1] = fmaf(h, wv.y, acc[g4 * 4 + 1]);
+                acc[g4 * 4 + 2] = fmaf(h, wv.z, acc[g4 * 4 + 2]);
+                acc[g4 * 4 + 3] = fmaf(h, wv.w, acc[g4 * 4 + 3]);
+            }
+        };
+#pragma unroll
+        for (int f = 0; f < 4; ++f)
+            if (f < F) fma_row(hreg[f], f);
+        for (int f = 4; f < F; ++f) fma_row(hs[f * UM + m], f);
+        act(0, n0, acc, ahi, alo);
+        if (c == 0) before_store();
+        activation_store<CW>(tb, lane_base, n0, ahi, alo);
+        umma::wait_st();
+        umma::fence_before_sync();
+        umma::mbar_arrive(&aready[c]);
+    }
+}
+
+// Hidden-layer drain: accumulator -> main + cross * 2^-11 + bias -> act -> the next activations, chunk c = accumulator
+// columns [32c + CW half, +CW) -> the same columns of the A operand, then aready[c].  The TMEM loads of chunk c+1 are in
+// flight during the arithmetic of chunk c.  FD: the one merged accumulator of the tensor-core first Dense (bias b0').
+template <int CW, bool FD, class Act>
+__device__ __forceinline__ void hidden_drain(uint32_t cmain, uint32_t ccross, const float* bh, int layer, int half,
+                                             uint32_t tb, uint32_t lane_base, uint64_t* aready, Act act) {
+    float vn[CW], wn[FD ? 1 : CW];
+    tmem_load<CW>(umma::taddr(tb, lane_base, cmain + half * CW), vn);                     // main products
+    if constexpr (!FD) tmem_load<CW>(umma::taddr(tb, lane_base, ccross + half * CW), wn);  // cross products (scale 2^11)
+#pragma unroll 1
+    for (int c = 0; c < 4; ++c) {
+        const int n0 = c * 32 + half * CW;
+        float v[CW];
+        uint32_t ahi[CW / 2], alo[CW / 2];
+        umma::wait_ld();
+        {
+            const float4* bv = reinterpret_cast<const float4*>(bh + n0);
+#pragma unroll
+            for (int g4 = 0; g4 < CW / 4; ++g4) {
+                const float4 t = bv[g4];
+                if constexpr (FD) {
+                    v[g4 * 4 + 0] = vn[g4 * 4 + 0] + t.x;
+                    v[g4 * 4 + 1] = vn[g4 * 4 + 1] + t.y;
+                    v[g4 * 4 + 2] = vn[g4 * 4 + 2] + t.z;
+                    v[g4 * 4 + 3] = vn[g4 * 4 + 3] + t.w;
+                } else {
+                    v[g4 * 4 + 0] = fmaf(wn[g4 * 4 + 0], umma::kF16LoUnscale, vn[g4 * 4 + 0]) + t.x;
+                    v[g4 * 4 + 1] = fmaf(wn[g4 * 4 + 1], umma::kF16LoUnscale, vn[g4 * 4 + 1]) + t.y;
+                    v[g4 * 4 + 2] = fmaf(wn[g4 * 4 + 2], umma::kF16LoUnscale, vn[g4 * 4 + 2]) + t.z;
+                    v[g4 * 4 + 3] = fmaf(wn[g4 * 4 + 3], umma::kF16LoUnscale, vn[g4 * 4 + 3]) + t.w;
+                }
+            }
+        }
+        if (c < 3) {
+            tmem_load<CW>(umma::taddr(tb, lane_base, cmain + n0 + 32), vn);
+            if constexpr (!FD) tmem_load<CW>(umma::taddr(tb, lane_base, ccross + n0 + 32), wn);
+        }
+        act(layer, n0, v, ahi, alo);
+        activation_store<CW>(tb, lane_base, n0, ahi, alo);
+        umma::wait_st();
+        umma::fence_before_sync();
+        umma::mbar_arrive(&aready[c]);
+    }
+}
+
+// Producer: one unit's weight image (N columns x 4 K-chunks of 32, fp16 hi | lo each) into the 4-stage ring
+__device__ __forceinline__ void stream_unit(uint64_t* full, uint64_t* empty, float* ring, const float* base, int N,
+                                            uint32_t& stage, uint32_t& phase) {
+    const uint32_t bytes = (uint32_t)N * 128u;   // one K-chunk (32): fp16 hi | lo images
+    for (int c = 0; c < 4; ++c) {
+        mbar_wait(&empty[stage], phase ^ 1u);
+        mbar_arrive_expect_tx(&full[stage], bytes);
+        bulk_copy_g2s(ring + (size_t)stage * URING_FLOATS, base + (size_t)c * N * 32, bytes, &full[stage]);
+        if (++stage == URING) { stage = 0; phase ^= 1u; }
+    }
+}
+
+// MMA issuer: the MMAs of one unit (N = 128 for a hidden layer, NL for one transformed dim of the last layer) into the
+// main (dmain) and cross (dcross) accumulators, then `done` is committed.  newver: the unit reads a new version of the
+// activations, whose K-chunk c is waited for (aready[c], phase p_ar) before chunk c's MMAs, and chunks [0, nfree) before
+// the first (the chunks whose accumulator columns this unit overwrites).  Advances the ring phase, and p_ar if newver.
+// One unit = 4 K-chunks = one lap of the 4-stage ring, so chunk c always sits in stage c and every descriptor is (a
+// hoisted ring address) + (a compile-time offset): the issuing thread's per-MMA work is what bounds the small-N units,
+// keep it to a couple of instructions.
+// wait (trace build only, may be null): cycles spent waiting for the activations ([0]) and the weights ([1]) are added.
+template <int N>
+__device__ __forceinline__ void issue_unit(uint64_t* full, uint64_t* empty, uint64_t* aready, uint64_t* done, const float* ring,
+                                           uint32_t tb, uint32_t dmain, uint32_t dcross, bool newver, int nfree,
+                                           uint32_t& phase, uint32_t& p_ar, long long* wait = nullptr) {
+    static_assert(URING == 4, "the MMA issuer maps chunk c to ring stage c");
+    constexpr uint32_t lbo = (uint32_t)(N >> 3) * 128u;
+    constexpr uint32_t idesc = umma::instr_desc_f16(N);
+    constexpr uint32_t desc_hi = (128u >> 4) | (1u << 14);   // SBO, descriptor version
+    const uint32_t ring16 = (smem_u32(ring) >> 4) | ((lbo >> 4) << 16);
+    int waited = 0;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+#ifdef ZF_TRACE
+        const long long t_a = wait ? clock64() : 0;
+#endif
+        if (newver) {
+            const int need = max(c + 1, nfree);
+#pragma unroll
+            for (int w = 0; w < 4; ++w)
+                if (w >= waited && w < need) mbar_wait(&aready[w], p_ar);
+            waited = max(waited, need);
+        }
+#ifdef ZF_TRACE
+        const long long t_f = wait ? clock64() : 0;
+        if (wait) wait[0] += t_f - t_a;
+#endif
+        mbar_wait(&full[c], phase);
+#ifdef ZF_TRACE
+        if (wait) wait[1] += clock64() - t_f;
+#endif
+        umma::fence_after_sync();
+        if (umma::elect_one()) {
+#pragma unroll
+            for (int ks = 0; ks < 2; ++ks) {   // K = 16 per kind::f16 instruction
+                const uint32_t off_hi = (uint32_t)(c * URING_FLOATS * 4 + ks * 2 * (int)lbo) >> 4;
+                const uint32_t off_lo = off_hi + ((uint32_t)N * 64u >> 4);   // lo image follows the hi image
+                const uint64_t dhi = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_hi);
+                const uint64_t dlo = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_lo);
+                const uint32_t acol = (uint32_t)(c * 16 + ks * 8);   // fp16 pairs: 8 columns per k-step
+                const bool first = (c | ks) == 0;
+                umma::mma_f16_ts(dcross, tb + TC_ALO + acol, dhi, idesc, !first);   // A_lo' * B_hi
+                umma::mma_f16_ts(dcross, tb + acol, dlo, idesc, true);              // A_hi * B_lo'
+                umma::mma_f16_ts(dmain, tb + acol, dhi, idesc, !first);             // A_hi * B_hi
+            }
+            umma::commit(&empty[c]);
+            if (c == 3) umma::commit(done);
+        }
+        __syncwarp();
+    }
+    phase ^= 1u;
+    if (newver) p_ar ^= 1u;
 }
 
 template <bool INVERSE, bool VJP = false>
@@ -1055,49 +1173,9 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                 }
             };
             if (VJP && !tcfd) vjp_side_outputs();
-            // ---- first Dense (K = F) on the FFMA pipe, output straight into tensor memory: couplings with more than 16
-            // conditioner inputs, and flows of single-dim couplings run through this kernel (F is 2 or 3 there).
-            // K-chunk c of the next GEMM = columns [32c, 32c+32): this half owns 16 of them.  The event's first four inputs
-            // stay in registers for all chunks, the rest are read from hs in a loop.
-            auto first_dense = [&]() {
-                float hreg[4];
-#pragma unroll
-                for (int f = 0; f < 4; ++f) hreg[f] = f < F ? hs[f * UM + m] : 0.f;
-#pragma unroll 1
-                for (int c = 0; c < 4; ++c) {
-                    const int n0 = c * 32 + half * CW;
-                    float acc[CW];
-                    uint32_t ahi[CW / 2], alo[CW / 2];
-                    {
-                        const float4* bv = reinterpret_cast<const float4*>(b0s + n0);
-#pragma unroll
-                        for (int g4 = 0; g4 < CW / 4; ++g4) {
-                            const float4 t = bv[g4];
-                            acc[g4 * 4 + 0] = t.x; acc[g4 * 4 + 1] = t.y; acc[g4 * 4 + 2] = t.z; acc[g4 * 4 + 3] = t.w;
-                        }
-                    }
-                    auto fma_row = [&](float h, int f) {
-                        const float4* w = reinterpret_cast<const float4*>(w0s + f * 128 + n0);
-#pragma unroll
-                        for (int g4 = 0; g4 < CW / 4; ++g4) {
-                            const float4 wv = w[g4];
-                            acc[g4 * 4 + 0] = fmaf(h, wv.x, acc[g4 * 4 + 0]);
-                            acc[g4 * 4 + 1] = fmaf(h, wv.y, acc[g4 * 4 + 1]);
-                            acc[g4 * 4 + 2] = fmaf(h, wv.z, acc[g4 * 4 + 2]);
-                            acc[g4 * 4 + 3] = fmaf(h, wv.w, acc[g4 * 4 + 3]);
-                        }
-                    };
-#pragma unroll
-                    for (int f = 0; f < 4; ++f)
-                        if (f < F) fma_row(hreg[f], f);
-                    for (int f = 4; f < F; ++f) fma_row(hs[f * UM + m], f);
-                    if (VJP) vjp_activation<CW>(a, 0, tile, m0, m, nm, n0, acc, ahi, alo);
-                    else activation_compute<CW>(acc, ahi, alo);
-                    activation_store<CW>(tb, lane_base, n0, ahi, alo);
-                    umma::wait_st();
-                    umma::fence_before_sync();
-                    umma::mbar_arrive(&bars[B_AREADY + c]);
-                }
+            auto act = [&](int l, int n0, const float (&z)[CW], uint32_t (&hi)[CW / 2], uint32_t (&lo)[CW / 2]) {
+                if (VJP) vjp_activation<CW>(a, l, tile, m0, m, nm, n0, z, hi, lo);
+                else activation_compute<CW>(z, hi, lo);
             };
             if (tcfd) {
                 // ---- first Dense on the tensor cores: (x - mean) * mul of the event's inputs (3xFP16 split) as a K = 16 A operand
@@ -1127,60 +1205,20 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                 umma::mbar_arrive(&bars[B_A0READY]);
                 if (VJP) vjp_side_outputs();   // under the first Dense's MMAs
             } else {
-                first_dense();
+                // first Dense on the FFMA pipe: couplings with more than 16 conditioner inputs, and flows of single-dim
+                // couplings run through this kernel (F is 2 or 3 there)
+                first_dense_ffma<CW>(hs, F, m, half, w0s, b0s, tb, lane_base, &bars[B_AREADY], act, [] {});
             }
             ZF_TR(trs);   // first dense done
-            // ---- hidden layers 1..L-1: accumulator -> bias + swish -> next activations
-            // FD: the accumulator of the tensor-core first Dense (one merged accumulator, bias b0'); otherwise a hidden
-            // layer's main + cross accumulators
+            // ---- hidden layers 1..L-1 (and the tensor-core first Dense's accumulator): drain -> next activations
             auto hidden_epilogue = [&](auto fdtag, int l) {
                 constexpr bool FD = decltype(fdtag)::value;
                 mbar_wait(&bars[B_DFULL_H], p_fh);
                 p_fh ^= 1u;
                 umma::fence_after_sync();
                 ZF_TR(trs);   // hidden accumulator ready
-                const float* bh = FD ? b0s : bhs + (l - 1) * 128;
-                constexpr uint32_t cmain = FD ? TC_FD : TC_HMAIN;
-                // chunk c: accumulator columns [32c + CW g, +CW) -> the same columns of the next activations.
-                // The TMEM loads of chunk c+1 are in flight during the arithmetic of chunk c.
-                float vn[CW], wn[FD ? 1 : CW];
-                tmem_load<CW>(umma::taddr(tb, lane_base, cmain + half * CW), vn);     // main products
-                if constexpr (!FD) tmem_load<CW>(umma::taddr(tb, lane_base, TC_HCROSS + half * CW), wn);    // cross products (scale 2^11)
-#pragma unroll 1
-                for (int c = 0; c < 4; ++c) {
-                    const int n0 = c * 32 + half * CW;
-                    float v[CW];
-                    uint32_t ahi[CW / 2], alo[CW / 2];
-                    umma::wait_ld();
-                    {
-                        const float4* bv = reinterpret_cast<const float4*>(bh + n0);
-#pragma unroll
-                        for (int g4 = 0; g4 < CW / 4; ++g4) {
-                            const float4 t = bv[g4];
-                            if constexpr (FD) {
-                                v[g4 * 4 + 0] = vn[g4 * 4 + 0] + t.x;
-                                v[g4 * 4 + 1] = vn[g4 * 4 + 1] + t.y;
-                                v[g4 * 4 + 2] = vn[g4 * 4 + 2] + t.z;
-                                v[g4 * 4 + 3] = vn[g4 * 4 + 3] + t.w;
-                            } else {
-                                v[g4 * 4 + 0] = fmaf(wn[g4 * 4 + 0], umma::kF16LoUnscale, vn[g4 * 4 + 0]) + t.x;
-                                v[g4 * 4 + 1] = fmaf(wn[g4 * 4 + 1], umma::kF16LoUnscale, vn[g4 * 4 + 1]) + t.y;
-                                v[g4 * 4 + 2] = fmaf(wn[g4 * 4 + 2], umma::kF16LoUnscale, vn[g4 * 4 + 2]) + t.z;
-                                v[g4 * 4 + 3] = fmaf(wn[g4 * 4 + 3], umma::kF16LoUnscale, vn[g4 * 4 + 3]) + t.w;
-                            }
-                        }
-                    }
-                    if (c < 3) {
-                        tmem_load<CW>(umma::taddr(tb, lane_base, cmain + n0 + 32), vn);
-                        if constexpr (!FD) tmem_load<CW>(umma::taddr(tb, lane_base, TC_HCROSS + n0 + 32), wn);
-                    }
-                    if (VJP) vjp_activation<CW>(a, l, tile, m0, m, nm, n0, v, ahi, alo);
-                    else activation_compute<CW>(v, ahi, alo);
-                    activation_store<CW>(tb, lane_base, n0, ahi, alo);
-                    umma::wait_st();
-                    umma::fence_before_sync();
-                    umma::mbar_arrive(&bars[B_AREADY + c]);
-                }
+                hidden_drain<CW, FD>(FD ? TC_FD : TC_HMAIN, TC_HCROSS, FD ? b0s : bhs + (l - 1) * 128, l, half, tb, lane_base,
+                                     &bars[B_AREADY], act);
                 ZF_TR(trs);   // hidden epilogue done
             };
             if (tcfd) hidden_epilogue(std::true_type{}, 0);
@@ -1229,37 +1267,6 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                             *reinterpret_cast<uint4*>(dt + (size_t)TW * 256 + (size_t)u * 2048) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
                         }
                     }
-                }
-            } else if (d == 1 && half < 2) {
-                // one transformed dim: the two spline groups share its row (see spline_row_search_half)
-                mbar_wait(&bars[B_DFULL_D + 0], p_fd);
-                p_fd ^= 1u;
-                umma::fence_after_sync();
-                ZF_TR(trs);   // theta ready
-                const uint32_t dbase = umma::taddr(tb, lane_base, tc_dmain(0));
-                const uint32_t cross = TC_XOFF;
-                float* px = xs + pmod(0 - rot, D) * UM + m;
-                const float v = *px;
-                float* ex = cx.pairx;   // [7][UM]: idx, ks, bs | ko, bo, dk, dkp1
-                RqsBin bin;
-                if (half == 0) {
-                    if (K == 16) spline_row_search_half<16, INVERSE>(dbase, cross, bls, v, bin);
-                    else spline_row_search_half<32, INVERSE>(dbase, cross, bls, v, bin);
-                    ex[0 * UM + m] = __int_as_float(bin.idx); ex[1 * UM + m] = bin.ks; ex[2 * UM + m] = bin.bs;
-                    if (m < nm) put_idx(a, s, m0 + m, 0, bin.idx);
-                    pair_barrier(3);                         // bin published; both threads' TMEM reads are done
-                    umma::fence_before_sync();
-                    umma::mbar_arrive(&bars[B_DEMPTY_D + 0]);
-                    ZF_TR(trs);   // released
-                    pair_barrier(4);                         // other-axis knot and slopes published
-                    bin.ko = ex[3 * UM + m]; bin.bo = ex[4 * UM + m]; bin.dk = ex[5 * UM + m]; bin.dkp1 = ex[6 * UM + m];
-                    *px = INVERSE ? rqs_eval_inverse(v, bin) : rqs_eval_forward_y(v, bin);
-                } else {
-                    if (K == 16) spline_row_other_half<16, INVERSE>(dbase, cross, bls, ex, m, bin);
-                    else spline_row_other_half<32, INVERSE>(dbase, cross, bls, ex, m, bin);
-                    ex[3 * UM + m] = bin.ko; ex[4 * UM + m] = bin.bo; ex[5 * UM + m] = bin.dk; ex[6 * UM + m] = bin.dkp1;
-                    pair_barrier(4);
-                    if (!INVERSE) ldc += rqs_eval_forward_ld(v, bin);
                 }
             } else {
                 for (int jj = half; jj < d && half < 2; jj += 2) {
@@ -1362,8 +1369,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
     // the VJP kernel runs ONE coupling: its constants are fetched once and both buffer indices name the same block
     const int cst_stride = VJP ? 0 : cl.total;
     float* ldx = cst + (VJP ? 1 : 2) * cl.total;
-    float* pairx = ldx + 3 * UM;              // [7][UM] exchange between the two threads of a shared spline row
-    float* scratch = pairx + 8 * UM;          // [2][8][UM] float4: scratch columns of the lean spline rows
+    float* scratch = ldx + 3 * UM;            // [2][8][UM] float4: scratch columns of the lean spline rows
     float* ring = scratch + (VJP ? 2 * UM * VJP_ROW : 2 * 8 * UM * 4);   // VJP: [2][UM][VJP_ROW] theta rows instead
     uint64_t* bars = reinterpret_cast<uint64_t*>(ring + (size_t)URING * URING_FLOATS);
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + B_COUNT);
@@ -1454,14 +1460,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
                         const bool hid = u < L - 1;
                         const int N = hid ? 128 : NL;
                         const float* base = hid ? wsf + s.off_U[u + 1] : wsf + s.off_U[L] + (size_t)(u - (L - 1)) * NL * 128;
-                        const uint32_t bytes = (uint32_t)N * 128u;   // one K-chunk (32): fp16 hi | lo images
-                        for (int c = 0; c < 4; ++c) {
-                            mbar_wait(&bars[B_EMPTY + stage], phase ^ 1u);
-                            mbar_arrive_expect_tx(&bars[B_FULL + stage], bytes);
-                            bulk_copy_g2s(ring + (size_t)stage * URING_FLOATS, base + (size_t)c * N * 32, bytes,
-                                          &bars[B_FULL + stage]);
-                            if (++stage == URING) { stage = 0; phase ^= 1u; }
-                        }
+                        stream_unit(&bars[B_FULL], &bars[B_EMPTY], ring, base, N, stage, phase);
                         if (u == 0) {
                             // behind this coupling's first unit: the next coupling's constants (their buffer is
                             // released when the previous coupling ends) and, once per tile, the next tile's rows
@@ -1529,9 +1528,9 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
                     // them, the first last-layer unit (theta buffer 0) only the hidden main columns of chunks 0 and 1
                     // (a tensor-core first Dense accumulates in [TC_FD, +128): only a theta unit right behind it overlaps)
                     const int nfree = (u == 0) ? ((tcfd && !hid) ? 4 : 0) : (hid ? 4 : 2);
-                    int waited = 0;
+                    long long w_ab[2] = {0, 0};   // trace build: cycles waited for the activations / the weights
 #ifdef ZF_TRACE
-                    long long w_pend = clock64(), w_full = 0, w_a = 0;
+                    long long w_pend = clock64();
 #endif
                     if ((hid || b == 0) && dim_pending0) { mbar_wait(&bars[B_DEMPTY_D + 0], p_ed0); p_ed0 ^= 1u; dim_pending0 = false; }
                     if ((hid || b == 1) && dim_pending1) { mbar_wait(&bars[B_DEMPTY_D + 1], p_ed1); p_ed1 ^= 1u; dim_pending1 = false; }
@@ -1541,70 +1540,23 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
 #endif
                     const uint32_t dmain = hid ? tb + TC_HMAIN : tb + tc_dmain(b);
                     const uint32_t dcross = hid ? tb + TC_HCROSS : dmain + TC_XOFF;
-                    // One unit = 4 K-chunks = one lap of the 4-stage ring, so chunk c always sits in stage c and every
-                    // descriptor is (a hoisted ring address) + (a compile-time offset): the issuing thread's
-                    // per-MMA work is what bounds the small-N units, keep it to a couple of instructions.
-                    static_assert(URING == 4, "the MMA issuer maps chunk c to ring stage c");
-                    auto issue_unit = [&](auto ntag) {
-                        constexpr int N = decltype(ntag)::value;
-                        constexpr uint32_t lbo = (uint32_t)(N >> 3) * 128u;
-                        constexpr uint32_t idesc = umma::instr_desc_f16(N);
-                        constexpr uint32_t desc_hi = (128u >> 4) | (1u << 14);   // SBO, descriptor version
-                        const uint32_t ring16 = (smem_u32(ring) >> 4) | ((lbo >> 4) << 16);
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) {
-#ifdef ZF_TRACE
-                            long long t_a = clock64();
-#endif
-                            if (newver) {
-                                const int need = max(c + 1, nfree);
-#pragma unroll
-                                for (int w = 0; w < 4; ++w)
-                                    if (w >= waited && w < need) mbar_wait(&bars[B_AREADY + w], p_ar);
-                                waited = max(waited, need);
-                            }
-#ifdef ZF_TRACE
-                            long long t_f = clock64();
-                            w_a += t_f - t_a;
-#endif
-                            mbar_wait(&bars[B_FULL + c], phase);
-#ifdef ZF_TRACE
-                            w_full += clock64() - t_f;
-#endif
-                            umma::fence_after_sync();
-                            if (umma::elect_one()) {
-#pragma unroll
-                                for (int ks = 0; ks < 2; ++ks) {   // K = 16 per kind::f16 instruction
-                                    const uint32_t off_hi = (uint32_t)(c * URING_FLOATS * 4 + ks * 2 * (int)lbo) >> 4;
-                                    const uint32_t off_lo = off_hi + ((uint32_t)N * 64u >> 4);   // lo image follows the hi image
-                                    const uint64_t dhi = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_hi);
-                                    const uint64_t dlo = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_lo);
-                                    const uint32_t acol = (uint32_t)(c * 16 + ks * 8);   // fp16 pairs: 8 columns per k-step
-                                    const bool first = (c | ks) == 0;
-                                    umma::mma_f16_ts(dcross, tb + TC_ALO + acol, dhi, idesc, !first);   // A_lo' * B_hi
-                                    umma::mma_f16_ts(dcross, tb + acol, dlo, idesc, true);              // A_hi * B_lo'
-                                    umma::mma_f16_ts(dmain, tb + acol, dhi, idesc, !first);             // A_hi * B_hi
-                                }
-                                umma::commit(&bars[B_EMPTY + c]);
-                                if (c == 3) umma::commit(&bars[hid ? B_DFULL_H : (B_DFULL_D + b)]);
-                            }
-                            __syncwarp();
-                        }
+                    uint64_t* done = &bars[hid ? B_DFULL_H : (B_DFULL_D + b)];
+                    auto unit = [&](auto n) {
+                        issue_unit<decltype(n)::value>(&bars[B_FULL], &bars[B_EMPTY], &bars[B_AREADY], done, ring, tb, dmain,
+                                                       dcross, newver, nfree, phase, p_ar, w_ab);
                     };
-                    if (hid) issue_unit(std::integral_constant<int, 128>{});
-                    else if (NL == 48) issue_unit(std::integral_constant<int, 48>{});
-                    else issue_unit(std::integral_constant<int, 96>{});
-                    phase ^= 1u;
+                    if (hid) unit(std::integral_constant<int, 128>{});
+                    else if (NL == 48) unit(std::integral_constant<int, 48>{});
+                    else unit(std::integral_constant<int, 96>{});
                     ZF_TR(2);
-                    ZF_TRV(2, -w_pend); ZF_TRV(2, -w_a); ZF_TRV(2, -w_full);
-                    if (newver) p_ar ^= 1u;
+                    ZF_TRV(2, -w_pend); ZF_TRV(2, -w_ab[0]); ZF_TRV(2, -w_ab[1]);
                     if (!hid) { if (b) dim_pending1 = true; else dim_pending0 = true; }
                 }
             }
         }
     };
     // ------------------------------------------------------------------ role dispatch
-    const UCtx cx{a, xs, cs, xraw, hs, cst, ldx, pairx, reinterpret_cast<float4*>(scratch), bars, steps, tb, n_tiles, cl, cst_stride, in16, in_bytes};
+    const UCtx cx{a, xs, cs, xraw, hs, cst, ldx, reinterpret_cast<float4*>(scratch), bars, steps, tb, n_tiles, cl, cst_stride, in16, in_bytes};
     if (warp == PW) producer_role();
     else if (warp == MW) mma_role();
     else umma_epilogue_role<INVERSE, VJP>(cx);
@@ -1758,13 +1710,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         const bool hid = u < L - 1;
                         const int N = hid ? 128 : NL;
                         const float* base = hid ? wsf + s.off_U[u + 1] : wsf + s.off_U[L];
-                        const uint32_t bytes = (uint32_t)N * 128u;
-                        for (int c = 0; c < 4; ++c) {
-                            mbar_wait(&bars[PP_EMPTY + stage], phase ^ 1u);
-                            mbar_arrive_expect_tx(&bars[PP_FULL + stage], bytes);
-                            bulk_copy_g2s(ring + (size_t)stage * URING_FLOATS, base + (size_t)c * N * 32, bytes, &bars[PP_FULL + stage]);
-                            if (++stage == URING) { stage = 0; phase ^= 1u; }
-                        }
+                        stream_unit(&bars[PP_FULL], &bars[PP_EMPTY], ring, base, N, stage, phase);
                         if (u == 0) {
                             issue_consts();                       // the next occurrence's constants
                             // once per tile: the rows of the tile that takes this slot in the next pair
@@ -1792,53 +1738,21 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         // a theta row at [384, 480) (K = 16) overlaps nothing but the next theta row
                         const bool clear = !hid && NL == 48;
                         const int nfree = (u == 0 || clear) ? 0 : 4;
-                        int waited = 0;
                         if (theta_pending && (!hid || pending_nl != 48)) {
                             mbar_wait(&bars[PP_DEMPTY_D], p_ed); p_ed ^= 1u; theta_pending = false;
                         }
                         umma::fence_after_sync();
                         const uint32_t dmain = hid ? tb + TC_PP_HMAIN : tb + tc_pp_theta(NL);
                         const uint32_t dcross = hid ? tb + TC_PP_HCROSS : dmain + tc_pp_xoff(NL);
-                        static_assert(URING == 4, "the MMA issuer maps chunk c to ring stage c");
-                        auto issue_unit = [&](auto ntag) {
-                            constexpr int N = decltype(ntag)::value;
-                            constexpr uint32_t lbo = (uint32_t)(N >> 3) * 128u;
-                            constexpr uint32_t idesc = umma::instr_desc_f16(N);
-                            constexpr uint32_t desc_hi = (128u >> 4) | (1u << 14);
-                            const uint32_t ring16 = (smem_u32(ring) >> 4) | ((lbo >> 4) << 16);
-#pragma unroll
-                            for (int c = 0; c < 4; ++c) {
-                                const int need = max(c + 1, nfree);
-#pragma unroll
-                                for (int w = 0; w < 4; ++w)
-                                    if (w >= waited && w < need) mbar_wait(&bars[PP_AREADY + w], p_ar);
-                                waited = max(waited, need);
-                                mbar_wait(&bars[PP_FULL + c], phase);
-                                umma::fence_after_sync();
-                                if (umma::elect_one()) {
-#pragma unroll
-                                    for (int ks = 0; ks < 2; ++ks) {
-                                        const uint32_t off_hi = (uint32_t)(c * URING_FLOATS * 4 + ks * 2 * (int)lbo) >> 4;
-                                        const uint32_t off_lo = off_hi + ((uint32_t)N * 64u >> 4);
-                                        const uint64_t dhi = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_hi);
-                                        const uint64_t dlo = ((uint64_t)desc_hi << 32) | (uint64_t)(ring16 + off_lo);
-                                        const uint32_t acol = (uint32_t)(c * 16 + ks * 8);
-                                        const bool first = (c | ks) == 0;
-                                        umma::mma_f16_ts(dcross, tb + TC_ALO + acol, dhi, idesc, !first);
-                                        umma::mma_f16_ts(dcross, tb + acol, dlo, idesc, true);
-                                        umma::mma_f16_ts(dmain, tb + acol, dhi, idesc, !first);
-                                    }
-                                    umma::commit(&bars[PP_EMPTY + c]);
-                                    if (c == 3) umma::commit(&bars[hid ? PP_DFULL_H : PP_DFULL_D]);
-                                }
-                                __syncwarp();
-                            }
+                        uint64_t* done = &bars[hid ? PP_DFULL_H : PP_DFULL_D];
+                        // every unit reads a new version of the activations (d == 1)
+                        auto unit = [&](auto n) {
+                            issue_unit<decltype(n)::value>(&bars[PP_FULL], &bars[PP_EMPTY], &bars[PP_AREADY], done, ring, tb, dmain,
+                                                           dcross, true, nfree, phase, p_ar);
                         };
-                        if (hid) issue_unit(std::integral_constant<int, 128>{});
-                        else if (NL == 48) issue_unit(std::integral_constant<int, 48>{});
-                        else issue_unit(std::integral_constant<int, 96>{});
-                        phase ^= 1u;
-                        p_ar ^= 1u;              // every unit reads a new version of the activations (d == 1)
+                        if (hid) unit(std::integral_constant<int, 128>{});
+                        else if (NL == 48) unit(std::integral_constant<int, 48>{});
+                        else unit(std::integral_constant<int, 96>{});
                         if (!hid) { theta_pending = true; pending_nl = NL; }
                     }
                 }
@@ -1851,6 +1765,9 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         const int q = warp & 3, half = warp >> 2, m = q * 32 + lane;
         const uint32_t lane_base = (uint32_t)(q * 32);
         constexpr int CW = 16;
+        auto act = [](int, int, const float (&z)[CW], uint32_t (&hi)[CW / 2], uint32_t (&lo)[CW / 2]) {
+            activation_compute<CW>(z, hi, lo);
+        };
         uint32_t p_fh = 0;
         long long n1 = 0;
         long long bn_done = -1;   // occurrence whose BatchNorm output is already in hs2[n & 1]
@@ -1890,50 +1807,15 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                     const float* hs = hs2 + (size_t)(n1 & 1) * a.u_fmax * UM;
                     if (bn_done != n1) batch_norm(n1, p, cj, slot);
                     s1_barrier();   // hs of this occurrence complete; every read of the other parity's hs is over
-                    float hreg[4];
-#pragma unroll
-                    for (int f = 0; f < 4; ++f) hreg[f] = f < F ? hs[f * UM + m] : 0.f;
-#pragma unroll 1
-                    for (int c = 0; c < 4; ++c) {
-                        const int n0 = c * 32 + half * CW;
-                        float acc[CW];
-                        uint32_t ahi[CW / 2], alo[CW / 2];
-                        {
-                            const float4* bv = reinterpret_cast<const float4*>(b0s + n0);
-#pragma unroll
-                            for (int g4 = 0; g4 < CW / 4; ++g4) {
-                                const float4 t = bv[g4];
-                                acc[g4 * 4 + 0] = t.x; acc[g4 * 4 + 1] = t.y; acc[g4 * 4 + 2] = t.z; acc[g4 * 4 + 3] = t.w;
-                            }
-                        }
-                        auto fma_row = [&](float h, int f) {
-                            const float4* w = reinterpret_cast<const float4*>(w0s + f * 128 + n0);
-#pragma unroll
-                            for (int g4 = 0; g4 < CW / 4; ++g4) {
-                                const float4 wv = w[g4];
-                                acc[g4 * 4 + 0] = fmaf(h, wv.x, acc[g4 * 4 + 0]);
-                                acc[g4 * 4 + 1] = fmaf(h, wv.y, acc[g4 * 4 + 1]);
-                                acc[g4 * 4 + 2] = fmaf(h, wv.z, acc[g4 * 4 + 2]);
-                                acc[g4 * 4 + 3] = fmaf(h, wv.w, acc[g4 * 4 + 3]);
-                            }
-                        };
-#pragma unroll
-                        for (int f = 0; f < 4; ++f)
-                            if (f < F) fma_row(hreg[f], f);
-                        for (int f = 4; f < F; ++f) fma_row(hs[f * UM + m], f);
-                        activation_compute<CW>(acc, ahi, alo);
-                        // the activations of the previous occurrence are still the A operand of its last-layer MMAs:
-                        // wait for their completion (the accumulator-full barrier the row warps also wait on) before
-                        // the first store; the first chunk's arithmetic has already run underneath that tail
-                        if (c == 0 && n1 > 0) {
+                    // the activations of the previous occurrence are still the A operand of its last-layer MMAs: wait
+                    // for their completion (the accumulator-full barrier the row warps also wait on) before the first
+                    // store; the first chunk's arithmetic has already run underneath that tail
+                    first_dense_ffma<CW>(hs, F, m, half, w0s, b0s, tb, lane_base, &bars[PP_AREADY], act, [&] {
+                        if (n1 > 0) {
                             mbar_wait(&bars[PP_DFULL_D], (uint32_t)((n1 - 1) & 1));
                             umma::fence_after_sync();
                         }
-                        activation_store<CW>(tb, lane_base, n0, ahi, alo);
-                        umma::wait_st();
-                        umma::fence_before_sync();
-                        umma::mbar_arrive(&bars[PP_AREADY + c]);
-                    }
+                    });
                     for (int l = 1; l < L; ++l) {
                         if (l == 1 && nslots == 2) {
                             // While the first hidden GEMM finishes: the BatchNorm of the next occurrence.  It belongs
@@ -1949,37 +1831,8 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         mbar_wait(&bars[PP_DFULL_H], p_fh);
                         p_fh ^= 1u;
                         umma::fence_after_sync();
-                        const float* bh = bhs + (l - 1) * 128;
-                        float vn[CW], wn[CW];
-                        tmem_load<CW>(umma::taddr(tb, lane_base, TC_PP_HMAIN + half * CW), vn);
-                        tmem_load<CW>(umma::taddr(tb, lane_base, TC_PP_HCROSS + half * CW), wn);
-#pragma unroll 1
-                        for (int c = 0; c < 4; ++c) {
-                            const int n0 = c * 32 + half * CW;
-                            float v[CW];
-                            uint32_t ahi[CW / 2], alo[CW / 2];
-                            umma::wait_ld();
-                            {
-                                const float4* bv = reinterpret_cast<const float4*>(bh + n0);
-#pragma unroll
-                                for (int g4 = 0; g4 < CW / 4; ++g4) {
-                                    const float4 t = bv[g4];
-                                    v[g4 * 4 + 0] = fmaf(wn[g4 * 4 + 0], umma::kF16LoUnscale, vn[g4 * 4 + 0]) + t.x;
-                                    v[g4 * 4 + 1] = fmaf(wn[g4 * 4 + 1], umma::kF16LoUnscale, vn[g4 * 4 + 1]) + t.y;
-                                    v[g4 * 4 + 2] = fmaf(wn[g4 * 4 + 2], umma::kF16LoUnscale, vn[g4 * 4 + 2]) + t.z;
-                                    v[g4 * 4 + 3] = fmaf(wn[g4 * 4 + 3], umma::kF16LoUnscale, vn[g4 * 4 + 3]) + t.w;
-                                }
-                            }
-                            if (c < 3) {
-                                tmem_load<CW>(umma::taddr(tb, lane_base, TC_PP_HMAIN + n0 + 32), vn);
-                                tmem_load<CW>(umma::taddr(tb, lane_base, TC_PP_HCROSS + n0 + 32), wn);
-                            }
-                            activation_compute<CW>(v, ahi, alo);
-                            activation_store<CW>(tb, lane_base, n0, ahi, alo);
-                            umma::wait_st();
-                            umma::fence_before_sync();
-                            umma::mbar_arrive(&bars[PP_AREADY + c]);
-                        }
+                        hidden_drain<CW, false>(TC_PP_HMAIN, TC_PP_HCROSS, bhs + (l - 1) * 128, l, half, tb, lane_base,
+                                                &bars[PP_AREADY], act);
                     }
                     umma::mbar_arrive(&bars[PP_CEMPTY + cb]);   // S1 is done with this occurrence's constants
                 }
