@@ -463,6 +463,111 @@ __device__ __forceinline__ void shift_bounds_row(const StepDesc& s, const float*
     ld_acc += ldc;
 }
 
+// step si in processing order: the inverse passes walk the program backwards
+template <bool INVERSE>
+__device__ __forceinline__ const StepDesc& step_at(const StepDesc* steps, int n_steps, int si) {
+    return steps[INVERSE ? (n_steps - 1 - si) : si];
+}
+
+// Rows -> feature-major tile of S events (xs[col][S], cs[col][S]), by a group of NT threads; thread t owns event t % S
+// and column group t / S.  xsrc / csrc: the tile's first row (in global memory or bulk-staged).  Padding events sit at
+// 0.5 / 0 and are never stored; when sampling, x is drawn from the latent instead of read.
+// X16 = false drops the 16-byte path of x at compile time, for callers whose D is never a multiple of 4.
+template <int NT, int S, bool X16 = true>
+__device__ __forceinline__ void load_tile(const ChainArgs& a, const float* xsrc, const float* csrc, long long m0, int nm,
+                                          int rot_in, float* xs, float* cs, int t) {
+    constexpr int NG = NT / S;
+    const int D = a.D, C = a.C, m = t % S, g = t / S;
+    const bool xs16 = X16 && (D & 3) == 0 && (a.sample || (reinterpret_cast<uintptr_t>(xsrc) & 15) == 0);
+    const bool cs16 = C > 0 && (C & 3) == 0 && (reinterpret_cast<uintptr_t>(csrc) & 15) == 0;
+    if (xs16) {
+        // this thread: every NG-th group of four columns of its own event, one 16-byte read per group and
+        // conflict-free writes into the feature-major tile
+        const float4* xr = reinterpret_cast<const float4*>(xsrc + (size_t)m * D);
+        for (int q = g; q < (D >> 2); q += NG) {
+            int col = pmod(4 * q - rot_in, D);
+            if (a.sample) {   // counter-based draws: the value of (event, column) does not depend on who computes it
+#pragma unroll 1
+                for (int i = 0; i < 4; ++i) {
+                    xs[col * S + m] = (m < nm) ? latent_draw(a.lc.kind, a.peakness, a.seed, m0 + m, 4 * q + i) : 0.5f;
+                    if (++col == D) col = 0;
+                }
+            } else {
+                const float4 v = (m < nm) ? xr[q] : make_float4(0.5f, 0.5f, 0.5f, 0.5f);
+                const float o[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    xs[col * S + m] = o[i];
+                    if (++col == D) col = 0;
+                }
+            }
+        }
+    } else {   // element e = mm * D + j, advanced by NT per round without dividing
+        int mm = t / D, j = t - mm * D;
+        const int dm = NT / D, dj = NT - dm * D;
+        for (int e = t; e < S * D; e += NT) {
+            int col = j - rot_in;
+            if (col < 0) col += D;
+            xs[col * S + mm] = (mm < nm) ? (a.sample ? latent_draw(a.lc.kind, a.peakness, a.seed, m0 + mm, j) : xsrc[e]) : 0.5f;
+            mm += dm; j += dj;
+            if (j >= D) { j -= D; ++mm; }
+        }
+    }
+    if (cs16) {
+        const float4* cr = reinterpret_cast<const float4*>(csrc + (size_t)m * C);
+        for (int q = g; q < (C >> 2); q += NG) {
+            const float4 v = (m < nm) ? cr[q] : make_float4(0.f, 0.f, 0.f, 0.f);
+            cs[(4 * q + 0) * S + m] = v.x; cs[(4 * q + 1) * S + m] = v.y;
+            cs[(4 * q + 2) * S + m] = v.z; cs[(4 * q + 3) * S + m] = v.w;
+        }
+    } else if (C) {
+        int mm = t / C, j = t - mm * C;
+        const int dm = NT / C, dj = NT - dm * C;
+        for (int e = t; e < S * C; e += NT) {
+            cs[j * S + mm] = (mm < nm) ? csrc[e] : 0.f;
+            mm += dm; j += dj;
+            if (j >= C) { j -= C; ++mm; }
+        }
+    }
+}
+
+// Feature-major tile of S events -> rows y[m0 .. m0 + nm), by a group of NT threads (thread t: event t % S, column
+// group t / S on the 16-byte path)
+template <int NT, int S>
+__device__ __forceinline__ void store_tile(float* y, long long m0, int nm, int D, int rot_out, const float* xs, int t) {
+    constexpr int NG = NT / S;
+    const int m = t % S, g = t / S;
+    if ((D & 3) == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0) {
+        // this thread: every NG-th group of four columns of its own event (conflict-free reads of the feature-major
+        // tile, one 16-byte store per group)
+        if (m < nm) {
+            float4* yr = reinterpret_cast<float4*>(y + (m0 + m) * D);
+            for (int q = g; q < (D >> 2); q += NG) {
+                int col = pmod(4 * q - rot_out, D);
+                float o[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    o[i] = xs[col * S + m];
+                    if (++col == D) col = 0;
+                }
+                yr[q] = make_float4(o[0], o[1], o[2], o[3]);
+            }
+        }
+    } else {
+        for (int e = t; e < nm * D; e += NT) {
+            const int mm = e / D, j = e - mm * D;
+            y[m0 * D + e] = xs[pmod(j - rot_out, D) * S + mm];
+        }
+    }
+}
+
+// log p of event m of a finished tile: sum of the latent log-pdf over its columns + the chain's log-det (flow.py:46-47)
+__device__ __forceinline__ float tile_lp(const ChainArgs& a, const float* xs, int S, int m, float ld) {
+    float lat = 0.f;
+    for (int j = 0; j < a.D; ++j) lat += latent_logpdf(xs[pmod(j - a.rot_total, a.D) * S + m], a.lc);
+    return nan_to_num_lp(lat + ld);
+}
+
 template <bool INVERSE>
 __device__ __forceinline__ void run_shift_bounds(const StepDesc& s, const float* __restrict__ wsf, int D,
                                                  float* xs, float& ld_acc, int tid) {
@@ -487,41 +592,21 @@ __global__ void __launch_bounds__(kChainThreads, 2) chain_kernel(const __grid_co
     for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const long long m0 = tile * TM;
         const int nm = (int)min((long long)TM, a.M - m0);
-        // ---- load the tile, feature-major; padding samples sit at 0.5 and are never stored
-        const int rot_in = INVERSE ? a.rot_total : 0;
-        for (int e = tid; e < TM * D; e += kChainThreads) {
-            const int m = e / D, j = e - m * D;
-            const float v = (m < nm) ? (a.sample ? latent_draw(a.lc.kind, a.peakness, a.seed, m0 + m, j) : a.x[m0 * D + e]) : 0.5f;
-            xs[pmod(j - rot_in, D) * TM + m] = v;
-        }
-        for (int e = tid; e < TM * C; e += kChainThreads) {
-            const int m = e / C, j = e - m * C;
-            cs[j * TM + m] = (m < nm) ? a.c[m0 * C + e] : 0.f;
-        }
+        load_tile<kChainThreads, TM>(a, a.x + m0 * D, a.c + m0 * C, m0, nm, INVERSE ? a.rot_total : 0, xs, cs, tid);
         __syncthreads();
 
         float ld_acc = 0.f;  // Chain: log_det = zeros(M)   (bijectors.py:107)
         for (int si = 0; si < a.n_steps; ++si) {
-            const StepDesc& s = steps[INVERSE ? (a.n_steps - 1 - si) : si];
+            const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
             if (s.kind == kStepKindShiftBounds) run_shift_bounds<INVERSE>(s, wsf, D, xs, ld_acc, tid);
             else run_coupling<INVERSE>(a, m0, nm, s, wsf, D, C, xs, cs, act0, act1, wst, ld_acc, tid);
         }
 
         // ---- store
         if (a.mode == kModeLogProb) {
-            if (tid < nm) {  // flow.py:46-47
-                float lat = 0.f;
-                for (int j = 0; j < D; ++j) lat += latent_logpdf(xs[pmod(j - a.rot_total, D) * TM + tid], a.lc);
-                a.lp[m0 + tid] = nan_to_num_lp(lat + ld_acc);
-            }
+            if (tid < nm) a.lp[m0 + tid] = tile_lp(a, xs, TM, tid, ld_acc);
         } else {
-            const int rot_out = INVERSE ? 0 : a.rot_total;
-            if (a.y) {
-                for (int e = tid; e < nm * D; e += kChainThreads) {
-                    const int m = e / D, j = e - m * D;
-                    a.y[m0 * D + e] = xs[pmod(j - rot_out, D) * TM + m];
-                }
-            }
+            if (a.y) store_tile<kChainThreads, TM>(a.y, m0, nm, D, INVERSE ? 0 : a.rot_total, xs, tid);
             if (!INVERSE && a.log_det && tid < nm) a.log_det[m0 + tid] = a.acc_log_det ? a.log_det[m0 + tid] + ld_acc : ld_acc;
         }
         __syncthreads();
@@ -529,25 +614,24 @@ __global__ void __launch_bounds__(kChainThreads, 2) chain_kernel(const __grid_co
 }
 
 // =============================================================================================
-// Tensor-core chain kernel (tcgen05, 3xTF32): same program, same outputs as chain_kernel.
+// Tensor-core chain kernel (tcgen05, 3xFP16 on kind::f16): same program, same outputs as chain_kernel.
 //
 // One CTA per SM, 128 events per tile, 10 warps:
-//   warps 0-7  epilogue / SIMT: ShiftBounds, BatchNorm + first Dense (K = F is tiny), bias+swish+split of
+//   warps 0-7  epilogue / SIMT: tile load and store, ShiftBounds, BatchNorm + first Dense, bias+swish+split of
 //              every hidden layer, the spline rows, latent log-pdf.  Thread (q*32+lane, half): TMEM lane
 //              quarter q = warp%4 (hardware rule), column half = warp/4.
-//   warp 8     weight producer: 1-D bulk copies of pre-split K-major weight images L2 -> 4-stage smem ring
-//   warp 9     MMA issuer: tcgen05.mma kind::tf32, A (activations) in tensor memory, B from the ring,
-//              fp32 accumulators in tensor memory; also owns the TMEM allocation.
-// Tensor memory (512 columns): A_hi [0,128) | A_lo [128,256) | D0 [256,384) | D1 [384,512).
-// Hidden layers accumulate into D0; the last layer runs one transformed dim at a time, alternating
-// D0/D1 so that the spline rows of dim j (warps 0-3 for even j, 4-7 for odd j) overlap the MMAs of j+1.
-// 3xFP16 split on kind::f16 (zf_umma.cuh): x = hi + lo' * 2^-11 (fp16 each), main = A_hi*B_hi and
-// cross = A_lo'*B_hi + A_hi*B_lo' in separate accumulators, theta = main + cross * 2^-11: fp32-class accuracy
-// (measured: below fp32 sgemm's error) at twice the tensor rate and half the operand bytes of the 3xTF32 split
-// it replaces; a single TF32/BF16 pass would break the rel-1e-5 parity (SURVEY H2).  Valid while the
-// conditioner's activations and weights stay below 65504 in magnitude (beyond that the event's result is NaN).
-// Tensor memory (512 columns): A_hi [0,64) | A_lo [64,128) as fp16 pairs; hidden layers main [256,384), cross
-// [384,512); last layer, buffer b: main [128 + 192 b, +96), cross 96 columns further.
+//   warp 8     producer: 1-D bulk copies of pre-split K-major weight images L2 -> 4-stage smem ring, the
+//              per-coupling constant blocks and the next tile's raw rows
+//   warp 9     MMA issuer: A (activations) in tensor memory, B from the ring, fp32 accumulators in tensor memory;
+//              also owns the TMEM allocation.
+// 3xFP16 split (zf_umma.cuh): x = hi + lo' * 2^-11 (fp16 each), main = A_hi*B_hi and cross = A_lo'*B_hi + A_hi*B_lo'
+// in separate accumulators, theta = main + cross * 2^-11: fp32-class accuracy (measured: below fp32 sgemm's error);
+// a single TF32/BF16 pass would break the rel-1e-5 parity (SURVEY H2).  Valid while the conditioner's activations
+// and weights stay below 65504 in magnitude (beyond that the event's result is NaN).
+// Tensor memory (512 columns): A_hi [0,64) | A_lo [64,128) as fp16 pairs; tensor-core first Dense [128,256); hidden
+// layers main [256,384), cross [384,512); last layer, buffer b: main [128 + 192 b, +96), cross 96 columns further.
+// The last layer runs one transformed dim at a time, alternating buffers, so that the spline rows of dim j (warps 0-3
+// for even j, 4-7 for odd j) overlap the MMAs of j+1.
 // =============================================================================================
 #ifdef ZF_TRACE   // developer build only (scripts/trace_chain.py): per-phase clock64 stamps of one steady-state tile
 __device__ long long g_zf_trace[4][64];
@@ -803,8 +887,6 @@ struct UCtx {
     long long n_tiles;
     UCst cl;
     int cst_stride;   // floats between the two constant buffers (0 in the VJP kernel: one coupling, one buffer)
-    bool in16;
-    uint32_t in_bytes;
 };
 template <int ET>
 __device__ __forceinline__ void epi_barrier() { asm volatile("bar.sync 1, %0;" ::"n"(ET) : "memory"); }
@@ -933,6 +1015,21 @@ __device__ __forceinline__ void stream_unit(uint64_t* full, uint64_t* empty, flo
     }
 }
 
+// Full tiles of 16-byte-aligned inputs are fetched ahead by the producer warp (bulk copies of the raw rows); the tail
+// tile and unaligned inputs are read by the tile-loading threads themselves, and so is everything when sampling
+// without conditioning inputs (nothing to fetch).
+__device__ __forceinline__ bool tile_by_bulk(const ChainArgs& a, long long t) {
+    return ((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.c)) & 15) == 0 && (!a.sample || a.C != 0) &&
+           (t + 1) * UM <= a.M;
+}
+// Producer: the raw rows of tile t ([UM][D] of x unless sampling, then [UM][C] of c) -> dst, completing on `full`
+__device__ __forceinline__ void fetch_tile_rows(const ChainArgs& a, long long t, float* dst, uint64_t* full) {
+    const uint32_t xbytes = a.sample ? 0u : (uint32_t)(UM * a.D * 4), cbytes = (uint32_t)(UM * a.C * 4);
+    mbar_arrive_expect_tx(full, xbytes + cbytes);
+    if (!a.sample) bulk_copy_g2s(dst, a.x + t * UM * a.D, xbytes, full);
+    if (a.C) bulk_copy_g2s(dst + UM * a.D, a.c + t * UM * a.C, cbytes, full);
+}
+
 // MMA issuer: the MMAs of one unit (N = 128 for a hidden layer, NL for one transformed dim of the last layer) into the
 // main (dmain) and cross (dcross) accumulators, then `done` is committed.  newver: the unit reads a new version of the
 // activations, whose K-chunk c is waited for (aready[c], phase p_ar) before chunk c's MMAs, and chunks [0, nfree) before
@@ -1009,7 +1106,6 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
     const float* wsf = a.ws;
     const uint32_t tb = cx.tb;
     const long long n_tiles = cx.n_tiles;
-    auto tile_by_bulk = [&](long long t) { return cx.in16 && cx.in_bytes != 0 && (t + 1) * UM <= a.M; };
     const uint32_t lane_base = (uint32_t)(q * 32);
     uint32_t p_fh = 0, p_fd = 0;
     ZF_TR_DECL;
@@ -1023,65 +1119,9 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
         ZF_TR(trs);
         const long long m0 = tile * UM;
         const int nm = (int)min((long long)UM, a.M - m0);
-        // rows -> feature-major tile; padding events sit at 0.5 / 0 and are never stored
-        const bool bulk = tile_by_bulk(tile);
+        const bool bulk = tile_by_bulk(a, tile);
         if (bulk) mbar_wait(&bars[B_XFULL], xk & 1u);
-        const float* xsrc = bulk ? xraw : a.x + m0 * D;
-        const float* csrc = bulk ? xraw + UM * D : a.c + m0 * C;
-        const bool xs16 = (D & 3) == 0 && (a.sample || (reinterpret_cast<uintptr_t>(xsrc) & 15) == 0);
-        const bool cs16 = C > 0 && (C & 3) == 0 && (reinterpret_cast<uintptr_t>(csrc) & 15) == 0;
-        if (xs16) {
-            // this thread: every second group of four columns of its own event, one 16-byte read per group and
-            // conflict-free writes into the feature-major tile
-            const float4* xr = reinterpret_cast<const float4*>(xsrc + (size_t)m * D);
-            for (int q = half; q < (D >> 2); q += NG) {
-                float4 v = make_float4(0.5f, 0.5f, 0.5f, 0.5f);
-                if (m < nm) {
-                    if (a.sample) {   // counter-based draws: the value of (event, column) does not depend on who computes it
-                        float dr[4];
-#pragma unroll 1
-                        for (int i = 0; i < 4; ++i) dr[i] = latent_draw(a.lc.kind, a.peakness, a.seed, m0 + m, 4 * q + i);
-                        v = make_float4(dr[0], dr[1], dr[2], dr[3]);
-                    } else {
-                        v = xr[q];
-                    }
-                }
-                int col = pmod(4 * q - rot_in, D);
-                const float o[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    xs[col * UM + m] = o[i];
-                    if (++col == D) col = 0;
-                }
-            }
-        } else {   // element e = mm * D + j, advanced by 256 per round without dividing
-            int mm = tid / D, j = tid - mm * D;
-            const int dm = ET / D, dj = ET - dm * D;
-            for (int e = tid; e < UM * D; e += ET) {
-                int col = j - rot_in;
-                if (col < 0) col += D;
-                xs[col * UM + mm] =
-                    (mm < nm) ? (a.sample ? latent_draw(a.lc.kind, a.peakness, a.seed, m0 + mm, j) : xsrc[e]) : 0.5f;
-                mm += dm; j += dj;
-                if (j >= D) { j -= D; ++mm; }
-            }
-        }
-        if (cs16) {
-            const float4* cr = reinterpret_cast<const float4*>(csrc + (size_t)m * C);
-            for (int q = half; q < (C >> 2); q += NG) {
-                const float4 v = (m < nm) ? cr[q] : make_float4(0.f, 0.f, 0.f, 0.f);
-                cs[(4 * q + 0) * UM + m] = v.x; cs[(4 * q + 1) * UM + m] = v.y;
-                cs[(4 * q + 2) * UM + m] = v.z; cs[(4 * q + 3) * UM + m] = v.w;
-            }
-        } else if (C) {
-            int mm = tid / C, j = tid - mm * C;
-            const int dm = ET / C, dj = ET - dm * C;
-            for (int e = tid; e < UM * C; e += ET) {
-                cs[j * UM + mm] = (mm < nm) ? csrc[e] : 0.f;
-                mm += dm; j += dj;
-                if (j >= C) { j -= C; ++mm; }
-            }
-        }
+        load_tile<ET, UM>(a, bulk ? xraw : a.x + m0 * D, bulk ? xraw + UM * D : a.c + m0 * C, m0, nm, rot_in, xs, cs, tid);
         if (bulk) { umma::mbar_arrive(&bars[B_XEMPTY]); ++xk; }
         // the log-det this tile accumulates onto (train forward: one launch per coupling) is requested now, not at the end
         float ld_prev = 0.f;
@@ -1091,7 +1131,7 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
 
         float ld_acc = 0.f;
         for (int si = 0; si < a.n_steps; ++si) {
-            const StepDesc& s = steps[INVERSE ? (a.n_steps - 1 - si) : si];
+            const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
             if (s.kind == kStepKindShiftBounds) {
                 // columns split between the groups; groups 1.. hand their log-det share over through ldx
                 float ld_sb = 0.f;
@@ -1310,37 +1350,9 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
         // ---- store
         if (VJP) {
         } else if (a.mode == kModeLogProb) {
-            if (half == 0 && m < nm) {
-                float lat = 0.f;
-                for (int j = 0; j < D; ++j) lat += latent_logpdf(xs[pmod(j - a.rot_total, D) * UM + m], a.lc);
-                a.lp[m0 + m] = nan_to_num_lp(lat + ld_acc);
-            }
+            if (half == 0 && m < nm) a.lp[m0 + m] = tile_lp(a, xs, UM, m, ld_acc);
         } else {
-            const int rot_out = INVERSE ? 0 : a.rot_total;
-            if (a.y) {
-                if ((D & 3) == 0 && (reinterpret_cast<uintptr_t>(a.y) & 15) == 0) {
-                    // this thread: every second group of four columns of its own event (conflict-free reads of the
-                    // feature-major tile, one 16-byte store per group)
-                    if (m < nm) {
-                        float4* yr = reinterpret_cast<float4*>(a.y + (m0 + m) * D);
-                        for (int q = half; q < (D >> 2); q += NG) {
-                            int col = pmod(4 * q - rot_out, D);
-                            float o[4];
-#pragma unroll
-                            for (int i = 0; i < 4; ++i) {
-                                o[i] = xs[col * UM + m];
-                                if (++col == D) col = 0;
-                            }
-                            yr[q] = make_float4(o[0], o[1], o[2], o[3]);
-                        }
-                    }
-                } else {
-                    for (int e = tid; e < nm * D; e += ET) {
-                        const int mm = e / D, j = e - mm * D;
-                        a.y[m0 * D + e] = xs[pmod(j - rot_out, D) * UM + mm];
-                    }
-                }
-            }
+            if (a.y) store_tile<ET, UM>(a.y, m0, nm, D, INVERSE ? 0 : a.rot_total, xs, tid);
             if (!INVERSE && a.log_det && half == 0 && m < nm)
                 a.log_det[m0 + m] = a.acc_log_det ? ld_prev + ld_acc : ld_acc;
         }
@@ -1404,23 +1416,17 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
     umma::fence_after_sync();
     const uint32_t tb = *tmem_slot;
     const long long n_tiles = (a.M + UM - 1) / UM;
-    // Full tiles of 16-byte-aligned inputs are fetched one tile ahead by the producer warp (bulk copies of the raw
-    // rows); the tail tile and unaligned inputs are read by the epilogue warps themselves.
-    const uint32_t in_bytes = (a.sample ? 0u : (uint32_t)(UM * D * 4)) + (uint32_t)(UM * C * 4);
-    const bool in16 = ((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.c)) & 15) == 0;
-    auto tile_by_bulk = [&](long long t) { return in16 && in_bytes != 0 && (t + 1) * UM <= a.M; };
     // the coupling that follows step position `si` in processing order, cyclically (the next tile starts over)
     auto next_coupling = [&](int si) -> const StepDesc& {
         for (int k = 1; k <= a.n_steps; ++k) {
-            const int sj = (si + k) % a.n_steps;
-            const StepDesc& t = steps[INVERSE ? (a.n_steps - 1 - sj) : sj];
+            const StepDesc& t = step_at<INVERSE>(steps, a.n_steps, (si + k) % a.n_steps);
             if (t.kind == kStepKindCoupling) return t;
         }
         return steps[0];   // not reached: this kernel is only launched for chains with a coupling
     };
     int last_coupling_si = 0;
     for (int si = 0; si < a.n_steps; ++si)
-        if (steps[INVERSE ? (a.n_steps - 1 - si) : si].kind == kStepKindCoupling) last_coupling_si = si;
+        if (step_at<INVERSE>(steps, a.n_steps, si).kind == kStepKindCoupling) last_coupling_si = si;
 
     auto producer_role = [&]() {
         // ------------------------------------------------------------------ producer: weights, constants, inputs
@@ -1438,11 +1444,9 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
                 ++kc;
             };
             auto issue_inputs = [&](long long t) {
-                if (!tile_by_bulk(t)) return;
+                if (!tile_by_bulk(a, t)) return;
                 mbar_wait(&bars[B_XEMPTY], (xk & 1u) ^ 1u);
-                mbar_arrive_expect_tx(&bars[B_XFULL], in_bytes);
-                if (!a.sample) bulk_copy_g2s(xraw, a.x + t * UM * D, (uint32_t)(UM * D * 4), &bars[B_XFULL]);
-                if (C) bulk_copy_g2s(xraw + UM * D, a.c + t * UM * C, (uint32_t)(UM * C * 4), &bars[B_XFULL]);
+                fetch_tile_rows(a, t, xraw, &bars[B_XFULL]);
                 ++xk;
             };
             if ((long long)blockIdx.x < n_tiles) {
@@ -1453,7 +1457,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
                 const bool more_tiles = tile + gridDim.x < n_tiles;
                 bool inputs_pending = more_tiles;
                 for (int si = 0; si < a.n_steps; ++si) {
-                    const StepDesc& s = steps[INVERSE ? (a.n_steps - 1 - si) : si];
+                    const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
                     if (s.kind != kStepKindCoupling) continue;
                     const int L = s.n_hidden, NL = ru(3 * s.K - 1, 16);
                     for (int u = 0; u < (L - 1) + s.d; ++u) {
@@ -1491,7 +1495,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
         for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             ZF_TR_TILE;
             for (int si = 0; si < a.n_steps; ++si) {
-                const StepDesc& s = steps[INVERSE ? (a.n_steps - 1 - si) : si];
+                const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
                 if (s.kind != kStepKindCoupling) continue;
                 const int L = s.n_hidden, NL = ru(3 * s.K - 1, 16);
                 const bool tcfd = a.u_w0img && s.F <= 16;
@@ -1556,7 +1560,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
         }
     };
     // ------------------------------------------------------------------ role dispatch
-    const UCtx cx{a, xs, cs, xraw, hs, cst, ldx, reinterpret_cast<float4*>(scratch), bars, steps, tb, n_tiles, cl, cst_stride, in16, in_bytes};
+    const UCtx cx{a, xs, cs, xraw, hs, cst, ldx, reinterpret_cast<float4*>(scratch), bars, steps, tb, n_tiles, cl, cst_stride};
     if (warp == PW) producer_role();
     else if (warp == MW) mma_role();
     else umma_epilogue_role<INVERSE, VJP>(cx);
@@ -1644,28 +1648,24 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
     if (tid == 0) {
         int n = 0;
         for (int si = 0; si < a.n_steps; ++si)
-            if (steps[INVERSE ? (a.n_steps - 1 - si) : si].kind == kStepKindCoupling) coup_si[n++] = si;
+            if (step_at<INVERSE>(steps, a.n_steps, si).kind == kStepKindCoupling) coup_si[n++] = si;
     }
     __syncthreads();
     int ncoup = 0;
     for (int si = 0; si < a.n_steps; ++si)
         if (steps[si].kind == kStepKindCoupling) ++ncoup;
-    auto step_at = [&](int si) -> const StepDesc& { return steps[INVERSE ? (a.n_steps - 1 - si) : si]; };
 
     const long long n_tiles = (a.M + UM - 1) / UM;
     const long long n_my = ((long long)blockIdx.x < n_tiles) ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     const long long n_occ = n_my * ncoup;       // (coupling, tile) occurrences of this CTA, in schedule order
     auto tile_of = [&](long long k) { return (long long)blockIdx.x + k * gridDim.x; };
-    const uint32_t in_bytes = (a.sample ? 0u : (uint32_t)(UM * D * 4)) + (uint32_t)(UM * C * 4);
-    const bool in16 = ((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.c)) & 15) == 0;
-    auto tile_by_bulk = [&](long long t) { return in16 && in_bytes != 0 && (t + 1) * UM <= a.M; };
     // the coupling step of occurrence n: pairs of tiles, coupling-major, slot-minor
     auto occ_step = [&](long long n) -> const StepDesc& {
         const long long per_pair = 2LL * ncoup;
         const long long p = n / per_pair;
         const long long r = n - p * per_pair;
         const int nslots = (2 * p + 1 < n_my) ? 2 : 1;
-        return step_at(coup_si[(int)(r / nslots)]);
+        return step_at<INVERSE>(steps, a.n_steps, coup_si[(int)(r / nslots)]);
     };
 
     // ------------------------------------------------------------------------------------------------ roles
@@ -1687,14 +1687,11 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         auto issue_inputs = [&](long long k) {
             if (k >= n_my) return;
             const long long t = tile_of(k);
-            if (!tile_by_bulk(t)) return;
+            if (!tile_by_bulk(a, t)) return;
             const int b = (int)(k & 1);
             const uint32_t use = (uint32_t)(k >> 1);
-            float* dst = xraw + (size_t)b * UM * (D + C);
             mbar_wait(&bars[PP_XEMPTY + b], (use & 1u) ^ 1u);
-            mbar_arrive_expect_tx(&bars[PP_XFULL + b], in_bytes);
-            if (!a.sample) bulk_copy_g2s(dst, a.x + t * UM * D, (uint32_t)(UM * D * 4), &bars[PP_XFULL + b]);
-            if (C) bulk_copy_g2s(dst + UM * D, a.c + t * UM * C, (uint32_t)(UM * C * 4), &bars[PP_XFULL + b]);
+            fetch_tile_rows(a, t, xraw + (size_t)b * UM * (D + C), &bars[PP_XFULL + b]);
         };
         issue_inputs(0);
         issue_inputs(1);
@@ -1702,7 +1699,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         for (long long p = 0; 2 * p < n_my; ++p) {
             const int nslots = (2 * p + 1 < n_my) ? 2 : 1;
             for (int si = 0; si < a.n_steps; ++si) {
-                const StepDesc& s = step_at(si);
+                const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
                 if (s.kind != kStepKindCoupling) continue;
                 const int L = s.n_hidden, NL = ru(3 * s.K - 1, 16);
                 for (int slot = 0; slot < nslots; ++slot) {
@@ -1729,7 +1726,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         for (long long p = 0; 2 * p < n_my; ++p) {
             const int nslots = (2 * p + 1 < n_my) ? 2 : 1;
             for (int si = 0; si < a.n_steps; ++si) {
-                const StepDesc& s = step_at(si);
+                const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
                 if (s.kind != kStepKindCoupling) continue;
                 const int L = s.n_hidden, NL = ru(3 * s.K - 1, 16);
                 for (int slot = 0; slot < nslots; ++slot) {
@@ -1773,7 +1770,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         long long bn_done = -1;   // occurrence whose BatchNorm output is already in hs2[n & 1]
         // waits + hstack(xc, c) + eval BatchNorm (bijectors.py:341-342) of occurrence n = (pair p, coupling cj, slot)
         auto batch_norm = [&](long long n, long long p, int cj, int slot) {
-            const StepDesc& s = step_at(coup_si[cj]);
+            const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, coup_si[cj]);
             const int d = s.d, F = s.F, F_p = ru(F, KC), rot = s.rot;
             const long long k = 2 * p + slot;
             const int tbuf = (int)(k % PP_TBUF);
@@ -1795,7 +1792,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
             const int nslots = (2 * p + 1 < n_my) ? 2 : 1;
             int cj = -1;   // ordinal of the coupling inside the step program
             for (int si = 0; si < a.n_steps; ++si) {
-                const StepDesc& s = step_at(si);
+                const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
                 if (s.kind != kStepKindCoupling) continue;
                 ++cj;
                 const int F = s.F, L = s.n_hidden;
@@ -1862,37 +1859,16 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
             const long long tile = tile_of(k), m0 = tile * UM;
             const int nm = (int)min((long long)UM, a.M - m0);
             const int rb = (int)(k & 1);
-            // rows -> feature-major tile; padding events sit at 0.5 / 0 and are never stored
-            const bool bulk = tile_by_bulk(tile);
+            const bool bulk = tile_by_bulk(a, tile);
             const float* raw = xraw + (size_t)rb * UM * (D + C);
             if (bulk) mbar_wait(&bars[PP_XFULL + rb], (uint32_t)((k >> 1) & 1));
-            const float* xsrc = bulk ? raw : a.x + m0 * D;
-            const float* csrc = bulk ? raw + UM * D : a.c + m0 * C;
-            {
-                int mm = t2 / D, j = t2 - mm * D;
-                const int dm = 128 / D, dj = 128 - dm * D;
-                for (int e = t2; e < UM * D; e += 128) {
-                    int col = j - rot_in;
-                    if (col < 0) col += D;
-                    xs[col * UM + mm] =
-                        (mm < nm) ? (a.sample ? latent_draw(a.lc.kind, a.peakness, a.seed, m0 + mm, j) : xsrc[e]) : 0.5f;
-                    mm += dm; j += dj;
-                    if (j >= D) { j -= D; ++mm; }
-                }
-            }
-            if (C) {
-                int mm = t2 / C, j = t2 - mm * C;
-                const int dm = 128 / C, dj = 128 - dm * C;
-                for (int e = t2; e < UM * C; e += 128) {
-                    cs[j * UM + mm] = (mm < nm) ? csrc[e] : 0.f;
-                    mm += dm; j += dj;
-                    if (j >= C) { j -= C; ++mm; }
-                }
-            }
+            // D is 2 or 3 here (d = D / 2 = 1): the 16-byte path of x would be dead code in the row warps' register budget
+            load_tile<128, UM, false>(a, bulk ? raw : a.x + m0 * D, bulk ? raw + UM * D : a.c + m0 * C, m0, nm, rot_in, xs, cs, t2);
             if (bulk) umma::mbar_arrive(&bars[PP_XEMPTY + rb]);
             s2_barrier();
             float ld0 = 0.f;
-            for (int si = 0; si < fc; ++si) shift_bounds_row<INVERSE>(step_at(si), wsf, D, xs, UM, m, ld0);   // only non-coupling kind
+            for (int si = 0; si < fc; ++si)   // only non-coupling kind
+                shift_bounds_row<INVERSE>(step_at<INVERSE>(steps, a.n_steps, si), wsf, D, xs, UM, m, ld0);
             lda[m] = ld0;
             signal_ready(k);   // the tile state is complete for the first coupling
         };
@@ -1901,7 +1877,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
         for (long long p = 0; 2 * p < n_my; ++p) {
             const int nslots = (2 * p + 1 < n_my) ? 2 : 1;
             for (int si = fc; si < a.n_steps; ++si) {
-                const StepDesc& s = step_at(si);
+                const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
 #pragma unroll 1
                 for (int slot = 0; slot < nslots; ++slot) {
                     const long long k = 2 * p + slot;
@@ -1946,7 +1922,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         ++n2;
                     }
                     // as soon as this tile's state is complete for its next coupling, tell the activation warps
-                    if (si + 1 < a.n_steps && step_at(si + 1).kind == kStepKindCoupling) signal_ready(k);
+                    if (si + 1 < a.n_steps && step_at<INVERSE>(steps, a.n_steps, si + 1).kind == kStepKindCoupling) signal_ready(k);
                     // the tile that takes this slot in the next pair: its buffers were released two pairs ago.  It is
                     // published here, not after both slots: the activation warps may wait for it while they still owe
                     // this pair's other slot (in a chain of one coupling, before that slot's spline rows can run).
@@ -1954,20 +1930,10 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                     if (si == a.n_steps - 1) {
                         // ---- store this tile
                         if (a.mode == kModeLogProb) {
-                            if (m < nm) {
-                                float lat = 0.f;
-                                for (int j = 0; j < D; ++j) lat += latent_logpdf(xs[pmod(j - a.rot_total, D) * UM + m], a.lc);
-                                a.lp[m0 + m] = nan_to_num_lp(lat + lda[m]);
-                            }
+                            if (m < nm) a.lp[m0 + m] = tile_lp(a, xs, UM, m, lda[m]);
                         } else {
-                            const int rot_out = INVERSE ? 0 : a.rot_total;
                             s2_barrier();
-                            if (a.y) {
-                                for (int e = t2; e < nm * D; e += 128) {
-                                    const int mm = e / D, j = e - mm * D;
-                                    a.y[m0 * D + e] = xs[pmod(j - rot_out, D) * UM + mm];
-                                }
-                            }
+                            if (a.y) store_tile<128, UM>(a.y, m0, nm, D, INVERSE ? 0 : a.rot_total, xs, t2);
                             if (!INVERSE && a.log_det && m < nm)
                                 a.log_det[m0 + m] = a.acc_log_det ? a.log_det[m0 + m] + lda[m] : lda[m];
                             s2_barrier();
