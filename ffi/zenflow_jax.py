@@ -14,6 +14,9 @@ reference call site                                   -> handler
   Flow.sample                        flow.py:50-78    -> ZfFlowSample       (flow_sample, a jax.custom_vjp; Philox mode)
                                                          or latent.sample (jax.random) + chain_inverse (parity mode)
   jax.grad of either (wrt z, c, params)               -> ZfChainInverseVjp  (their backward rule)
+  Flow.sample_and_log_prob / inverse_and_log_prob     -> ZfFlowSampleLogProb (flow_sample_and_log_prob,
+                                                         inverse_and_log_prob: jax.custom_vjps with two outputs)
+  jax.grad of either (wrt z, c, params)               -> ZfFlowSampleLogProbVjp (their backward rule)
   Flow.__call__(train=True, mutable=["batch_stats"]) + jax.grad(loss_fn)   train.py:64-86
                                                       -> ZfFlowTrain        (flow_log_prob_train, a jax.custom_vjp)
   optimizer.update + apply_updates  train.py:84-85    -> ZfNadamwUpdate     (nadamw_update)
@@ -37,6 +40,8 @@ _TARGETS = {
     "zf_chain_inverse": "ZfChainInverse",
     "zf_flow_sample": "ZfFlowSample",
     "zf_chain_inverse_vjp": "ZfChainInverseVjp",
+    "zf_flow_sample_log_prob": "ZfFlowSampleLogProb",
+    "zf_flow_sample_log_prob_vjp": "ZfFlowSampleLogProbVjp",
     "zf_flow_train": "ZfFlowTrain",
     "zf_nadamw_update": "ZfNadamwUpdate",
 }
@@ -303,6 +308,77 @@ def flow_sample(flow, variables, conditions_or_size, dim: int, *, seed: int = 0,
     _, leaves, is_stat, _, attrs = _operands(flow, variables, like, c)
     extra = dict(_latent(flow), seed=np.int64(seed))
     return _inverse_custom_vjp("zf_flow_sample", like, c, leaves, is_stat, attrs, extra, True, micro_batch)
+
+
+def _sample_log_prob_custom_vjp(z_or_like, c, leaves, is_stat, attrs, extra, sample, micro_batch):
+    """ZfFlowSampleLogProb wrapped in a jax.custom_vjp with two outputs (x, lp) whose backward runs
+    ZfFlowSampleLogProbVjp (one zf_flow_sample_log_prob_vjp call) with the running statistics held fixed; the statistics
+    leaves get zero cotangents, and z gets none when sampling (the draw is a constant)."""
+    import jax
+    import jax.numpy as jnp
+    import numpy as np
+
+    def _head(z, c):
+        return [z] if c is None else [z, c]
+
+    flags = dict(extra, sample=np.int32(1 if sample else 0))
+
+    @jax.custom_vjp
+    def f(z, c, leaves):
+        outs = (jax.ShapeDtypeStruct(z.shape, jnp.float32), jax.ShapeDtypeStruct(z.shape[:1], jnp.float32))
+        call = jax.ffi.ffi_call("zf_flow_sample_log_prob", outs)
+        return tuple(call(*_head(z, c), *leaves, **attrs, **flags))
+
+    def f_fwd(z, c, leaves):
+        return f(z, c, leaves), (z, c, leaves)
+
+    def f_bwd(saved, cts):
+        z, c, leaves = saved
+        ct_x, ct_lp = cts
+        outs = [] if sample else [jax.ShapeDtypeStruct(z.shape, jnp.float32)]
+        outs += [] if c is None else [jax.ShapeDtypeStruct(c.shape, jnp.float32)]
+        outs += [jax.ShapeDtypeStruct(v.shape, jnp.float32) for v, s in zip(leaves, is_stat) if not s]
+        call = jax.ffi.ffi_call("zf_flow_sample_log_prob_vjp", outs)
+        res = iter(call(*_head(z, c), ct_x, ct_lp, *leaves, **attrs, **flags, micro_batch=np.int64(micro_batch)))
+        gz = jnp.zeros_like(z) if sample else next(res)
+        gc = None if c is None else next(res)
+        gl = [jnp.zeros_like(v) if s else next(res) for v, s in zip(leaves, is_stat)]
+        return gz, gc, gl
+
+    f.defvjp(f_fwd, f_bwd)
+    return f(z_or_like, c, list(leaves))
+
+
+def inverse_and_log_prob(flow, variables, z, c=None, *, micro_batch: int = 1 << 18):
+    """(Chain.inverse(z, c), its log-density) in one fused pass: lp = nan_to_num(latent.log_prob(z) - log|det dx/dz|),
+    the density of the map that produced x (include/zenflow_b200.h, zf_flow_sample_log_prob).  A jax.custom_vjp with two
+    outputs: jax.grad wrt z, c and the params leaves runs ZfFlowSampleLogProbVjp."""
+    import numpy as np
+
+    register()
+    _, leaves, is_stat, _, attrs = _operands(flow, variables, z, c)
+    extra = dict(_latent(flow), seed=np.int64(0))
+    return _sample_log_prob_custom_vjp(z, c, leaves, is_stat, attrs, extra, False, micro_batch)
+
+
+def flow_sample_and_log_prob(flow, variables, conditions_or_size, dim: int, *, seed: int = 0, micro_batch: int = 1 << 18):
+    """Flow.sample (Philox draw in-kernel, as flow_sample) and the samples' log-density in one fused pass.  A
+    jax.custom_vjp with two outputs: jax.grad wrt c and the params leaves runs ZfFlowSampleLogProbVjp, which redraws
+    the same latent."""
+    import jax.numpy as jnp
+    import numpy as np
+
+    register()
+    if isinstance(conditions_or_size, int):
+        c, n = None, conditions_or_size
+    else:
+        c = jnp.asarray(conditions_or_size, jnp.float32)
+        c = c.reshape(-1, 1) if c.ndim == 1 else c  # flow.py:100-108 _normalize_c
+        n = c.shape[0]
+    like = jnp.zeros((n, dim), jnp.float32)  # shape carrier (values unread)
+    _, leaves, is_stat, _, attrs = _operands(flow, variables, like, c)
+    extra = dict(_latent(flow), seed=np.int64(seed))
+    return _sample_log_prob_custom_vjp(like, c, leaves, is_stat, attrs, extra, True, micro_batch)
 
 
 def make_flow_log_prob_train(flow, dim: int, cdim: int, *, global_count=None, micro_batch: int = 0):

@@ -212,6 +212,21 @@ int zf_flow_log_prob(void* stream, const zf_chain* chain, int32_t latent_kind, f
 int zf_flow_sample(void* stream, const zf_chain* chain, int32_t latent_kind, float peakness, uint64_t seed,
                    const float* c, int64_t M, float* x, void* workspace, size_t workspace_bytes);
 
+/* Flow.sample_and_log_prob / Flow.inverse_and_log_prob: a draw and its log-density in ONE inverse pass.
+ *   x  = Chain.inverse(z, c), bit-identical to zf_chain_inverse (z given) / zf_flow_sample (z NULL: drawn in-kernel
+ *        from (latent_kind, peakness, seed) exactly as zf_flow_sample draws it)
+ *   lp = nan_to_num(sum_j log p_latent(z_j) - log|det dx/dz|), nan_to_num as zf_flow_log_prob's
+ * log|det dx/dz| is the exact change of variables of the inverse as bijectors.py / utils.py write it: per transformed
+ * element, log|dx/dy| of the analytic quadratic-root inverse (utils.py:191-201: no EPS, no clip) in the bin the inverse
+ * searched; ShiftBounds.inverse adds log(b - a) (two-sided column), log(xmax - xmin) (unbounded) or
+ * u + log(xmax - xmin) (one-sided: x = a + e^u or b - e^u); Roll and elements outside [0, 1) add 0.  This is the
+ * density of the map that produced x, not zf_flow_log_prob(x): that one differs by the forward's EPS terms and clip
+ * and by bin flips near knots.  The idx == K corner gives NaN x (as zf_chain_inverse) and lp = -FLT_MAX.
+ *   x (M,D)     optional output (NULL: lp only); log_prob (M,) required; same workspace as zf_chain_inverse */
+int zf_flow_sample_log_prob(void* stream, const zf_chain* chain, int32_t latent_kind, float peakness, uint64_t seed,
+                            const float* z, const float* c, int64_t M, float* x, float* log_prob, void* workspace,
+                            size_t workspace_bytes);
+
 /* The same passes with the per-call parameter re-layout hoisted out: zf_chain_pack writes the packed parameter
  * blocks of `chain` into `workspace` once (after every parameter / statistics update); the *_packed calls then
  * only launch the fused kernel.  `chain` must describe the same ops and the same workspace must be passed. */
@@ -388,6 +403,21 @@ int zf_chain_inverse_vjp(void* stream, const zf_chain* chain, const zf_coupling_
                          int32_t latent_kind, float peakness, uint64_t seed, const float* c, int64_t M,
                          const float* x_cotangent, float* x, float* gz, float* gc,
                          void* workspace, size_t workspace_bytes, int64_t micro_batch);
+
+/* ---- VJP of zf_flow_sample_log_prob: (x, lp) jointly ------------------------------------------------------------
+ * zf_chain_inverse_vjp's plan and loop plus the log-density: every group's inverse log-det takes the per-event
+ * cotangent -lp_cotangent, gz also takes lp_cotangent d log p_latent / dz, and events whose lp is not finite
+ * (nan_to_num) take a zero lp cotangent (their x cotangent flows as in zf_chain_inverse_vjp).  Running statistics are
+ * constants.  Validation and layout as zf_chain_inverse_vjp, except:
+ *   x_cotangent (M,D) or NULL, lp_cotangent (M,) or NULL; not both NULL.  With lp_cotangent NULL the outputs are
+ *                 bit-identical to zf_chain_inverse_vjp's
+ *   lp (M,)       optional output: the log-density as zf_flow_sample_log_prob computes it
+ *   workspace     zf_flow_sample_log_prob_vjp_workspace_bytes (the plan's, with room for the whole chain's pass) */
+size_t zf_flow_sample_log_prob_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch);
+int zf_flow_sample_log_prob_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, const float* z,
+                                int32_t latent_kind, float peakness, uint64_t seed, const float* c, int64_t M,
+                                const float* x_cotangent, const float* lp_cotangent, float* x, float* lp, float* gz,
+                                float* gc, void* workspace, size_t workspace_bytes, int64_t micro_batch);
 
 /* ---- Deep-Set conditioner Phi (examples/deep_set.ipynb:138-160; SURVEY.md 8f-4) ---------------------------
  * The FLAX module on the other side of the flow's conditions in the deep_set config:

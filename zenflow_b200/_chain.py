@@ -1,5 +1,5 @@
-"""Host-side assembly of the native chain description (zf_chain), the eval calls and the VJPs of the eval log-density
-and of the inverse / sample pass.
+"""Host-side assembly of the native chain description (zf_chain), the eval calls and the VJPs of the eval log-density,
+of the inverse / sample pass and of the fused sample-and-log-density pass.
 
 A ``ChainSpec`` is what the bijector modules emit: the op list of a Chain with device
 pointers to the FLAX variable leaves.  It owns the torch tensors behind those pointers for
@@ -251,6 +251,75 @@ class ChainSpec:
                    "zf_chain_inverse_vjp")
         return gz, gc, grads, x
 
+    def _draw_inputs(self, z, c, n):
+        """(zd, cd, M): the float32 device tensors of a given draw z and its conditions, or (z None) zd = None and the
+        conditions of ``n`` rows drawn in-kernel."""
+        if z is not None:
+            zd, cd = self._inputs(z, c)
+            return zd, cd, int(zd.shape[0])
+        return None, self._conditions(int(n), c), int(n)
+
+    def sample_log_prob(self, z, c, latent_kind: int, peakness: float, *, draw_seed: Optional[int] = None,
+                        n: Optional[int] = None, want_x: bool = True):
+        """Flow.sample_and_log_prob / Flow.inverse_and_log_prob: x = Chain.inverse(z, c) and its log-density in one fused
+        pass (zf_flow_sample_log_prob).  z None: draw ``n`` latent rows in-kernel with ``draw_seed`` as zf_flow_sample
+        does.  Returns ``(x, lp)`` (x None when not asked for)."""
+        lib = _lib.load()
+        zd, cd, M = self._draw_inputs(z, c, n)
+        ch = self._chain()
+        ws, nbytes = self._workspace(lib, ch, M)
+        x = torch.empty((M, self.dim), dtype=torch.float32, device=self.device) if want_x else None
+        lp = torch.empty(M, dtype=torch.float32, device=self.device)
+        seed = int(draw_seed or 0) if zd is None else 0
+        _lib.check(lib.zf_flow_sample_log_prob(stream_ptr(), C.byref(ch), int(latent_kind), float(peakness),
+                                               seed & 0xFFFFFFFFFFFFFFFF, ptr(zd), ptr(cd), M, ptr(x), ptr(lp), ptr(ws),
+                                               nbytes), "zf_flow_sample_log_prob")
+        return x, lp
+
+    def sample_log_prob_vjp(self, z, c, latent_kind: int, peakness: float, x_cotangent=None, lp_cotangent=None, *,
+                            draw_seed: Optional[int] = None, n: Optional[int] = None, want_gz: bool = True,
+                            want_gc: bool = True, want_params: bool = True, micro_batch: int = 1 << 18,
+                            want_x: bool = False, want_lp: bool = False):
+        """Joint VJP of (x, lp) of sample_log_prob (zf_flow_sample_log_prob_vjp) for the cotangents ``x_cotangent``
+        (M, D) and ``lp_cotangent`` (M,); either may be None, not both.  z None: the in-kernel draw (no gz).
+
+        Returns ``(gz, gc, param_grads, x, lp)``: float32 device tensors, None where not asked for;
+        ``param_grads[k]`` lists coupling k's gradients in the order of ``coupling_params[k]``."""
+        lib = _lib.load()
+        if x_cotangent is None and lp_cotangent is None:
+            raise ValueError("sample_log_prob_vjp: pass x_cotangent, lp_cotangent or both")
+        zd, cd, M = self._draw_inputs(z, c, n)
+        if zd is None:
+            want_gz = False
+        ch = self._chain()
+        gxc = None
+        if x_cotangent is not None:
+            gxc = to_device_f32(x_cotangent, self.device)
+            if tuple(gxc.shape) != (M, self.dim):
+                raise ValueError(f"x_cotangent must have shape ({M}, {self.dim}), got {tuple(gxc.shape)}")
+        glc = None
+        if lp_cotangent is not None:
+            glc = to_device_f32(lp_cotangent, self.device).reshape(-1)
+            if glc.shape[0] != M:
+                raise ValueError(f"lp_cotangent must have shape ({M},), got {tuple(glc.shape)}")
+        nbytes = int(lib.zf_flow_sample_log_prob_vjp_workspace_bytes(C.byref(ch), M, int(micro_batch)))
+        if nbytes == 0:
+            _lib.check(1, "zf_flow_sample_log_prob_vjp_workspace_bytes")
+        ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
+        base = (ws.data_ptr() + 255) & ~255
+        gz = torch.empty((M, self.dim), dtype=torch.float32, device=self.device) if want_gz else None
+        gc = torch.empty_like(cd) if (want_gc and cd is not None) else None
+        x = torch.empty((M, self.dim), dtype=torch.float32, device=self.device) if want_x else None
+        lp = torch.empty(M, dtype=torch.float32, device=self.device) if want_lp else None
+        grads, arr = self._grads_array(want_params)
+        seed = int(draw_seed or 0) if zd is None else 0
+        _lib.check(lib.zf_flow_sample_log_prob_vjp(stream_ptr(), C.byref(ch), arr, ptr(zd), int(latent_kind),
+                                                   float(peakness), seed & 0xFFFFFFFFFFFFFFFF, ptr(cd), M, ptr(gxc),
+                                                   ptr(glc), ptr(x), ptr(lp), ptr(gz), ptr(gc), base,
+                                                   ws.numel() - (base - ws.data_ptr()), int(micro_batch)),
+                   "zf_flow_sample_log_prob_vjp")
+        return gz, gc, grads, x, lp
+
     def _conditions(self, n: int, c):
         cd = None
         if self.cdim:
@@ -371,3 +440,49 @@ def flow_inverse_differentiable(spec: ChainSpec, z, c) -> torch.Tensor:
 def flow_sample_differentiable(spec: ChainSpec, n: int, c, latent_kind: int, peakness: float, seed: int) -> torch.Tensor:
     """Flow.sample's draw and inverse pass with a grad_fn wrt c and the couplings' params leaves (the draw is a constant)."""
     return _FlowInverse.apply(spec, (int(n), int(latent_kind), float(peakness), int(seed)), None, c, *_param_leaves(spec))
+
+
+class _FlowSampleLogProb(torch.autograd.Function):
+    """Flow.inverse_and_log_prob (``n`` None: the given draw z) or Flow.sample_and_log_prob (``n`` rows drawn in-kernel
+    with ``seed``, z None) as a differentiable op with two outputs (x, lp): forward = zf_flow_sample_log_prob (the
+    non-grad call, so both are bit-identical to it), backward = one zf_flow_sample_log_prob_vjp with the incoming
+    gradients as the cotangents; a gradient autograd does not provide is passed as NULL."""
+
+    @staticmethod
+    def forward(ctx, spec, latent, n, seed, z, c, *leaves):
+        zd, cd, _ = spec._draw_inputs(z, c, n)   # the device tensors the backward reads
+        x, lp = spec.sample_log_prob(zd, cd, *latent, draw_seed=seed, n=n)
+        ctx.spec, ctx.latent, ctx.n, ctx.seed = spec, latent, n, seed
+        ctx.z_like = z.detach() if isinstance(z, torch.Tensor) else None
+        ctx.c_like = c.detach() if isinstance(c, torch.Tensor) else None
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(zd, cd)
+        return x, lp
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_x, g_lp):
+        zd, cd = ctx.saved_tensors
+        spec = ctx.spec
+        need = ctx.needs_input_grad
+        n_in = 6 + len(spec.param_slots)
+        if g_x is None and g_lp is None:
+            return (None,) * n_in
+        gz, gc, grads, _, _ = spec.sample_log_prob_vjp(zd, cd, *ctx.latent, g_x, g_lp, draw_seed=ctx.seed, n=ctx.n,
+                                                       want_gz=need[4], want_gc=need[5], want_params=any(need[6:]))
+        out_p = []
+        for i, (k, j) in enumerate(spec.param_slots):
+            out_p.append(_grad_like(grads[k][j], spec.coupling_params[k][0][j]) if need[6 + i] else None)
+        return (None, None, None, None, _grad_like(gz, ctx.z_like) if need[4] else None,
+                _grad_like(gc, ctx.c_like) if need[5] else None, *out_p)
+
+
+def flow_inverse_log_prob_differentiable(spec: ChainSpec, z, c, latent_kind: int, peakness: float):
+    """(Chain.inverse(z, c), its log-density) with grad_fns wrt every torch tensor among z, c and the params leaves."""
+    return _FlowSampleLogProb.apply(spec, (int(latent_kind), float(peakness)), None, 0, z, c, *_param_leaves(spec))
+
+
+def flow_sample_log_prob_differentiable(spec: ChainSpec, n: int, c, latent_kind: int, peakness: float, seed: int):
+    """Flow.sample's draw, inverse pass and log-density with grad_fns wrt c and the params leaves (the draw is a constant)."""
+    return _FlowSampleLogProb.apply(spec, (int(latent_kind), float(peakness)), int(n), int(seed), None, c,
+                                    *_param_leaves(spec))

@@ -75,7 +75,7 @@ struct PackJob {
     const float *xmin, *xmax;
 };
 
-constexpr int kSbStride = 8;  // floats per column: kind, a, b, xmin, xmax, mul, log(mul), -
+constexpr int kSbStride = 8;  // floats per column: kind, a, b, xmin, xmax, mul, log(mul), log of the inverse's span
 
 // Up to kPackBatch steps per launch (blockIdx.y = step of the batch): kernel parameters may be 32 KB since CUDA 12.1,
 // so a whole chain's jobs travel in one launch instead of one launch per step.
@@ -104,7 +104,9 @@ __global__ void __launch_bounds__(256) pack_step_kernel(const __grid_constant__ 
                 mul = __fdiv_rn(1.0f, __fsub_rn(xmax, xmin));      // bijectors.py:265
             }
             t[0] = (float)kind; t[1] = a; t[2] = b; t[3] = xmin; t[4] = xmax;
-            t[5] = mul; t[6] = logf(mul); t[7] = 0.f;
+            // the inverse's log-det: log(b - a), or log(xmax - xmin) (+ u for a one-sided column)
+            const float span = kind == ZF_BOUND_BOTH ? __fsub_rn(b, a) : __fsub_rn(xmax, xmin);
+            t[5] = mul; t[6] = logf(mul); t[7] = logf(span);
         }
         return;
     }
@@ -224,14 +226,15 @@ __global__ void __launch_bounds__(256) pack_step_kernel(const __grid_constant__ 
     }
 }
 
-enum ChainMode : int { kModeForward = 0, kModeLogProb = 1, kModeInverse = 2, kModeVjp = 3 };
+// kModeInvLogProb: the inverse (or sampling) pass that also writes the log-density of what it produced (ILP kernels)
+enum ChainMode : int { kModeForward = 0, kModeLogProb = 1, kModeInverse = 2, kModeVjp = 3, kModeInvLogProb = 4 };
 
 struct ChainArgs {
     const float* x;     // (M, D) input (x for forward/log_prob, z for inverse)
     const float* c;     // (M, C) or null
     float* y;           // (M, D) output or null
     float* log_det;     // (M,) or null (forward)
-    float* lp;          // (M,) (log_prob)
+    float* lp;          // (M,) (log_prob, inverse log-density)
     const float* ws;    // workspace: StepDesc[n_steps] then packed parameters
     long long M;
     int D, C;
@@ -319,7 +322,8 @@ __device__ __forceinline__ void gemm_pass(const float* __restrict__ act_in, int 
     }
 }
 
-template <bool INVERSE>
+// ILP (inverse log-density mode): ldc accumulates minus the inverse's log|dx/dy|
+template <bool INVERSE, bool ILP = false>
 __device__ __forceinline__ int spline_rows(float* th, int Pst, int K, const KnotNorm& kn, float* xcol,
                                            float& ldc, int tid) {
     // one thread per sample of the tile (tid < TM): theta row -> bin -> transform
@@ -338,11 +342,12 @@ __device__ __forceinline__ int spline_rows(float* th, int Pst, int K, const Knot
         ldc += ld;
     } else {
         xcol[tid] = rqs_eval_inverse(v, b);
+        if (ILP) ldc -= rqs_inverse_log_det(v, b);
     }
     return b.idx;
 }
 
-template <bool INVERSE>
+template <bool INVERSE, bool ILP = false>
 __device__ __forceinline__ void run_coupling(const ChainArgs& a, long long m0, int nm, const StepDesc& s,
                                              const float* __restrict__ wsf, int D, int C,
                                              float* xs, const float* cs, float* act0, float* act1,
@@ -414,7 +419,7 @@ __device__ __forceinline__ void run_coupling(const ChainArgs& a, long long m0, i
         }
         __syncthreads();
         if (tid < TM) {
-            const int idx = spline_rows<INVERSE>(nxt, Pst, K, kn, xs + pmod(jj - rot, D) * TM, ldc, tid);
+            const int idx = spline_rows<INVERSE, ILP>(nxt, Pst, K, kn, xs + pmod(jj - rot, D) * TM, ldc, tid);
             if (tid < nm) put_idx(a, s, m0 + tid, jj, idx);
         }
         __syncthreads();
@@ -422,8 +427,9 @@ __device__ __forceinline__ void run_coupling(const ChainArgs& a, long long m0, i
     ld_acc += ldc;  // Chain: log_det += ld   (bijectors.py:110)
 }
 
-// ShiftBounds for one event m of a tile held as xs[col][stride] (bijectors.py:183-207 / :214-238)
-template <bool INVERSE>
+// ShiftBounds for one event m of a tile held as xs[col][stride] (bijectors.py:183-207 / :214-238).  ILP: ld_acc also
+// takes minus the inverse's log|dx/dv|: log(b - a), log(xmax - xmin), or u + log(xmax - xmin) for x = a + e^u, b - e^u
+template <bool INVERSE, bool ILP = false>
 __device__ __forceinline__ void shift_bounds_row(const StepDesc& s, const float* __restrict__ wsf, int D, float* xs,
                                                  int stride, int m, float& ld_acc, int i0 = 0, int istep = 1) {
     float ldc = 0.f;
@@ -456,8 +462,10 @@ __device__ __forceinline__ void shift_bounds_row(const StepDesc& s, const float*
                 if (kind == ZF_BOUND_LOWER) x = expf(u) + a;
                 else if (kind == ZF_BOUND_UPPER) x = b - expf(u);
                 else x = u;
+                if (ILP && kind != ZF_BOUND_NONE) ldc -= u;
             }
             *px = x;
+            if (ILP) ldc -= t[7];
         }
     }
     ld_acc += ldc;
@@ -561,21 +569,29 @@ __device__ __forceinline__ void store_tile(float* y, long long m0, int nm, int D
     }
 }
 
-// log p of event m of a finished tile: sum of the latent log-pdf over its columns + the chain's log-det (flow.py:46-47)
-__device__ __forceinline__ float tile_lp(const ChainArgs& a, const float* xs, int S, int m, float ld) {
+// Sum of the latent log-pdf over the columns of event m of a tile whose column j sits at (j - rot_total) mod D: a
+// finished forward tile, or an inverse tile right after its load (the latent draw)
+__device__ __forceinline__ float tile_latent(const ChainArgs& a, const float* xs, int S, int m) {
     float lat = 0.f;
     for (int j = 0; j < a.D; ++j) lat += latent_logpdf(xs[pmod(j - a.rot_total, a.D) * S + m], a.lc);
-    return nan_to_num_lp(lat + ld);
+    return lat;
 }
 
-template <bool INVERSE>
+// log p of event m of a finished tile: sum of the latent log-pdf over its columns + the chain's log-det (flow.py:46-47)
+__device__ __forceinline__ float tile_lp(const ChainArgs& a, const float* xs, int S, int m, float ld) {
+    return nan_to_num_lp(tile_latent(a, xs, S, m) + ld);
+}
+
+template <bool INVERSE, bool ILP = false>
 __device__ __forceinline__ void run_shift_bounds(const StepDesc& s, const float* __restrict__ wsf, int D,
                                                  float* xs, float& ld_acc, int tid) {
-    if (tid < TM) shift_bounds_row<INVERSE>(s, wsf, D, xs, TM, tid, ld_acc);
+    if (tid < TM) shift_bounds_row<INVERSE, ILP>(s, wsf, D, xs, TM, tid, ld_acc);
     __syncthreads();
 }
 
-template <bool INVERSE>
+// ILP (with INVERSE): the inverse log-density mode.  The accumulator starts at the latent log-pdf of the loaded draw, every
+// spline row and ShiftBounds subtracts its inverse log-det, and the store writes nan_to_num of it to a.lp (y optional).
+template <bool INVERSE, bool ILP = false>
 __global__ void __launch_bounds__(kChainThreads, 2) chain_kernel(const __grid_constant__ ChainArgs a) {
     extern __shared__ __align__(128) float smem[];
     const int tid = threadIdx.x;
@@ -596,14 +612,18 @@ __global__ void __launch_bounds__(kChainThreads, 2) chain_kernel(const __grid_co
         __syncthreads();
 
         float ld_acc = 0.f;  // Chain: log_det = zeros(M)   (bijectors.py:107)
+        if (ILP && tid < TM) ld_acc = tile_latent(a, xs, TM, tid);
         for (int si = 0; si < a.n_steps; ++si) {
             const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
-            if (s.kind == kStepKindShiftBounds) run_shift_bounds<INVERSE>(s, wsf, D, xs, ld_acc, tid);
-            else run_coupling<INVERSE>(a, m0, nm, s, wsf, D, C, xs, cs, act0, act1, wst, ld_acc, tid);
+            if (s.kind == kStepKindShiftBounds) run_shift_bounds<INVERSE, ILP>(s, wsf, D, xs, ld_acc, tid);
+            else run_coupling<INVERSE, ILP>(a, m0, nm, s, wsf, D, C, xs, cs, act0, act1, wst, ld_acc, tid);
         }
 
         // ---- store
-        if (a.mode == kModeLogProb) {
+        if (ILP) {
+            if (a.y) store_tile<kChainThreads, TM>(a.y, m0, nm, D, 0, xs, tid);
+            if (tid < nm) a.lp[m0 + tid] = nan_to_num_lp(ld_acc);
+        } else if (a.mode == kModeLogProb) {
             if (tid < nm) a.lp[m0 + tid] = tile_lp(a, xs, TM, tid, ld_acc);
         } else {
             if (a.y) store_tile<kChainThreads, TM>(a.y, m0, nm, D, INVERSE ? 0 : a.rot_total, xs, tid);
@@ -821,8 +841,9 @@ __device__ __forceinline__ void vjp_activation(const ChainArgs& a, int layer, lo
 // ---- VJP row of the fused train kernel: theta from tensor memory -> cotangent of theta in this thread's row buffer
 // (row[0, 3 KT - 1), row[3 KT - 1] = 0).  Fast path: theta stays in registers (rqs_row_vjp_regs); rows with
 // |theta| >= kThetaFastBound, inf or NaN go through the IEEE path on the row buffer (rqs_row_backward).
-// INVERSE: the VJP of the spline inverse at y = x (no log-det), always on the row buffer (rqs_row_inverse_backward).
-template <int KT, bool INVERSE, class Release>
+// INVERSE: the VJP of the spline inverse at y = x, always on the row buffer (rqs_row_inverse_backward); with LD, gld is the
+// cotangent of its log|dx/dy|.
+template <int KT, bool INVERSE, bool LD, class Release>
 __device__ __forceinline__ float vjp_row_tmem(uint32_t dbase, const float* __restrict__ bias, float* row, float x, float gy,
                                               float gld, Release release) {
     const KnotNorm kn = make_knot_norm(KT);
@@ -837,7 +858,7 @@ __device__ __forceinline__ float vjp_row_tmem(uint32_t dbase, const float* __res
 #pragma unroll
             for (int j = 0; j < KT; ++j) row[blk * KT + j] = fmaf(w[j], umma::kF16LoUnscale, p[j]) + bias[blk * KT + j];
         }
-        const float g = rqs_row_inverse_backward<KT>(row, KT, x, gy, kn);
+        const float g = rqs_row_inverse_backward<KT, LD>(row, KT, x, gy, gld, kn);
         row[3 * KT - 1] = 0.f;
         return g;
     } else {
@@ -1091,7 +1112,7 @@ __device__ __forceinline__ void issue_unit(uint64_t* full, uint64_t* empty, uint
     if (newver) p_ar ^= 1u;
 }
 
-template <bool INVERSE, bool VJP = false>
+template <bool INVERSE, bool VJP = false, bool ILP = false>
 __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
     constexpr int NG = 2;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1130,12 +1151,13 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
         ZF_TR(trs);   // 1: inputs loaded
 
         float ld_acc = 0.f;
+        if (ILP && !VJP && half == 0) ld_acc = tile_latent(a, xs, UM, m);
         for (int si = 0; si < a.n_steps; ++si) {
             const StepDesc& s = step_at<INVERSE>(steps, a.n_steps, si);
             if (s.kind == kStepKindShiftBounds) {
                 // columns split between the groups; groups 1.. hand their log-det share over through ldx
                 float ld_sb = 0.f;
-                shift_bounds_row<INVERSE>(s, wsf, D, xs, UM, m, ld_sb, half, NG);
+                shift_bounds_row<INVERSE, ILP>(s, wsf, D, xs, UM, m, ld_sb, half, NG);
                 if (half > 0) ldx[(half - 1) * UM + m] = ld_sb;
                 epi_barrier<ET>();
                 if (half == 0) {
@@ -1271,7 +1293,8 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                 float* wrows = reinterpret_cast<float*>(cx.scratch) + ((size_t)half * UM + q * 32) * VJP_ROW;   // this warp's 32 rows
                 float* row = wrows + lane * VJP_ROW;
                 const KnotNorm kn = make_knot_norm(K);
-                const float gld = (!INVERSE && m < nm) ? a.glp[m0 + m] : 0.f;   // the inverse has no log-det
+                // the inverse's log-det cotangent: only in the log-density instance (ILP)
+                const float gld = ((!INVERSE || ILP) && m < nm) ? a.glp[m0 + m] : 0.f;
                 float gy_next = (half < d && m < nm) ? a.gy[(m0 + m) * D + pmod(half + a.gy_rot, D)] : 0.f;
                 for (int jj = half; jj < d; jj += 2) {
                     const float gyv = gy_next;
@@ -1288,8 +1311,8 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                     };
                     const float xv = xs[pmod(jj - rot, D) * UM + m];
                     float g_x;
-                    if (K == 16) g_x = vjp_row_tmem<16, INVERSE>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
-                    else g_x = vjp_row_tmem<32, INVERSE>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
+                    if (K == 16) g_x = vjp_row_tmem<16, INVERSE, ILP>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
+                    else g_x = vjp_row_tmem<32, INVERSE, ILP>(dbase, bls + jj * NL, row, xv, gyv, gld, release);
                     ZF_TR(trs);   // row cotangent done
                     if (m < nm) a.gx[(m0 + m) * D + jj] = g_x;
                     {   // this thread's row -> the event-row image: 16-byte units of 8 columns, hi and lo parts; the 32 lanes of a
@@ -1334,6 +1357,7 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
                         ldc += ld;
                     } else {
                         *px = rqs_eval_inverse(v, bin);
+                        if (ILP) ldc -= rqs_inverse_log_det(v, bin);
                     }
                 }
             }
@@ -1349,6 +1373,9 @@ __device__ __forceinline__ void umma_epilogue_role(const UCtx& cx) {
 
         // ---- store
         if (VJP) {
+        } else if (ILP) {
+            if (a.y) store_tile<ET, UM>(a.y, m0, nm, D, 0, xs, tid);
+            if (half == 0 && m < nm) a.lp[m0 + m] = nan_to_num_lp(ld_acc);
         } else if (a.mode == kModeLogProb) {
             if (half == 0 && m < nm) a.lp[m0 + m] = tile_lp(a, xs, UM, m, ld_acc);
         } else {
@@ -1365,7 +1392,7 @@ template <int N> __device__ __forceinline__ void reg_inc() { asm volatile("setma
 template <int N> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
 
 // 8 epilogue warps (two column groups) + producer + MMA issuer (320 threads).
-template <bool INVERSE, bool VJP = false>
+template <bool INVERSE, bool VJP = false, bool ILP = false>
 __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constant__ ChainArgs a) {
     constexpr int NG = 2;
     extern __shared__ __align__(128) float smem[];
@@ -1563,7 +1590,7 @@ __global__ void __launch_bounds__(320, 1) chain_umma_kernel(const __grid_constan
     const UCtx cx{a, xs, cs, xraw, hs, cst, ldx, reinterpret_cast<float4*>(scratch), bars, steps, tb, n_tiles, cl, cst_stride};
     if (warp == PW) producer_role();
     else if (warp == MW) mma_role();
-    else umma_epilogue_role<INVERSE, VJP>(cx);
+    else umma_epilogue_role<INVERSE, VJP, ILP>(cx);
 
     umma::fence_before_sync();
     __syncthreads();
@@ -1602,7 +1629,7 @@ __host__ __device__ inline size_t umma_pp_smem_floats(int D, int C, int Fmax, in
 __device__ __forceinline__ void s1_barrier() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 __device__ __forceinline__ void s2_barrier() { asm volatile("bar.sync 2, 128;" ::: "memory"); }
 
-template <bool INVERSE>
+template <bool INVERSE, bool ILP = false>
 __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __grid_constant__ ChainArgs a) {
     extern __shared__ __align__(128) float smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1866,9 +1893,9 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
             load_tile<128, UM, false>(a, bulk ? raw : a.x + m0 * D, bulk ? raw + UM * D : a.c + m0 * C, m0, nm, rot_in, xs, cs, t2);
             if (bulk) umma::mbar_arrive(&bars[PP_XEMPTY + rb]);
             s2_barrier();
-            float ld0 = 0.f;
+            float ld0 = ILP ? tile_latent(a, xs, UM, m) : 0.f;
             for (int si = 0; si < fc; ++si)   // only non-coupling kind
-                shift_bounds_row<INVERSE>(step_at<INVERSE>(steps, a.n_steps, si), wsf, D, xs, UM, m, ld0);
+                shift_bounds_row<INVERSE, ILP>(step_at<INVERSE>(steps, a.n_steps, si), wsf, D, xs, UM, m, ld0);
             lda[m] = ld0;
             signal_ready(k);   // the tile state is complete for the first coupling
         };
@@ -1887,7 +1914,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                     const int nm = (int)min((long long)UM, a.M - m0);
                     if (s.kind == kStepKindShiftBounds) {
                         float ld_sb = 0.f;
-                        shift_bounds_row<INVERSE>(s, wsf, D, xs, UM, m, ld_sb);
+                        shift_bounds_row<INVERSE, ILP>(s, wsf, D, xs, UM, m, ld_sb);
                         lda[m] += ld_sb;
                     } else {
                         const int K = s.K, rot = s.rot;
@@ -1918,6 +1945,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                             lda[m] += ld;
                         } else {
                             *px = rqs_eval_inverse(v, bin);
+                            if (ILP) lda[m] -= rqs_inverse_log_det(v, bin);
                         }
                         ++n2;
                     }
@@ -1934,6 +1962,7 @@ __global__ void __launch_bounds__(PP_THREADS, 1) chain_umma_pp_kernel(const __gr
                         } else {
                             s2_barrier();
                             if (a.y) store_tile<128, UM>(a.y, m0, nm, D, INVERSE ? 0 : a.rot_total, xs, t2);
+                            if (ILP && m < nm) a.lp[m0 + m] = nan_to_num_lp(lda[m]);
                             if (!INVERSE && a.log_det && m < nm)
                                 a.log_det[m0 + m] = a.acc_log_det ? a.log_det[m0 + m] + lda[m] : lda[m];
                             s2_barrier();
@@ -2194,7 +2223,7 @@ static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int l
             ZF_REQUIRE(latent_kind >= 0 && latent_kind <= 3, "unknown latent kind %d", latent_kind);
             ZF_REQUIRE(latent_kind != ZF_LATENT_BETA || peakness >= 1.f, "peakness must be at least 1 (distributions.py:96-97)");
         }
-        if (mode == kModeLogProb) {
+        if (mode == kModeLogProb || mode == kModeInvLogProb) {
             ZF_REQUIRE(lp != nullptr, "log_prob output is NULL");
             ZF_REQUIRE(latent_kind >= 0 && latent_kind <= 3, "unknown latent kind %d", latent_kind);
             ZF_REQUIRE(latent_kind != ZF_LATENT_BETA || peakness >= 1.f, "peakness must be at least 1 (distributions.py:96-97)");
@@ -2250,20 +2279,23 @@ static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int l
         ZF_CUDA_CHECK(cudaGetLastError());
         return ZF_OK;
     };
-    const bool inv = mode == kModeInverse;
+    const bool inv = mode == kModeInverse, ilp = mode == kModeInvLogProb;
     const long long utiles = (M + UM - 1) / UM;
     switch (k.kernel) {
         case ChainKernel::kUmmaPP: {   // two tiles in flight per CTA
             const long long blocks = std::min<long long>((utiles + 1) / 2, di.sm_count);
+            if (ilp) return launch(chain_umma_pp_kernel<true, true>, blocks, PP_THREADS);
             return inv ? launch(chain_umma_pp_kernel<true>, blocks, PP_THREADS) : launch(chain_umma_pp_kernel<false>, blocks, PP_THREADS);
         }
         case ChainKernel::kUmma: {
             const long long blocks = std::min<long long>(utiles, di.sm_count);
+            if (ilp) return launch(chain_umma_kernel<true, false, true>, blocks, 320);
             return inv ? launch(chain_umma_kernel<true>, blocks, 320) : launch(chain_umma_kernel<false>, blocks, 320);
         }
         default: {   // kFfma (an eval pass is never kNone or kUmmaVjp)
             const int bps = (2 * (k.smem + 1024) <= (size_t)di.max_smem_optin) ? 2 : 1;
             const long long blocks = std::min<long long>((M + TM - 1) / TM, (long long)di.sm_count * bps);
+            if (ilp) return launch(chain_kernel<true, true>, blocks, kChainThreads);
             return inv ? launch(chain_kernel<true>, blocks, kChainThreads) : launch(chain_kernel<false>, blocks, kChainThreads);
         }
     }
@@ -2271,7 +2303,8 @@ static int run_chain(cudaStream_t stream, const zf_chain* chain, int mode, int l
 
 // ---- fused conditioner recompute + spline VJP of ONE coupling (tensor-core path of zf_coupling_backward) ---------
 // The coupling is planned and packed as a chain of one op; the kernel is chain_umma_kernel<false, true>, or
-// chain_umma_kernel<true, true> for the VJP of the coupling's inverse (x_in is then the inverse's input, glp unused).
+// chain_umma_kernel<true, true> for the VJP of the coupling's inverse (x_in is then the inverse's input), or
+// chain_umma_kernel<true, true, true> when glp, the cotangent of the inverse's log-det, is given.
 static int vjp_plan(const zf_coupling* cp, int D, int C, Plan& plan, zf_op& op, zf_chain& chain) {
     op = zf_op{};
     op.kind = ZF_OP_COUPLING;
@@ -2338,7 +2371,7 @@ int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, c
     ChainLaunch k;
     if (int rc = choose_chain_kernel(plan, di, true, impl_switch().chain, &k)) return rc;
     ZF_REQUIRE(k.kernel == ChainKernel::kUmmaVjp, "coupling_vjp: the coupling does not take the fused kernel (coupling_vjp_ws_floats is 0)");
-    auto kern = inverse ? chain_umma_kernel<true, true> : chain_umma_kernel<false, true>;
+    auto kern = !inverse ? chain_umma_kernel<false, true> : glp ? chain_umma_kernel<true, true, true> : chain_umma_kernel<true, true>;
     if (int rc = smem_optin((const void*)kern, k.smem)) return rc;
     const long long tiles = (M + UM - 1) / UM;
     if (tiles == 0) return ZF_OK;
@@ -2388,6 +2421,14 @@ extern "C" int zf_flow_sample(void* stream, const zf_chain* chain, int32_t laten
     ZF_REQUIRE(x != nullptr || M == 0, "output tensor is NULL");
     return zf::run_chain((cudaStream_t)stream, chain, zf::kModeInverse, latent_kind, peakness, nullptr, c, (long long)M, x,
                          nullptr, nullptr, workspace, workspace_bytes, 0, 1, (unsigned long long)seed);
+}
+
+extern "C" int zf_flow_sample_log_prob(void* stream, const zf_chain* chain, int32_t latent_kind, float peakness, uint64_t seed,
+                                       const float* z, const float* c, int64_t M, float* x, float* log_prob, void* workspace,
+                                       size_t workspace_bytes) {
+    ZF_REQUIRE(log_prob != nullptr || M == 0, "sample_log_prob: log_prob is NULL");
+    return zf::run_chain((cudaStream_t)stream, chain, zf::kModeInvLogProb, latent_kind, peakness, z, c, (long long)M, x,
+                         nullptr, log_prob, workspace, workspace_bytes, 0, z ? 0 : 1, (unsigned long long)seed);
 }
 
 extern "C" int zf_flow_log_prob(void* stream, const zf_chain* chain, int32_t latent_kind, float peakness,

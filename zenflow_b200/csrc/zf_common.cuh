@@ -83,7 +83,8 @@ int coupling_vjp_run(cudaStream_t stream, const zf_coupling* cp, int D, int C, c
 
 // zf_coupling_backward (zf_train.cu) for either direction.  inverse = false: the VJP of the coupling's forward, as the
 // public entry.  inverse = true: the VJP of NeuralSplineCoupling.inverse (bijectors.py:367-371) with x_in its input (the
-// forward's output), gy the cotangent of its output read at column (j + gy_rot) % D, glp unused (no log-det); gx is the
+// forward's output), gy the cotangent of its output read at column (j + gy_rot) % D, glp the cotangent of the inverse's
+// log|dx/dy| per event or NULL (Flow.sample_and_log_prob's VJP passes one, Flow.inverse's does not); gx is the
 // cotangent of x_in.  The BatchNorm running statistics are constants either way (the inverse is always eval-mode).
 int coupling_backward(cudaStream_t st, const zf_coupling* cp, const zf_coupling_grads* gr, int D, int C, const float* x_in,
                       const float* c, const float* gy, int gy_rot, const float* glp, long long M, float* gx, float* gh0,
@@ -125,9 +126,16 @@ int shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, con
                           const float* glp, long long M, float* gx);
 // VJP of ShiftBounds.inverse (bijectors.py:210-240) with the running sb->xmin / sb->xmax: gz (M, D) = d/dz for the
 // cotangent gx of its output x.  dx/dz is b - a (both bounds), xmax - xmin (running statistics), exp(t) (xmax - xmin)
-// (lower bound) or -exp(t) (xmax - xmin) (upper bound), t = z xmax + (1 - z) xmin.
-int shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* z, const float* gx, long long M,
-                                  float* gz);
+// (lower bound) or -exp(t) (xmax - xmin) (upper bound), t = z xmax + (1 - z) xmin.  glp (or NULL) is the cotangent of
+// the inverse's log-det (log(b - a), log(xmax - xmin), + t on one-sided columns).
+int shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* z, const float* gx,
+                                  const float* glp, long long M, float* gz);
+// Flow.sample_and_log_prob's VJP (zf_train.cu).  glp = the cotangent of the chain's inverse log-det, -lp_cotangent, or 0 on
+// rows whose lp (the nan_to_num'ed output) was not finite.  latent_score_acc: gz -= glp * d log p_latent / dz, the latent
+// term of lp = sum_j log p(z_j) - log|det dx/dz| (rows with glp = 0 are left alone: the score may be infinite there).
+int inverse_lp_cotangent(cudaStream_t st, const float* lp, const float* lp_cotangent, long long M, float* glp);
+int latent_score_acc(cudaStream_t st, int latent_kind, float peakness, const float* z, const float* glp, long long M, int D,
+                     float* gz);
 
 // ---- PTX wrappers ----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

@@ -23,6 +23,10 @@
 //   backward  per group, first to last (the cotangent travels from x toward z): the ShiftBounds' inverse VJP, or the
 //             coupling's (conditioner recompute + spline-inverse VJP + Dense VJPs) and the diagonal BatchNorm VJP;
 //             the cotangent of u_g reaches the next group's output through its Rolls by index arithmetic.
+// zf_flow_sample_log_prob_vjp: the joint VJP of (x, lp) of zf_flow_sample_log_prob, the same inverse mode with a log-density:
+// lp = sum_j log p(z_j) - sum of the inverse log-dets, so every group's log-det takes the per-event cotangent -g_lp (0 on
+// rows whose lp was not finite; the whole chain's lp is recomputed by one fused pass to find them), and gz also takes
+// g_lp d log p / dz.
 #include "zf_common.cuh"
 
 #include <algorithm>
@@ -59,9 +63,11 @@ static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // kernel keeps; it also accepts a chain with no coupling, whose only derivative is d/dx through the ShiftBounds.
 // Inverse mode uses the states for u_g, the input of group g's own inverse, and adds one (M, D) buffer for the outputs
 // that are not states (x_g when group g-1 has Rolls, and x when the caller does not ask for it).
-static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, StepMode mode, StepPlan& p) {
+// with_lp (inverse mode): the chain workspace also holds the whole chain's, for the fused lp pass
+static int build_step_plan(const zf_chain* chain, long long M, long long micro_batch, StepMode mode, StepPlan& p,
+                           bool with_lp = false) {
     const bool train = mode == kStepTrain;
-    const char* who = train ? "value_and_grad" : mode == kStepEval ? "log_prob_vjp" : "chain_inverse_vjp";
+    const char* who = train ? "value_and_grad" : mode == kStepEval ? "log_prob_vjp" : with_lp ? "sample_log_prob_vjp" : "chain_inverse_vjp";
     ZF_REQUIRE(chain && chain->n_ops >= 1 && chain->ops, "%s: empty chain", who);
     const int D = chain->dim, C = chain->cdim;
     ZF_REQUIRE(D >= (train ? 2 : 1) && D <= ZF_MAX_DIM, "%s: dim must be in [%d, %d]", who, train ? 2 : 1, ZF_MAX_DIM);
@@ -108,6 +114,11 @@ static int build_step_plan(const zf_chain* chain, long long M, long long micro_b
         if (g.kind == ZF_OP_COUPLING)
             p.bwd_bytes = std::max(p.bwd_bytes, zf_coupling_backward_workspace_bytes(g.ops[0].coupling, D, C, mb));
     }
+    if (with_lp) {
+        const size_t cb = zf_chain_workspace_bytes(chain, M);
+        if (cb == 0) return ZF_ERR_INVALID;
+        p.chain_bytes = std::max(p.chain_bytes, cb);
+    }
     p.off_chain = take(p.chain_bytes);
     p.off_bwd = take(p.bwd_bytes);
     if (mode == kStepEval) p.off_lp_sum = take(sizeof(double));
@@ -133,9 +144,10 @@ static int aux_events(AuxEvents** out) {
     return ZF_OK;
 }
 
-// The arguments of the three entry points.  Train-only fields (global_count, lp_sum, the communicators and buckets) are
+// The arguments of the entry points.  Train-only fields (global_count, lp_sum, the communicators and buckets) are
 // unused in eval mode; gx (d/dx) is eval-only.  Inverse mode reads x as z (NULL: sample with latent_kind, peakness, seed),
-// x_ct as the cotangent of its output, writes x_out (optional) and gz (optional), and uses none of the loss fields.
+// x_ct as the cotangent of its output (NULL: zero), writes x_out (optional) and gz (optional); with a log-density it reads
+// lp_cotangent (or NULL) and writes lp (optional).
 struct StepCall {
     StepMode mode;
     cudaStream_t st, aux;
@@ -190,6 +202,18 @@ static int run_step(StepPlan& p, const StepCall& a) {
 
     if (!inv) ZF_CUDA_CHECK(cudaMemsetAsync(ld, 0, (size_t)M * 4, st));
     if (a.gc && C) ZF_CUDA_CHECK(cudaMemsetAsync(a.gc, 0, (size_t)M * C * 4, st));
+    // inverse mode with a log-density: lp of the whole chain (fused pass), and the cotangent of every group's log-det
+    const float* gld_inv = nullptr;
+    if (inv && (a.lp || a.lp_cotangent)) {
+        float* lp = a.lp ? a.lp : ld;
+        if (int rc = zf_flow_sample_log_prob(st, a.chain, a.latent_kind, a.peakness, a.seed, x, c, M, nullptr, lp, chain_ws,
+                                             p.chain_bytes))
+            return rc;
+        if (a.lp_cotangent) {
+            if (int rc = inverse_lp_cotangent(st, lp, a.lp_cotangent, M, glp)) return rc;
+            gld_inv = glp;
+        }
+    }
 
     // ---- forward, one bijector group at a time (in train mode the batch statistics couple the events)
     std::vector<zf_coupling> batch_cp(G);    // couplings reading the BATCH statistics (train mode)
@@ -265,6 +289,10 @@ static int run_step(StepPlan& p, const StepCall& a) {
     if (overlap)
         if (int rc = aux_events(&ev)) return rc;
     const float* g_in = a.x_ct;   // inverse mode: the cotangent of the current group's output, read at (j + g_rot) % D
+    if (inv && !g_in) {           // no cotangent of x: zeros, in the buffer the first group does not write
+        ZF_CUDA_CHECK(cudaMemsetAsync(gx, 0, (size_t)M * D * 4, st));
+        g_in = gx;
+    }
     int g_rot = 0;
     for (size_t k = 0; k < G; ++k) {
         const size_t gi = inv ? k : G - 1 - k;
@@ -274,12 +302,12 @@ static int run_step(StepPlan& p, const StepCall& a) {
             const bool last = gi + 1 == G;
             float* dst = (last && a.gz && pmod_rot(g.rot, D) == 0) ? a.gz : gy;
             if (g.kind == ZF_OP_SHIFT_BOUNDS) {
-                if (int rc = shift_bounds_inverse_backward(st, g.ops[0].shift_bounds, D, u_in[gi], g_in, M, dst)) return rc;
+                if (int rc = shift_bounds_inverse_backward(st, g.ops[0].shift_bounds, D, u_in[gi], g_in, gld_inv, M, dst)) return rc;
             } else {
                 const zf_coupling* cp = g.ops[0].coupling;
                 const zf_coupling_grads* gr = a.grads ? &a.grads[g.coupling_index] : nullptr;
                 double* bsums = gr ? reinterpret_cast<double*>(stats(gi) + align_up((size_t)2 * F * 4, 8)) + 2 * F : nullptr;
-                if (int rc = coupling_backward(st, cp, gr, D, C, u_in[gi], c, g_in, g_rot, nullptr, M, dst, gh0, bsums, bwd_ws,
+                if (int rc = coupling_backward(st, cp, gr, D, C, u_in[gi], c, g_in, g_rot, gld_inv, M, dst, gh0, bsums, bwd_ws,
                                                p.bwd_bytes, mb, true))
                     return rc;
                 if (gr)
@@ -291,6 +319,8 @@ static int run_step(StepPlan& p, const StepCall& a) {
                 zf_chain rolls{D, 0, (int32_t)g.ops.size() - 1, g.ops.data() + 1};
                 if (int rc = zf_chain_forward(st, &rolls, dst, nullptr, M, a.gz, nullptr, chain_ws, p.chain_bytes)) return rc;
             }
+            if (last && a.gz && gld_inv)   // the latent term of lp
+                if (int rc = latent_score_acc(st, a.latent_kind, a.peakness, x, gld_inv, M, D, a.gz)) return rc;
             g_in = dst;
             g_rot = pmod_rot(-g.rot, D);
             std::swap(gy, gx);
@@ -415,6 +445,33 @@ extern "C" int zf_chain_inverse_vjp(void* stream, const zf_chain* chain, const z
     if (workspace_bytes < p.total)
         return fail(ZF_ERR_WORKSPACE, "chain_inverse_vjp: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
     StepCall a{kStepInverse, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, z, c, M, 1.0, nullptr, nullptr,
+               nullptr, nullptr, gc, nullptr, nullptr, nullptr, nullptr, static_cast<char*>(workspace), micro_batch,
+               x_cotangent, x, gz, (unsigned long long)seed};
+    return run_step(p, a);
+}
+
+extern "C" size_t zf_flow_sample_log_prob_vjp_workspace_bytes(const zf_chain* chain, int64_t M, int64_t micro_batch) {
+    StepPlan p;
+    if (build_step_plan(chain, M, micro_batch, kStepInverse, p, true) != ZF_OK) return 0;
+    return p.total;
+}
+
+extern "C" int zf_flow_sample_log_prob_vjp(void* stream, const zf_chain* chain, const zf_coupling_grads* grads, const float* z,
+                                           int32_t latent_kind, float peakness, uint64_t seed, const float* c, int64_t M,
+                                           const float* x_cotangent, const float* lp_cotangent, float* x, float* lp, float* gz,
+                                           float* gc, void* workspace, size_t workspace_bytes, int64_t micro_batch) {
+    StepPlan p;
+    if (int rc = build_step_plan(chain, M, micro_batch, kStepInverse, p, true)) return rc;
+    ZF_REQUIRE(workspace, "sample_log_prob_vjp: null argument");
+    ZF_REQUIRE(x_cotangent || lp_cotangent, "sample_log_prob_vjp: x_cotangent and lp_cotangent are both NULL");
+    ZF_REQUIRE(chain->cdim == 0 || c, "sample_log_prob_vjp: chain has cdim=%d but c is NULL", chain->cdim);
+    ZF_REQUIRE(z || !gz, "sample_log_prob_vjp: gz must be NULL when sampling (z is NULL): the latent draw is a constant");
+    ZF_REQUIRE(latent_kind >= 0 && latent_kind <= 3, "sample_log_prob_vjp: unknown latent kind %d", latent_kind);
+    ZF_REQUIRE(latent_kind != ZF_LATENT_BETA || peakness >= 1.f, "sample_log_prob_vjp: peakness must be at least 1");
+    ZF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "sample_log_prob_vjp: workspace must be 256-byte aligned");
+    if (workspace_bytes < p.total)
+        return fail(ZF_ERR_WORKSPACE, "sample_log_prob_vjp: workspace too small: need %zu bytes, got %zu", p.total, workspace_bytes);
+    StepCall a{kStepInverse, (cudaStream_t)stream, nullptr, chain, grads, latent_kind, peakness, z, c, M, 1.0, lp_cotangent, lp,
                nullptr, nullptr, gc, nullptr, nullptr, nullptr, nullptr, static_cast<char*>(workspace), micro_batch,
                x_cotangent, x, gz, (unsigned long long)seed};
     return run_step(p, a);

@@ -347,10 +347,13 @@ __global__ void __launch_bounds__(256) sb_bwd_kernel(const __grid_constant__ SbV
 }
 
 // VJP of ShiftBounds.inverse (forward: shift_bounds_row<true> in zf_chain.cu, bijectors.py:210-240); cols.mul_both holds
-// (float)(b - a) of the ZF_BOUND_BOTH columns here
+// (float)(b - a) of the ZF_BOUND_BOTH columns here.  LD: glp is the cotangent of the inverse's log-det, whose one-sided
+// columns' term u = v xmax + (1 - v) xmin adds glp (xmax - xmin); the other terms are constants.
+template <bool LD>
 __global__ void __launch_bounds__(256) sb_inv_bwd_kernel(const __grid_constant__ SbVjpCols cols, const float* __restrict__ xmin,
                                                          const float* __restrict__ xmax, const float* __restrict__ z,
-                                                         const float* __restrict__ gx, long long M, int D, float* __restrict__ gz) {
+                                                         const float* __restrict__ gx, long long M, int D, float* __restrict__ gz,
+                                                         const float* __restrict__ glp) {
     const long long n = M * D;
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
         const int i = (int)(e % D);
@@ -366,6 +369,10 @@ __global__ void __launch_bounds__(256) sb_inv_bwd_kernel(const __grid_constant__
                 const float v = z[e];
                 const float t = __fadd_rn(__fmul_rn(v, hi), __fmul_rn(__fsub_rn(1.f, v), lo));   // as the chain's inverse
                 r *= (kind == ZF_BOUND_LOWER) ? expf(t) : -expf(t);
+                if (LD) {
+                    const float gl = glp[e / D];
+                    if (gl != 0.f) r += gl * span;
+                }
             }
         }
         gz[e] = r;
@@ -375,6 +382,14 @@ __global__ void __launch_bounds__(256) sb_inv_bwd_kernel(const __grid_constant__
 // ---------------------------------------------------------------------------------------------
 // loss and latent gradient
 // ---------------------------------------------------------------------------------------------
+// d log p / dz of one latent element (0 outside the support, where the log-pdf is the constant -inf)
+__device__ __forceinline__ float latent_score(float v, const LatentConst& lc) {
+    if (lc.kind == kLatentBeta) return (v > 1.f || v < 0.f) ? 0.f : (lc.p1 / v - lc.p1 / (1.f - v));
+    if (lc.kind == kLatentNormal) return -(v - 0.5f) / 0.01f;
+    if (lc.kind == kLatentTruncNormal) return (v > 1.f || v < 0.f) ? 0.f : -(v - 0.5f) / 0.01f;
+    return 0.f;
+}
+
 __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const float* __restrict__ z,
                                                         const float* __restrict__ log_det, long long M, int D,
                                                         float wgt, const float* __restrict__ cot,
@@ -393,11 +408,7 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
         glp[m] = w;
         local += (double)lp;
         for (int j = 0; j < D; ++j) {
-            const float v = z[m * D + j];
-            float dl = 0.f;
-            if (lc.kind == kLatentBeta) dl = (v > 1.f || v < 0.f) ? 0.f : (lc.p1 / v - lc.p1 / (1.f - v));
-            else if (lc.kind == kLatentNormal) dl = -(v - 0.5f) / 0.01f;
-            else if (lc.kind == kLatentTruncNormal) dl = (v > 1.f || v < 0.f) ? 0.f : -(v - 0.5f) / 0.01f;
+            const float dl = latent_score(z[m * D + j], lc);
             gz[m * D + j] = (zero_dead && w == 0.f) ? 0.f : w * dl;   // 0 * inf at a latent boundary
         }
     }
@@ -412,8 +423,8 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(LatentConst lc, const fl
 
 // ---------------------------------------------------------------------------------------------
 // spline VJP: theta row -> d(theta) row in place; d/dx of the transformed columns; pass-through
-// of the conditioning columns' cotangent.  INVERSE: the VJP of the spline inverse, x_in is the inverse's input y and
-// glp is not read.
+// of the conditioning columns' cotangent.  INVERSE: the VJP of the spline inverse, x_in is the inverse's input y, and glp
+// (the cotangent of the inverse's log|dx/dy|) is read only by the LD instances.
 // ---------------------------------------------------------------------------------------------
 struct SplineBwdArgs {
     float* theta;          // (Mb, d, P) in: raw params, out: their cotangent
@@ -438,9 +449,11 @@ template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 
 // theta tiles stream HBM -> smem ring (bulk copies) -> in-place VJP, one thread per (sample, dim) row ->
-// HBM (bulk store); same pipeline shape as rqs_stage_kernel.
-template <int KT, bool INVERSE>
-__global__ void __launch_bounds__(256) spline_bwd_kernel(const __grid_constant__ SplineBwdArgs a) {
+// HBM (bulk store); same pipeline shape as rqs_stage_kernel.  The LD instances (the inverse's VJP with its log-det) run one
+// block per SM: held to two blocks' 128 registers, the K = 32 instance spills; the others leave the register choice to
+// ptxas as before (a minimum of 0 blocks is no minimum).
+template <int KT, bool INVERSE, bool LD = false>
+__global__ void __launch_bounds__(256, LD ? 1 : 0) spline_bwd_kernel(const __grid_constant__ SplineBwdArgs a) {
     extern __shared__ __align__(128) float sm[];
     const int tid = threadIdx.x;
     const int K = KT > 0 ? KT : a.K;
@@ -492,7 +505,7 @@ __global__ void __launch_bounds__(256) spline_bwd_kernel(const __grid_constant__
             const long long m = a.m0 + s0 + sidx;
             const float x = a.x_in[m * D + jj];
             const float gy = a.gy[m * D + (jj + a.rot) % D];
-            a.gx[m * D + jj] = INVERSE ? rqs_row_inverse_backward<KT>(buf + (size_t)r * P, K, x, gy, kn)
+            a.gx[m * D + jj] = INVERSE ? rqs_row_inverse_backward<KT, LD>(buf + (size_t)r * P, K, x, gy, LD ? a.glp[m] : 0.f, kn)
                                        : rqs_row_backward<KT>(buf + (size_t)r * P, K, x, gy, a.glp[m], kn);
         }
         // conditioning columns pass through unchanged: d y[:, j] / d x[:, j] = 1   (bijectors.py:364)
@@ -697,6 +710,42 @@ extern "C" int zf_bn_finalize(void* stream, const double* sums, double count, in
     return ZF_OK;
 }
 
+// Flow.sample_and_log_prob's VJP: see zf_common.cuh
+__global__ void __launch_bounds__(256) inv_lp_ct_kernel(const float* __restrict__ lp, const float* __restrict__ cot, long long M,
+                                                        float* __restrict__ glp) {
+    for (long long m = blockIdx.x * (long long)blockDim.x + threadIdx.x; m < M; m += (long long)gridDim.x * blockDim.x)
+        glp[m] = fabsf(lp[m]) < FLT_MAX ? -cot[m] : 0.f;   // nan_to_num maps NaN and +-inf to +-FLT_MAX
+}
+
+__global__ void __launch_bounds__(256) latent_score_kernel(LatentConst lc, const float* __restrict__ z, const float* __restrict__ glp,
+                                                           long long M, int D, float* __restrict__ gz) {
+    const long long n = M * D;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+        const float w = glp[e / D];
+        if (w != 0.f) gz[e] -= w * latent_score(z[e], lc);
+    }
+}
+
+int zf::inverse_lp_cotangent(cudaStream_t st, const float* lp, const float* lp_cotangent, long long M, float* glp) {
+    ZF_REQUIRE(lp && lp_cotangent && glp && M >= 1, "inverse_lp_cotangent: bad argument");
+    inv_lp_ct_kernel<<<grid_for(M, 256, 148 * 8), 256, 0, st>>>(lp, lp_cotangent, M, glp);
+    count_launch();
+    ZF_CUDA_CHECK(cudaGetLastError());
+    return ZF_OK;
+}
+
+int zf::latent_score_acc(cudaStream_t st, int latent_kind, float peakness, const float* z, const float* glp, long long M, int D,
+                         float* gz) {
+    ZF_REQUIRE(z && glp && gz && M >= 1 && D >= 1, "latent_score_acc: bad argument");
+    LatentConst lc{};
+    lc.kind = latent_kind;
+    lc.p1 = (float)((double)peakness - 1.0);
+    latent_score_kernel<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(lc, z, glp, M, D, gz);
+    count_launch();
+    ZF_CUDA_CHECK(cudaGetLastError());
+    return ZF_OK;
+}
+
 int zf::flow_loss_grad(cudaStream_t st, int latent_kind, float peakness, const float* z, const float* log_det, long long M,
                        int D, double global_count, const float* lp_cotangent, float* lp, float* gz, float* glp,
                        double* lp_sum, int zero_dead) {
@@ -890,11 +939,14 @@ int zf::coupling_backward(cudaStream_t st, const zf_coupling* cp, const zf_coupl
     const size_t tile_bytes = (size_t)TS * d * P * 4;
     int sp_stages = (int)std::min<size_t>(3, ((size_t)di.max_smem_optin - 256) / tile_bytes);
     int sp_bps = 1;
-    if (2 * (2 * tile_bytes + 256) + 2048 <= (size_t)di.max_smem_optin) { sp_stages = 2; sp_bps = 2; }
+    const bool sp_ld = inverse && glp;   // spline_bwd_kernel<K, true, true>: one block per SM (its launch bounds)
+    if (!sp_ld && 2 * (2 * tile_bytes + 256) + 2048 <= (size_t)di.max_smem_optin) { sp_stages = 2; sp_bps = 2; }
     if (sp_stages < 1) return fail(ZF_ERR_UNSUPPORTED, "coupling_backward: spline tile does not fit shared memory");
     const size_t sp_smem = (size_t)sp_stages * tile_bytes + 64;
-    auto sp_kernel = inverse ? ((K == 16) ? spline_bwd_kernel<16, true> : (K == 32) ? spline_bwd_kernel<32, true> : spline_bwd_kernel<0, true>)
-                             : ((K == 16) ? spline_bwd_kernel<16, false> : (K == 32) ? spline_bwd_kernel<32, false> : spline_bwd_kernel<0, false>);
+    auto sp_kernel = !inverse ? ((K == 16) ? spline_bwd_kernel<16, false> : (K == 32) ? spline_bwd_kernel<32, false> : spline_bwd_kernel<0, false>)
+                     : !sp_ld ? ((K == 16) ? spline_bwd_kernel<16, true> : (K == 32) ? spline_bwd_kernel<32, true> : spline_bwd_kernel<0, true>)
+                              : ((K == 16) ? spline_bwd_kernel<16, true, true> : (K == 32) ? spline_bwd_kernel<32, true, true>
+                                                                                           : spline_bwd_kernel<0, true, true>);
     if (int rc = smem_optin((const void*)sp_kernel, sp_smem)) return rc;
 
     float* ws = static_cast<float*>(workspace);
@@ -1036,7 +1088,7 @@ int zf::shift_bounds_backward(cudaStream_t st, const zf_shift_bounds* sb, int D,
 }
 
 int zf::shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb, int D, const float* z, const float* gx,
-                                      long long M, float* gz) {
+                                      const float* glp, long long M, float* gz) {
     ZF_REQUIRE(sb && z && gx && gz && M >= 1 && D >= 1 && D <= ZF_MAX_DIM, "shift_bounds_inverse_backward: bad argument");
     SbVjpCols cols{};
     fill_cols(sb, D, cols.c);
@@ -1046,7 +1098,8 @@ int zf::shift_bounds_inverse_backward(cudaStream_t st, const zf_shift_bounds* sb
         else running = true;
     }
     ZF_REQUIRE(!running || (sb->xmin && sb->xmax), "shift_bounds_inverse_backward: xmin / xmax are NULL");
-    sb_inv_bwd_kernel<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(cols, sb->xmin, sb->xmax, z, gx, M, D, gz);
+    auto kern = glp ? sb_inv_bwd_kernel<true> : sb_inv_bwd_kernel<false>;
+    kern<<<grid_for(M * D, 256 * 8, 148 * 16), 256, 0, st>>>(cols, sb->xmin, sb->xmax, z, gx, M, D, gz, glp);
     count_launch();
     ZF_CUDA_CHECK(cudaGetLastError());
     return ZF_OK;

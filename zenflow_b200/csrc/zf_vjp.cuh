@@ -149,9 +149,13 @@ __device__ __forceinline__ float rqs_row_backward(float* row, int K_rt, float x,
 // Adjoints of the analytic inverse (utils.py:191-201, rqs_eval_inverse): y -> x inside bin [yk, yk + h) x [xk, xk + w)
 // with knot derivatives d0, d1; gx is the cotangent of x.  The formula is differentiated as written (a quadratic root,
 // no EPS, no clip), which is what jax.grad of the reference's inverse gives; it is not 1 / (dy/dx) of the forward.
-__device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, float yk, float h, float xk, float w, float d0,
-                                                            float d1, float& g_y, float& g_yk, float& g_h, float& g_xk, float& g_w,
-                                                            float& g_d0, float& g_d1) {
+// LD: gld is the cotangent of the inverse's log|dx/dy| = 2 log(den) - 2 log(s) - log(num2) at the root
+// (rqs_inverse_log_det), its terms formed only where gld != 0 (no 0 * inf); without LD gld is not read and the code is
+// that of the inverse's VJP alone.
+template <bool LD = false>
+__device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, float gld, float yk, float h, float xk, float w,
+                                                            float d0, float d1, float& g_y, float& g_yk, float& g_h, float& g_xk,
+                                                            float& g_w, float& g_d0, float& g_d1) {
     const float s = h / w;
     const float dy = y - yk;
     const float beta = d1 + d0 - 2.0f * s;
@@ -164,7 +168,22 @@ __device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, f
     // x = z w + xk,  z = 2c / Dq,  Dq = -bq - sqrt(bq^2 - 4ac)
     g_xk = gx;
     g_w = gx * z;
-    const float g_z = gx * w;
+    float g_z = gx * w;
+    // log-det: den = s + beta z (1 - z), num2 = d1 z^2 + 2 s z (1 - z) + d0 (1 - z)^2, differentiated at fixed z here and
+    // through the root (g_z) below
+    float gl_s = 0.f, gl_d0 = 0.f, gl_d1 = 0.f;
+    const bool with_ld = LD && gld != 0.f;
+    if (with_ld) {
+        const float az = 1.0f - z, zz = z * az;
+        const float den = s + beta * zz;
+        const float num2 = z * (d1 * z + 2.0f * s * az) + d0 * (az * az);
+        const float g_den = 2.0f * gld / den, g_num2 = -gld / num2;
+        const float gl_beta = g_den * zz;
+        g_z += g_den * beta * (1.0f - 2.0f * z) + g_num2 * 2.0f * (d1 * z + s * (1.0f - 2.0f * z) - d0 * az);
+        gl_s = g_den - 2.0f * gld / s + g_num2 * 2.0f * zz - 2.0f * gl_beta;
+        gl_d0 = g_num2 * az * az + gl_beta;
+        gl_d1 = g_num2 * z * z + gl_beta;
+    }
     float g_c = g_z * 2.0f / Dq;
     const float g_Dq = -g_z * z / Dq;
     const float g_disc = -g_Dq * 0.5f / sq;
@@ -182,6 +201,11 @@ __device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, f
     g_d1 = g_beta;
     g_d0 += g_beta;
     g_s -= 2.0f * g_beta;
+    if (with_ld) {
+        g_s += gl_s;
+        g_d0 += gl_d0;
+        g_d1 += gl_d1;
+    }
     // dy = y - yk;  s = h / w
     g_y = g_dy;
     g_yk = -g_dy;
@@ -190,11 +214,12 @@ __device__ __forceinline__ void rqs_scalar_inverse_adjoints(float y, float gx, f
 }
 
 // The VJP of normalize_spline_params + rational_quadratic_spline_inverse (utils.py:144-202) on a row: raw theta (3K-1)
-// in shared memory, overwritten by its cotangent; gx is the cotangent of x.  Returns d/dy.  The bin is searched in the
-// heights, as the eval inverse searches it.  Conventions as rqs_row_backward: identity branch (y outside [0, 1)):
-// d/dy = gx and no parameter gradient; the reference's NaN corner (past the last knot, NaN input): zero gradients.
-template <int KT>
-__device__ __forceinline__ float rqs_row_inverse_backward(float* row, int K_rt, float y, float gx, const KnotNorm& kn) {
+// in shared memory, overwritten by its cotangent; gx is the cotangent of x, gld (read only with LD) that of the row's
+// log|dx/dy|.  Returns d/dy.  The bin is searched in the heights, as the eval inverse searches it.  Conventions as
+// rqs_row_backward: identity branch (y outside [0, 1)): d/dy = gx and no parameter gradient (the log-det is 0 there); the
+// reference's NaN corner (past the last knot, NaN input): zero gradients.
+template <int KT, bool LD = false>
+__device__ __forceinline__ float rqs_row_inverse_backward(float* row, int K_rt, float y, float gx, float gld, const KnotNorm& kn) {
     const int K = KT > 0 ? KT : K_rt;
     RqsBin b;
     rqs_locate<KT>(row, K, false, y, kn, b);
@@ -207,7 +232,7 @@ __device__ __forceinline__ float rqs_row_inverse_backward(float* row, int K_rt, 
     }
     const float yk = b.ks, h = b.bs, xk = b.ko, w = b.bo, d0 = b.dk, d1 = b.dkp1;
     float g_y, g_yk, g_h, g_xk, g_w, g_d0, g_d1;
-    rqs_scalar_inverse_adjoints(y, gx, yk, h, xk, w, d0, d1, g_y, g_yk, g_h, g_xk, g_w, g_d0, g_d1);
+    rqs_scalar_inverse_adjoints<LD>(y, gx, gld, yk, h, xk, w, d0, d1, g_y, g_yk, g_h, g_xk, g_w, g_d0, g_d1);
     rqs_theta_adjoints<KT>(row, K, idx, kn, g_xk, g_w, g_yk, g_h, g_d0, g_d1);
     return g_y;
 }

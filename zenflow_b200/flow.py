@@ -7,7 +7,9 @@ requires grad, the result is differentiable: its backward is one zf_flow_log_pro
 (the running statistics stay fixed, as under jax.grad of the reference's eval call).  ``Flow.sample`` draws the latent
 on the device and runs the fused inverse chain (zf_flow_sample); ``Flow.inverse`` runs it on a given draw
 (zf_chain_inverse).  Both are differentiable in the same way, wrt c and the params leaves (and u for ``inverse``): the
-backward is one zf_chain_inverse_vjp call.
+backward is one zf_chain_inverse_vjp call.  ``Flow.sample_and_log_prob`` / ``Flow.inverse_and_log_prob`` return the
+samples together with their log-density from one fused inverse pass (zf_flow_sample_log_prob), differentiable the
+same way through one zf_flow_sample_log_prob_vjp call (reverse-KL fitting, importance weights, entropy estimates).
 """
 from __future__ import annotations
 
@@ -16,8 +18,8 @@ from typing import Optional, Union
 import numpy as np
 import torch
 
-from ._chain import (ChainSpec, _wants_grad, flow_inverse_differentiable, flow_log_prob_differentiable,
-                     flow_sample_differentiable)
+from ._chain import (ChainSpec, _wants_grad, flow_inverse_differentiable, flow_inverse_log_prob_differentiable,
+                     flow_log_prob_differentiable, flow_sample_differentiable, flow_sample_log_prob_differentiable)
 from ._device import like_input
 from .bijectors import Bijector, Chain, _cdim, _shape2
 from .distributions import Beta, Distribution
@@ -127,6 +129,57 @@ class Flow(Module):
             return flow_inverse_differentiable(spec, u, c)
         self.bijector._emit(spec, self.scope.child("bijector"))
         return like_input(spec.inverse(u, c), u)
+
+    def sample_and_log_prob(self, conditions_or_size: Union[int, "np.ndarray", "torch.Tensor"], *, seed: int = 0,
+                            as_numpy: Optional[bool] = None):
+        """Return ``(x, lp)``: the samples ``sample`` returns for the same arguments (bit for bit) and their
+        log-density, from one fused inverse pass.
+
+        lp = nan_to_num(sum_j log p_latent(z_j) - log|det dx/dz|) is the exact density of the map that produced x: the
+        change of variables of the inverse as the reference writes it (the analytic quadratic-root spline inverse, no EPS,
+        no clip; ShiftBounds.inverse's scale).  It is not ``self(x, c)`` evaluated on the samples, which differs by the
+        forward's EPS terms and clip and by bin flips near knots.  Return types and differentiability follow ``sample``:
+        with grad mode on and c or a ``params`` leaf requiring grad, both outputs are CUDA tensors with grad_fns (the
+        draw is a constant), unless ``as_numpy=True``."""
+        if isinstance(conditions_or_size, (int, np.integer)):
+            size = int(conditions_or_size)
+            c = None
+        else:
+            size = conditions_or_size.shape[0]
+            c = _normalize_c(conditions_or_size)
+        if self.latent.dim is None:
+            raise ValueError("latent.dim is not set yet: evaluate the flow (init/apply) once before sampling")
+        from .distributions import _seed_of
+
+        spec = ChainSpec(self.latent.dim, _cdim(c))
+        kind, peak = self.latent._native()
+        if as_numpy is not True and torch.is_grad_enabled() and (
+                _wants_grad(c) or _any_wants_grad(self.scope.subtree("params"))):
+            with torch.no_grad():
+                self.bijector._emit(spec, self.scope.child("bijector"))
+            return flow_sample_log_prob_differentiable(spec, size, c, kind, peak, _seed_of(seed))
+        self.bijector._emit(spec, self.scope.child("bijector"))
+        x, lp = spec.sample_log_prob(None, c, kind, peak, draw_seed=_seed_of(seed), n=size)
+        if as_numpy is None:
+            as_numpy = not (c is None or isinstance(c, torch.Tensor))
+        return (x.cpu().numpy(), lp.cpu().numpy()) if as_numpy else (x, lp)
+
+    def inverse_and_log_prob(self, u, c=None):
+        """Return ``(x, lp)``: ``inverse(u, c)`` (bit for bit) and the log-density of x under the map that produced it
+        from the latent draw u, as ``sample_and_log_prob`` defines it; the parity-mode counterpart of
+        ``sample_and_log_prob``.  Differentiable wrt u, c and the params leaves as ``inverse`` is."""
+        c = _normalize_c(c)
+        D = _shape2(u)[1]
+        self.latent._latch_dim(D)  # the log-density reads latent.log_prob(u)
+        spec = ChainSpec(D, _cdim(c))
+        kind, peak = self.latent._native()
+        if torch.is_grad_enabled() and (_wants_grad(u) or _wants_grad(c) or _any_wants_grad(self.scope.subtree("params"))):
+            with torch.no_grad():
+                self.bijector._emit(spec, self.scope.child("bijector"))
+            return flow_inverse_log_prob_differentiable(spec, u, c, kind, peak)
+        self.bijector._emit(spec, self.scope.child("bijector"))
+        x, lp = spec.sample_log_prob(u, c, kind, peak)
+        return like_input(x, u), like_input(lp, u)
 
     def _steps(self, x, c=None, *, inverse: bool = False):
         """Per-bijector intermediate outputs (flow.py:80-95)."""
